@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- verified pairs/s of the matching + verification hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (tcgen05 match -> ratio filter -> RANSAC-F) over one batch of synthetic input.
 N = 1: BASELINE.json configs[1], the 50-image exhaustive run (1,225 pairs x 8192 SIFT-like features per image).
@@ -10,6 +10,8 @@ over the ranks -- strong scaling; every rank holds the broadcast bank, there is 
 timed step the WHOLE result (per-pair summaries, packed match rows, inlier flags) is gathered on rank 0, which then
 checks a sample of it against its own single-GPU recomputation.  ``--scaling weak`` keeps round 1's replicated block.
 Prints ONE JSON line on rank 0.  See DESIGN.md "Measurement" for every field.
+``--dump-outputs DIR`` also writes what the last timed step returned to its caller as DIR/<name>.npy (see dump_outputs), so
+that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -38,6 +40,46 @@ RANSAC = dict(thr=3.0, confidence=0.99, max_iters=2000, solver="8pt", score="sym
 RATIO = 0.75
 OPS_PER_PAIR = 2.0 * N_FEATS * N_FEATS * 128            # algorithmic int8 ops (SURVEY.md §8d)
 NOMINAL_INT8_TOPS = 4500.0
+DUMP_BYTES = 64 * 10**6                                 # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes ``arrays`` (name -> torch tensor or ndarray) as ``out_dir/<name>.npy``: float32 stays float32, every other
+    type becomes float64 (exact for the int32 counts and indices).  Each array and its row index may fill an equal share of
+    DUMP_BYTES; an array with more rows than its share holds keeps a fixed sample of them (seed 0, in ascending order, taken
+    before the copy to the host), and the sampled row numbers go to ``<name>.rows.npy``.  Returns the paths written."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // (2 * max(len(arrays), 1)) - 256            # (npy header)
+    written = []
+    for name, a in sorted(arrays.items()):
+        f32 = str(a.dtype).endswith("float32")
+        shape = tuple(a.shape) or (1,)
+        keep = share // max((4 if f32 else 8) * int(np.prod(shape[1:])), 8)
+        if shape[0] > keep:
+            rows = np.sort(np.random.default_rng(0).permutation(shape[0])[:keep])
+            a = a[torch.as_tensor(rows, device=a.device)] if isinstance(a, torch.Tensor) else np.asarray(a)[rows]
+            written.append(os.path.join(out_dir, f"{name}.rows.npy"))
+            np.save(written[-1], rows.astype(np.float64))
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        written.append(os.path.join(out_dir, f"{name}.npy"))
+        np.save(written[-1], np.atleast_1d(a.astype(np.float32 if f32 else np.float64)))
+    return written
+
+
+def sharded_outputs(gathered, row_fields):
+    """The gathered result of a sharded step as its caller reads it: the per-pair tensors, and every row field (names in
+    ``row_fields``) in pair order -- pair p owns rows row_start[p] : row_start[p] + n_matches[p] of rank slices that have
+    unwritten room after their rows, so the buffers themselves are not the result."""
+    import torch
+
+    out = {k: v for k, v in gathered.items() if isinstance(v, torch.Tensor) and k != "row_start" and k not in row_fields}
+    if "row_start" in gathered:
+        n = gathered["n_matches"].to(torch.int64)
+        rows = torch.repeat_interleave(gathered["row_start"] - (torch.cumsum(n, 0) - n), n) + torch.arange(int(n.sum()), device=n.device)
+        out.update({k: v.index_select(0, rows) for k, v in gathered.items() if k in row_fields})
+    return out
 
 
 def load_traffic():
@@ -396,6 +438,10 @@ def run_ours(args):
             clocks["per_rank_power_w_max"] = [c.get("power_w_max") for c in every]
     value = P_total * args.steps / (total_ms * 1e-3)
     gathered, res = (None, last) if world == 1 else last
+    if args.dump_outputs and rank == 0:
+        # what the caller of the timed path holds after the last step: the VerifiedPairs of one GPU, the gathered result when sharded
+        dump_outputs(args.dump_outputs, {k: v for k, v in vars(res).items() if isinstance(v, torch.Tensor)} if world == 1
+                     else sharded_outputs(gathered, splan.RowSink.ROW_BYTES))
     ev_rows = list(step_events)
     # per-rank compute time (own kernels + row pushes) and time to the end of the gather, max / min over ranks
     sharded_info = None
@@ -628,7 +674,12 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="diagnostics: one stream (no two-stream pipeline)")
     ap.add_argument("--gather", default="full", choices=["full", "summaries"], help="what rank 0 receives inside the timed step (N > 1)")
     ap.add_argument("--transport", default="auto", choices=["auto", "p2p", "sendrecv"], help="row gather transport (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)
