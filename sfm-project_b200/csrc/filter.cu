@@ -165,6 +165,39 @@ int launch_refine_filter(const sfm_bank* b, const int32_t* pairs, int n_pairs, i
 
 using namespace sfm;
 
+// The parameter checks every filter entry point shares.  `scratch` (the sweep records) and `out_corr` may be NULL; `packed`
+// outputs address their rows with int32 offsets.
+static int check_filter_args(const char* fn, const sfm_bank* bank, int n_pairs, const sfm_filter_params* prm, const int32_t* knn_rev,
+                             const int32_t* scratch, const float* out_corr, bool packed)
+{
+    SFM_REQUIRE(n_pairs >= 0, "%s: negative pair count", fn);
+    SFM_REQUIRE(!packed || (long long)n_pairs * bank->L.feat_stride < (1ll << 31), "%s: batch too large for int32 offsets", fn);
+    SFM_REQUIRE(!prm->mutual || knn_rev, "%s: mutual check needs the reverse direction's kNN table", fn);
+    SFM_REQUIRE(prm->ratio_mode >= SFM_RATIO_NONE && prm->ratio_mode <= SFM_RATIO_EXACT_INT, "%s: unknown ratio mode %d", fn, prm->ratio_mode);
+    if (prm->ratio_mode == SFM_RATIO_EXACT_INT)
+        SFM_REQUIRE(prm->ratio_num > 0 && prm->ratio_den > 0 && prm->ratio_num < 4096 && prm->ratio_den < 4096,
+                    "%s: exact_int ratio needs 0 < num, den < 4096", fn);
+    SFM_REQUIRE(((uintptr_t)scratch & 15) == 0, "%s: scratch must be 16-byte aligned", fn);
+    SFM_REQUIRE(((uintptr_t)out_corr & 15) == 0, "%s: out_corr must be 16-byte aligned", fn);
+    return SFM_OK;
+}
+
+// Refinement + filter -> offsets -> gather for n_pairs > 0, arguments checked, on the bank's device.
+static int refine_filter_gather(const sfm_bank* bank, const int32_t* pairs_dev, int n_pairs, const sfm_filter_params* prm,
+                                const int32_t* knn_rev, int32_t* scratch, int32_t* blk_count, int32_t* out_count, int32_t* out_offset,
+                                int32_t* out_match, float* out_corr, cudaStream_t st)
+{
+    int rc = launch_refine_filter(bank, pairs_dev, n_pairs, scratch, prm, knn_rev, blk_count, out_count, st);
+    if (rc) return rc;
+    const int bpp = (int)(bank->L.feat_stride / 256);
+    offsets_scan_kernel<<<1, 1024, 0, st>>>(out_count, n_pairs, out_offset);
+    gather_packed_kernel<<<(unsigned)((long long)n_pairs * bpp), 256, 0, st>>>(pairs_dev, bank->xy, (int)bank->L.feat_stride, scratch, blk_count, bpp,
+                                                                              out_offset, out_match, out_corr);
+    SFM_CUDA_CHECK(cudaGetLastError());
+    count_launch(2);
+    return SFM_OK;
+}
+
 // Sweep -> fused refinement + filter -> offsets -> gather: the matcher of the throughput path.  Output identical to
 // sfm_match_knn2 + sfm_filter_matches_packed with the same parameters.
 extern "C" int sfm_match_pairs_packed(const sfm_bank_t* bank, const int32_t* pairs_dev, int n_pairs, const sfm_match_params* mp,
@@ -173,15 +206,8 @@ extern "C" int sfm_match_pairs_packed(const sfm_bank_t* bank, const int32_t* pai
 {
     SFM_REQUIRE(bank && pairs_dev && prm && scratch && blk_count && out_count && out_offset && out_match, "sfm_match_pairs_packed: NULL argument");
     SFM_REQUIRE(bank->metric == SFM_METRIC_L2, "sfm_match_pairs_packed: bank metric is not L2");
-    SFM_REQUIRE(n_pairs >= 0, "sfm_match_pairs_packed: negative pair count");
-    SFM_REQUIRE((long long)n_pairs * bank->L.feat_stride < (1ll << 31), "sfm_match_pairs_packed: batch too large for int32 offsets");
-    SFM_REQUIRE(!prm->mutual || knn_rev, "sfm_match_pairs_packed: mutual check needs the reverse direction's kNN table");
-    SFM_REQUIRE(prm->ratio_mode >= SFM_RATIO_NONE && prm->ratio_mode <= SFM_RATIO_EXACT_INT, "unknown ratio mode %d", prm->ratio_mode);
-    if (prm->ratio_mode == SFM_RATIO_EXACT_INT)
-        SFM_REQUIRE(prm->ratio_num > 0 && prm->ratio_den > 0 && prm->ratio_num < 4096 && prm->ratio_den < 4096,
-                    "exact_int ratio needs 0 < num, den < 4096");
-    SFM_REQUIRE(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
-    SFM_REQUIRE(!out_corr || ((uintptr_t)out_corr & 15) == 0, "out_corr must be 16-byte aligned");
+    int rc = check_filter_args("sfm_match_pairs_packed", bank, n_pairs, prm, knn_rev, scratch, out_corr, true);
+    if (rc) return rc;
     SFM_REQUIRE(!mp || mp->impl == SFM_MATCH_AUTO || mp->impl == SFM_MATCH_TCGEN05, "the fused path runs on the tcgen05 kernel");
     if (bank->n_filled <= 0) {
         set_error("sfm_match_pairs_packed: bank is empty");
@@ -204,9 +230,9 @@ extern "C" int sfm_match_pairs_packed(const sfm_bank_t* bank, const int32_t* pai
         if (pf.mode == SFM_RATIO_CV2_F32) SFM_REQUIRE(pf.ratio == prm->ratio, "prefilter ratio must equal the filter's ratio");
         else SFM_REQUIRE(pf.num2 * prm->ratio_den * prm->ratio_den == pf.den2 * prm->ratio_num * prm->ratio_num, "prefilter ratio must equal the filter's ratio");
     }
-    int rc = launch_match_tc(bank, pairs_dev, n_pairs, mp ? mp->grid : 0, scratch, nullptr, 3, pf, st);     // sweep only: records stay in scratch
+    rc = launch_match_tc(bank, pairs_dev, n_pairs, mp ? mp->grid : 0, scratch, nullptr, 3, pf, st);     // sweep only: records stay in scratch
     if (rc) return rc;
-    return sfm_refine_filter_packed(bank, pairs_dev, n_pairs, prm, knn_rev, scratch, blk_count, out_count, out_offset, out_match, out_corr, stream);
+    return refine_filter_gather(bank, pairs_dev, n_pairs, prm, knn_rev, scratch, blk_count, out_count, out_offset, out_match, out_corr, st);
 }
 
 // The second half of sfm_match_pairs_packed on its own: `scratch` holds the candidate records of a sweep
@@ -217,26 +243,20 @@ extern "C" int sfm_refine_filter_packed(const sfm_bank_t* bank, const int32_t* p
                                         int32_t* out_match, float* out_corr, void* stream)
 {
     SFM_REQUIRE(bank && pairs_dev && prm && scratch && blk_count && out_count && out_offset && out_match, "sfm_refine_filter_packed: NULL argument");
-    SFM_REQUIRE(bank->metric == SFM_METRIC_L2 && n_pairs >= 0, "sfm_refine_filter_packed: bad argument");
-    SFM_REQUIRE((long long)n_pairs * bank->L.feat_stride < (1ll << 31), "sfm_refine_filter_packed: batch too large for int32 offsets");
-    SFM_REQUIRE(!prm->mutual || knn_rev, "sfm_refine_filter_packed: mutual check needs the reverse direction's kNN table");
-    SFM_REQUIRE(prm->ratio_mode >= SFM_RATIO_NONE && prm->ratio_mode <= SFM_RATIO_EXACT_INT, "unknown ratio mode %d", prm->ratio_mode);
-    SFM_REQUIRE(((uintptr_t)scratch & 15) == 0 && (!out_corr || ((uintptr_t)out_corr & 15) == 0), "scratch / out_corr must be 16-byte aligned");
+    SFM_REQUIRE(bank->metric == SFM_METRIC_L2, "sfm_refine_filter_packed: bank metric is not L2");
+    int rc = check_filter_args("sfm_refine_filter_packed", bank, n_pairs, prm, knn_rev, scratch, out_corr, true);
+    if (rc) return rc;
+    if (bank->n_filled <= 0) {
+        set_error("sfm_refine_filter_packed: bank is empty");
+        return SFM_ERR_STATE;
+    }
     cudaStream_t st = (cudaStream_t)stream;
     SFM_ON_DEVICE(bank->device);
     if (n_pairs == 0) {
         SFM_CUDA_CHECK(cudaMemsetAsync(out_offset, 0, sizeof(int32_t), st));
         return SFM_OK;
     }
-    int rc = launch_refine_filter(bank, pairs_dev, n_pairs, scratch, prm, knn_rev, blk_count, out_count, st);
-    if (rc) return rc;
-    const int bpp = (int)(bank->L.feat_stride / 256);
-    offsets_scan_kernel<<<1, 1024, 0, st>>>(out_count, n_pairs, out_offset);
-    gather_packed_kernel<<<(unsigned)((long long)n_pairs * bpp), 256, 0, st>>>(pairs_dev, bank->xy, (int)bank->L.feat_stride, scratch, blk_count, bpp,
-                                                                              out_offset, out_match, out_corr);
-    SFM_CUDA_CHECK(cudaGetLastError());
-    count_launch(2);
-    return SFM_OK;
+    return refine_filter_gather(bank, pairs_dev, n_pairs, prm, knn_rev, scratch, blk_count, out_count, out_offset, out_match, out_corr, st);
 }
 
 extern "C" int sfm_filter_matches(const sfm_bank_t* bank, const int32_t* pairs_dev, int n_pairs, const int32_t* knn_fwd,
@@ -244,13 +264,8 @@ extern "C" int sfm_filter_matches(const sfm_bank_t* bank, const int32_t* pairs_d
                                   int32_t* out_match, float* out_corr, void* stream)
 {
     SFM_REQUIRE(bank && pairs_dev && knn_fwd && prm && out_count && out_match, "sfm_filter_matches: NULL argument");
-    SFM_REQUIRE(n_pairs >= 0, "sfm_filter_matches: negative pair count");
-    SFM_REQUIRE(!prm->mutual || knn_rev, "sfm_filter_matches: mutual check needs knn_rev");
-    SFM_REQUIRE(prm->ratio_mode >= SFM_RATIO_NONE && prm->ratio_mode <= SFM_RATIO_EXACT_INT, "unknown ratio mode %d", prm->ratio_mode);
-    if (prm->ratio_mode == SFM_RATIO_EXACT_INT)
-        SFM_REQUIRE(prm->ratio_num > 0 && prm->ratio_den > 0 && prm->ratio_num < 4096 && prm->ratio_den < 4096,
-                    "exact_int ratio needs 0 < num, den < 4096");
-    SFM_REQUIRE(!out_corr || ((uintptr_t)out_corr & 15) == 0, "out_corr must be 16-byte aligned");
+    int rc = check_filter_args("sfm_filter_matches", bank, n_pairs, prm, knn_rev, nullptr, out_corr, false);
+    if (rc) return rc;
     if (n_pairs == 0) return SFM_OK;
     SFM_ON_DEVICE(bank->device);
     filter_kernel<true><<<n_pairs, 256, 0, (cudaStream_t)stream>>>(
@@ -270,14 +285,8 @@ extern "C" int sfm_filter_matches_packed(const sfm_bank_t* bank, const int32_t* 
 {
     SFM_REQUIRE(bank && pairs_dev && knn_fwd && prm && out_count && out_offset && out_match,
                 "sfm_filter_matches_packed: NULL argument");
-    SFM_REQUIRE(n_pairs >= 0, "sfm_filter_matches_packed: negative pair count");
-    SFM_REQUIRE((long long)n_pairs * bank->L.feat_stride < (1ll << 31), "sfm_filter_matches_packed: batch too large for int32 offsets");
-    SFM_REQUIRE(!prm->mutual || knn_rev, "sfm_filter_matches_packed: mutual check needs knn_rev");
-    SFM_REQUIRE(prm->ratio_mode >= SFM_RATIO_NONE && prm->ratio_mode <= SFM_RATIO_EXACT_INT, "unknown ratio mode %d", prm->ratio_mode);
-    if (prm->ratio_mode == SFM_RATIO_EXACT_INT)
-        SFM_REQUIRE(prm->ratio_num > 0 && prm->ratio_den > 0 && prm->ratio_num < 4096 && prm->ratio_den < 4096,
-                    "exact_int ratio needs 0 < num, den < 4096");
-    SFM_REQUIRE(!out_corr || ((uintptr_t)out_corr & 15) == 0, "out_corr must be 16-byte aligned");
+    int rc = check_filter_args("sfm_filter_matches_packed", bank, n_pairs, prm, knn_rev, nullptr, out_corr, true);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     SFM_ON_DEVICE(bank->device);
     if (n_pairs == 0) {

@@ -18,12 +18,13 @@ No collective runs inside the compute phase, so there is nothing to fuse with a 
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import numpy as np
 import torch
 import torch.distributed as dist
 
-from .plan import RowSink
+from .plan import OUTPUTS, RowSink, outputs
 
 
 def world():
@@ -136,23 +137,10 @@ def summary_columns(homography: bool = False, pose: bool = False):
     rank whose block is empty must contribute a tile of the same width as everybody else).  name -> (first column, width,
     dtype, trailing shape); column 0 is reserved."""
     cols, w = {}, 1
-
-    def add(name, width, dt, shape):
-        nonlocal w
-        cols[name] = (w, width, dt, shape)
-        w += width
-
-    add("n_matches", 1, torch.int32, ())
-    add("n_inliers", 1, torch.int32, ())
-    add("iters", 1, torch.int32, ())
-    add("F", 9, torch.float64, (3, 3))
-    if homography:
-        add("H", 9, torch.float64, (3, 3))
-        add("n_inliers_h", 1, torch.int32, ())
-    if pose:
-        add("R", 9, torch.float64, (3, 3))
-        add("t", 3, torch.float64, (3,))
-        add("n_pose", 1, torch.int32, ())
+    for o in outputs(homography, pose):
+        if o.per == "pair":
+            cols[o.name] = (w, math.prod(o.shape), o.dtype, o.shape)
+            w += math.prod(o.shape)
     return cols, w
 
 
@@ -207,10 +195,6 @@ class _DevArray:
         self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 2, "strides": None}
 
 
-_TORCH_ROW = {"matches": (torch.int32, 3, "<i4"), "inlier": (torch.uint8, 1, "|u1"), "inlier_h": (torch.uint8, 1, "|u1"),
-              "in_front": (torch.uint8, 1, "|u1"), "points3d": (torch.float32, 3, "<f4")}
-
-
 class GatherRegion:
     """Receive buffers on ``dst`` for the packed rows of every rank's pair block, and each rank's way into its slice.
 
@@ -254,14 +238,12 @@ class GatherRegion:
         if want == "sendrecv":
             my_cap = max(self.caps[self.rank], 1)
             for name in self.fields:
-                dt, width, _ = _TORCH_ROW[name]
-                shape = (lambda n: (n, width) if width > 1 else (n,))          # noqa: E731
                 if self.rank == self.dst:
-                    self.full[name] = torch.empty(shape(max(self.total_cap, 1)), dtype=dt, device=self.device)
+                    self.full[name] = OUTPUTS[name].empty(max(self.total_cap, 1), device=self.device)
                     b = int(self.base[self.rank])
                     self.local[name] = self.full[name][b: b + my_cap]
                 else:
-                    self.local[name] = torch.empty(shape(my_cap), dtype=dt, device=self.device)
+                    self.local[name] = OUTPUTS[name].empty(my_cap, device=self.device)
         self._sink = None
         self._fence = None
 
@@ -291,9 +273,8 @@ class GatherRegion:
         try:
             if self.rank == self.dst:
                 for name in self.fields:
-                    dt, width, typestr = _TORCH_ROW[name]
-                    n = max(self.total_cap, 1)
-                    arr = _DevArray(self._owned_ptrs[name], (n, width) if width > 1 else (n,), typestr)
+                    o = OUTPUTS[name]
+                    arr = _DevArray(self._owned_ptrs[name], (max(self.total_cap, 1),) + o.shape, o.empty(0).numpy().dtype.str)
                     self.full[name] = torch.as_tensor(arr, device=self.device)
                     self._peer_ptrs[name] = self._owned_ptrs[name]
             else:
@@ -472,7 +453,7 @@ def match_and_verify_sharded(bank, pairs, *, mode: str = "block", dst: int = 0, 
     pose = params.get("intrinsics") is not None
     region = sink = None
     if gather == "full":
-        fields = ("matches", "inlier") + (("inlier_h",) if homography else ()) + (("in_front", "points3d") if pose else ())
+        fields = tuple(o.name for o in outputs(homography, pose) if o.per == "row")
         region, twin = get_regions(bank, n_total, mode, fields, dst, rows_per_pair_cap, transport).next()
         sink = region.sink()
         region.fence_wait(sink)                       # issued one job ago

@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from .bank import DescriptorBank
-from .plan import HotPathPlan, RowSink
+from .plan import OUTPUTS, HotPathPlan, RowSink, outputs
 
 
 @dataclass
@@ -45,20 +45,19 @@ class VerifiedPairs:
         if self.host is not None:
             out = dict(self.host)
             if not with_matches:
-                for k in ("matches", "inlier", "offsets", "inlier_h", "in_front", "points3d"):
+                for k in ["offsets"] + [o.name for o in OUTPUTS.values() if o.per == "row"]:
                     out.pop(k, None)
             return out
         if with_matches:
             raise ValueError("matches were not fetched: call match_and_verify(..., fetch=True)")
-        out = {"pairs": self.pairs.cpu().numpy(), "n_matches": self.n_matches.cpu().numpy(), "F": self.F.cpu().numpy(),
-               "n_inliers": self.n_inliers.cpu().numpy(), "iters": self.iters.cpu().numpy()}
-        for k in ("H", "n_inliers_h", "R", "t", "n_pose"):
-            if getattr(self, k) is not None:
-                out[k] = getattr(self, k).cpu().numpy()
+        out = {"pairs": self.pairs.cpu().numpy()}
+        for o in OUTPUTS.values():
+            if o.per == "pair" and getattr(self, o.name) is not None:
+                out[o.name] = getattr(self, o.name).cpu().numpy()
         return out
 
 
-_PLAN_KEYS = ("ratio", "ratio_mode", "mutual", "impl", "thr", "confidence", "max_iters", "solver", "score", "lo", "seed",
+_PLAN_KEYS = ("ratio", "ratio_mode", "mutual", "thr", "confidence", "max_iters", "solver", "score", "lo", "seed",
               "min_inliers", "prefilter", "homography", "distance_thresh", "h_stop_ratio", "overlap")
 
 
@@ -79,7 +78,7 @@ def get_plan(bank: DescriptorBank, batch: int, **params) -> HotPathPlan:
     return plan
 
 
-def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2_f32", mutual=False, impl="auto",
+def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2_f32", mutual=False,
                      thr=3.0, confidence=0.99, max_iters=2000, solver="7pt", score="sym_epipolar", lo=False, seed=0,
                      min_inliers=0, pair_batch: int = 2048, pair_ids=None, fetch=False,
                      prefilter: bool = True, homography: bool = False, intrinsics=None, distance_thresh: float = 50.0,
@@ -91,7 +90,7 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
     inlier flags to the host (pinned buffers, copies overlapped with the RANSAC kernel of the same batch and the
     sweep of the next one); ``fetch="view"`` hands out the pinned result arrays themselves
     (zero host copies; valid until the next call with the same parameters on this bank).  ``prefilter`` lets the sweep drop rows that provably fail the ratio test before the
-    exact refinement (results are identical with or without it).  ``overlap`` (tcgen05 path) runs the sweep of batch k + 1 on the caller's
+    exact refinement (results are identical with or without it).  ``overlap`` runs the sweep of batch k + 1 on the caller's
     stream while batch k is refined, filtered and verified on a second stream (a job that fits one batch is cut in two for it); on return the
     caller's stream has waited for everything.
 
@@ -111,27 +110,17 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
     if sink is not None and fetch:
         raise ValueError("fetch and sink are alternatives: rows go either to pinned host memory or to a device sink")
     if P == 0:
-        z = lambda *s, dt=torch.int32: torch.zeros(s, dtype=dt, device=dev)  # noqa: E731
+        # the arrays of every requested stage exist (empty), so that callers never have to special-case P == 0
+        outs = outputs(homography, intrinsics is not None)
         host = None
         if fetch:
-            host = {"pairs": pairs_host, "n_matches": np.zeros(0, np.int32), "F": np.zeros((0, 3, 3)), "n_inliers": np.zeros(0, np.int32),
-                    "iters": np.zeros(0, np.int32), "matches": np.zeros((0, 3), np.int32), "inlier": np.zeros(0, np.uint8),
-                    "offsets": np.zeros(1, np.int64)}
-        extra0 = {}
-        if homography:                               # the optional stages were requested: their (empty) arrays exist, so that
-            extra0.update(H=z(0, 3, 3, dt=torch.float64), n_inliers_h=z(0))      # callers never have to special-case P == 0
-            if host is not None:
-                host.update(H=np.zeros((0, 3, 3)), n_inliers_h=np.zeros(0, np.int32), inlier_h=np.zeros(0, np.uint8))
-        if intrinsics is not None:
-            extra0.update(R=z(0, 3, 3, dt=torch.float64), t=z(0, 3, dt=torch.float64), n_pose=z(0))
-            if host is not None:
-                host.update(R=np.zeros((0, 3, 3)), t=np.zeros((0, 3)), n_pose=np.zeros(0, np.int32), in_front=np.zeros(0, np.uint8),
-                            points3d=np.zeros((0, 3), np.float32))
-        return VerifiedPairs(z(0, 2), z(0), z(0, 3, 3, dt=torch.float64), z(0), z(0), host, **extra0)
+            host = {"pairs": pairs_host, "offsets": np.zeros(1, np.int64), **{o.name: o.empty(0).numpy() for o in outs}}
+        return VerifiedPairs(pairs=torch.zeros((0, 2), dtype=torch.int32, device=dev), host=host,
+                             **{o.name: o.empty(0, device=dev) for o in outs if o.per == "pair"})
     batch = int(min(pair_batch, P))
-    if overlap and impl in ("auto", "tcgen05") and not _segments and 512 <= P <= batch:
+    if overlap and not _segments and 512 <= P <= batch:
         batch = -(-P // 2)                          # one-batch job: two halves, so that the first half's refinement hides under the second sweep
-    plan = get_plan(bank, batch, ratio=ratio, ratio_mode=ratio_mode, mutual=mutual, impl=impl, thr=thr, confidence=confidence,
+    plan = get_plan(bank, batch, ratio=ratio, ratio_mode=ratio_mode, mutual=mutual, thr=thr, confidence=confidence,
                     max_iters=max_iters, solver=solver, score=score, lo=lo, seed=seed, min_inliers=min_inliers, prefilter=prefilter,
                     homography=homography, intrinsics=intrinsics, distance_thresh=distance_thresh, h_stop_ratio=h_stop_ratio, overlap=overlap)
     # one upload of the whole pair list and its RANSAC stream ids through a pinned staging buffer kept on the bank
@@ -153,20 +142,7 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
     rev_d = pairs_d.flip(1).contiguous() if mutual else None
     # (the full-length result arrays are allocated after the first batch has been enqueued: every host microsecond before
     #  the first kernel is GPU idle time, everything after it hides behind the sweep)
-    n_matches = F = n_inl = iters = None
-    extra = {}
-
-    def _allocate_results():
-        nonlocal n_matches, F, n_inl, iters
-        n_matches = torch.empty(P, dtype=torch.int32, device=dev)
-        F = torch.empty((P, 3, 3), dtype=torch.float64, device=dev)
-        n_inl = torch.empty(P, dtype=torch.int32, device=dev)
-        iters = torch.empty(P, dtype=torch.int32, device=dev)
-        if homography:
-            extra.update(H=torch.empty((P, 3, 3), dtype=torch.float64, device=dev), n_inliers_h=torch.empty(P, dtype=torch.int32, device=dev))
-        if intrinsics is not None:
-            extra.update(R=torch.empty((P, 3, 3), dtype=torch.float64, device=dev), t=torch.empty((P, 3), dtype=torch.float64, device=dev),
-                         n_pose=torch.empty(P, dtype=torch.int32, device=dev))
+    results = {}
 
     # batches: consecutive runs of <= batch pairs; with _segments (streamed upload) a batch never crosses a segment end and
     # first waits for the event that says the segment's images are in the bank
@@ -201,23 +177,14 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
         o = plan.launch(pairs_d[s: s + n], ids_d[s: s + n], None if rev_d is None else rev_d[s: s + n])
         if trace is not None:
             trace.append(time.perf_counter())
-        if n_matches is None:
-            _allocate_results()
+        if not results:
+            results = {a.name: a.empty(P, device=dev) for a in plan.outputs if a.per == "pair"}
             if plan.overlap:                         # the result arrays were allocated on the caller's stream and are written on the second one
                 plan.post_stream.wait_stream(torch.cuda.current_stream(dev))
         # per-pair summaries of this batch into the full-length device arrays (tiny device copies, ordered behind the batch's kernels)
         with torch.cuda.stream(plan.result_stream()):
-            n_matches[s: s + n].copy_(o.counts[:n])
-            F[s: s + n].copy_(o.F[:n])
-            n_inl[s: s + n].copy_(o.ninl[:n])
-            iters[s: s + n].copy_(o.iters[:n])
-            if homography:
-                extra["H"][s: s + n].copy_(o.H[:n])
-                extra["n_inliers_h"][s: s + n].copy_(o.ninl_h[:n])
-            if intrinsics is not None:
-                extra["R"][s: s + n].copy_(o.R[:n])
-                extra["t"][s: s + n].copy_(o.t[:n])
-                extra["n_pose"][s: s + n].copy_(o.ngood[:n])
+            for name, full in results.items():
+                full[s: s + n].copy_(getattr(o, name)[:n])
         if fetch:
             # the host learns batch k's packed size only after batch k + 1 has been enqueued: the GPU never waits for it
             if prev is not None:
@@ -246,7 +213,7 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
             h = {k: v.copy() for k, v in h.items()}
         host = dict(h)
         host["pairs"] = pairs_host
-    return VerifiedPairs(pairs_d.clone(), n_matches, F, n_inl, iters, host, d2h, plan=plan, **extra)      # (pairs_d is a view of the staging buffer)
+    return VerifiedPairs(pairs=pairs_d.clone(), host=host, d2h_bytes=d2h, plan=plan, **results)      # (pairs_d is a view of the staging buffer)
 
 
 def match_and_verify_host(desc, xy, pairs, *, bank: DescriptorBank | None = None, n_chunks: int = 3, fetch=True, pair_ids=None, chunk_growth: float = 1.0, **params):

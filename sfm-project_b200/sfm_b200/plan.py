@@ -1,11 +1,12 @@
 """Execution plan of the hot path for batches of image pairs: preallocated device and pinned-host buffers, a
 fixed launch sequence on the caller's stream, and result copies on a side stream that overlap the RANSAC kernel.
 
-    sweep (tcgen05) -> refine -> [reverse sweep -> refine]      sfm_match_knn2
-    count -> scan -> write (packed matches + correspondences)    sfm_filter_matches_packed
+    [reverse sweep -> refine: the full kNN table]                sfm_match_knn2                 (mutual=True)
+    sweep (tcgen05): candidate records into the scratch          sfm_match_knn2, sweep_only = 4
+    refine + ratio / mutual filter -> scan -> gather             sfm_refine_filter_packed       (on a second stream with overlap=True)
     RANSAC-F on the packed correspondences                       sfm_ransac_f_packed
-    [RANSAC-H on the same correspondences]                       sfm_ransac_h_packed       (homography=True)
-    [E, (R, t) by cheirality vote, triangulated inliers]         sfm_two_view_pose_packed  (intrinsics given)
+    [RANSAC-H on the same correspondences]                       sfm_ransac_h_packed            (homography=True)
+    [E, (R, t) by cheirality vote, triangulated inliers]         sfm_two_view_pose_packed       (intrinsics given)
 
 This is the batched body of the reference's pair loop (code/pipeline.py:38-47) plus the verification stage it left
 empty (code/pipeline.py:60-65).  Nothing here computes: every array is produced by lib/libsfm_b200.so.
@@ -13,6 +14,8 @@ empty (code/pipeline.py:60-65).  Nothing here computes: every array is produced 
 from __future__ import annotations
 
 import ctypes as C
+import math
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -39,8 +42,53 @@ def intrinsics_rows(intrinsics, n_images: int) -> np.ndarray:
     return np.ascontiguousarray(a[:n_images])
 
 
-# When bench.py sets this to a list, every sweep launch of the two-stream pipeline appends (start event, end event, pairs):
-# the roofline's launch duration is then the one measured inside the timed steps, on the stream the kernel runs on.
+class Output(NamedTuple):
+    """One result array of the pipeline.  ``per`` is "pair" or "row" (one row per surviving match, packed: pair p owns rows
+    [offsets[p], offsets[p+1])); ``shape`` is the trailing shape; ``stage`` is None (always), "homography" or "pose"; ``ready``
+    says when a row array is complete: "filter" (written by the filter) or "done" (after the batch's last kernel)."""
+
+    name: str
+    per: str
+    dtype: torch.dtype
+    shape: tuple
+    stage: str | None = None
+    ready: str = "done"
+
+    @property
+    def nbytes(self) -> int:
+        """Bytes per pair or per row."""
+        return self.dtype.itemsize * math.prod(self.shape)
+
+    def empty(self, n: int, **kw) -> torch.Tensor:
+        return torch.empty((n,) + self.shape, dtype=self.dtype, **kw)
+
+
+# Every result array, in the order results list them.  n_matches is never copied to the host: the host derives it from the offsets.
+OUTPUTS = {o.name: o for o in (
+    Output("n_matches", "pair", torch.int32, ()),
+    Output("F", "pair", torch.float64, (3, 3)),                     # zeros when no model
+    Output("n_inliers", "pair", torch.int32, ()),
+    Output("iters", "pair", torch.int32, ()),                       # hypotheses evaluated
+    Output("H", "pair", torch.float64, (3, 3), "homography"),       # x2 ~ H x1, H[2,2] == 1 (zeros when no model)
+    Output("n_inliers_h", "pair", torch.int32, (), "homography"),
+    Output("R", "pair", torch.float64, (3, 3), "pose"),             # x2 ~ R x1 + t
+    Output("t", "pair", torch.float64, (3,), "pose"),               # |t| = 1
+    Output("n_pose", "pair", torch.int32, (), "pose"),              # inliers in front of both cameras
+    Output("matches", "row", torch.int32, (3,), ready="filter"),    # (queryIdx, trainIdx, squared L2)
+    Output("inlier", "row", torch.uint8, ()),
+    Output("inlier_h", "row", torch.uint8, (), "homography"),
+    Output("in_front", "row", torch.uint8, (), "pose"),
+    Output("points3d", "row", torch.float32, (3,), "pose"),         # in the first camera's frame
+)}
+
+
+def outputs(homography: bool = False, pose: bool = False) -> list[Output]:
+    """The result arrays of a run with the given optional stages."""
+    return [o for o in OUTPUTS.values() if o.stage is None or (o.stage == "homography" and homography) or (o.stage == "pose" and pose)]
+
+
+# When bench.py sets this to a list, every sweep launch appends (start event, end event, pairs): the roofline's launch
+# duration is then the one measured inside the timed steps, on the stream the kernel runs on.
 SWEEP_EVENTS = None
 
 
@@ -50,7 +98,7 @@ class RowSink:
     dist.GatherRegion).  ``fields`` maps a row array name to (base pointer of this job's slice, bytes per row); the rows of
     consecutive batches land back to back, ``rows`` is the host-side cursor."""
 
-    ROW_BYTES = {"matches": 12, "inlier": 1, "inlier_h": 1, "in_front": 1, "points3d": 12}
+    ROW_BYTES = {o.name: o.nbytes for o in OUTPUTS.values() if o.per == "row"}
 
     def __init__(self, fields: dict, cap_rows: int):
         for name in fields:
@@ -69,31 +117,15 @@ class RowSink:
 
 
 class _OutSet:
-    """Device outputs of one batch.  Two sets alternate so that batch k + 1 can be enqueued before the host has read
-    batch k's packed size and started its copies."""
+    """Device outputs of one batch, one attribute per result array of the plan (``OUTPUTS``) plus the packed offsets and
+    correspondences.  Two sets alternate so that batch k + 1 can be enqueued before the host has read batch k's packed size
+    and started its copies."""
 
-    def __init__(self, B, cap, dev, homography=False, pose=False):
-        i32 = dict(dtype=torch.int32, device=dev)
-        f64 = dict(dtype=torch.float64, device=dev)
-        self.H = self.ninl_h = self.mask_h = self.R = self.t = self.ngood = self.pmask = self.X = None
-        if homography:
-            self.H = torch.zeros((B, 3, 3), **f64)
-            self.ninl_h = torch.zeros(B, **i32)
-            self.mask_h = torch.empty(B * cap, dtype=torch.uint8, device=dev)
-        if pose:
-            self.R = torch.zeros((B, 3, 3), **f64)
-            self.t = torch.zeros((B, 3), **f64)
-            self.ngood = torch.zeros(B, **i32)
-            self.pmask = torch.empty(B * cap, dtype=torch.uint8, device=dev)
-            self.X = torch.empty((B * cap, 3), dtype=torch.float32, device=dev)
-        self.counts = torch.zeros(B, **i32)
-        self.offsets = torch.zeros(B + 1, **i32)
-        self.matches = torch.empty((B * cap, 3), **i32)
+    def __init__(self, B, cap, dev, outs):
+        for o in outs:
+            setattr(self, o.name, o.empty(B, device=dev).zero_() if o.per == "pair" else o.empty(B * cap, device=dev))
+        self.offsets = torch.zeros(B + 1, dtype=torch.int32, device=dev)
         self.corr = torch.empty((B * cap, 4), dtype=torch.float32, device=dev)
-        self.mask = torch.empty(B * cap, dtype=torch.uint8, device=dev)
-        self.F = torch.zeros((B, 3, 3), dtype=torch.float64, device=dev)
-        self.ninl = torch.zeros(B, **i32)
-        self.iters = torch.zeros(B, **i32)
         self.offsets_h = torch.zeros(B + 1, dtype=torch.int32).pin_memory()
         self.ev_filter, self.ev_done = torch.cuda.Event(), torch.cuda.Event()
         self.ev_offsets, self.ev_copied = torch.cuda.Event(), torch.cuda.Event()
@@ -101,16 +133,20 @@ class _OutSet:
         self.P = 0
         self.pair_id = None
 
+    @property
+    def counts(self) -> torch.Tensor:
+        return self.n_matches
+
 
 class HotPathPlan:
     """Buffers + launch sequence for up to ``max_pairs`` pairs per batch on one bank.
 
-    Packed result layout (device and host): pair p of a batch owns rows [offsets[p], offsets[p+1]) of
-    ``matches`` int32 [total,3] = (queryIdx, trainIdx, squared L2), ``corr`` float32 [total,4] and ``mask`` uint8 [total].
-    Host results of a whole job (any number of batches) land back to back in ONE set of pinned arrays.
+    Packed result layout (device and host): pair p of a batch owns rows [offsets[p], offsets[p+1]) of every row array
+    (``OUTPUTS``) and of ``corr`` float32 [total,4].  Host results of a whole job (any number of batches) land back to back
+    in ONE set of pinned arrays.
     """
 
-    def __init__(self, bank: DescriptorBank, max_pairs: int, *, ratio=0.75, ratio_mode="cv2_f32", mutual=False, impl="auto",
+    def __init__(self, bank: DescriptorBank, max_pairs: int, *, ratio=0.75, ratio_mode="cv2_f32", mutual=False,
                  thr=3.0, confidence=0.99, max_iters=2000, solver="7pt", score="sym_epipolar", lo=False, seed=0,
                  min_inliers=0, prefilter=True, homography=False, intrinsics=None, distance_thresh=50.0, h_stop_ratio=0.8, overlap=True):
         if bank.metric != "l2":
@@ -124,25 +160,28 @@ class HotPathPlan:
         self.fprm = filter_params(ratio, ratio_mode, mutual)
         self.rprm = ransac_params(thr=thr, confidence=confidence, max_iters=max_iters, solver=solver, score=score, lo=lo,
                                   seed=seed, min_inliers=min_inliers)
+        # The sweep alone: candidate records into the scratch, refined and filtered by sfm_refine_filter_packed.  With the
+        # prefilter it marks rows that cannot pass the ratio test; the refinement skips them (they read as "no match").
         self.mprm = _lib.MatchParams()
-        self.mprm.impl = _lib.MATCH_IMPLS[impl]
+        self.mprm.sweep_only = 4
+        if prefilter:
+            self.mprm.prefilter_mode, self.mprm.prefilter_ratio = self.fprm.ratio_mode, self.fprm.ratio
+            self.mprm.prefilter_num, self.mprm.prefilter_den = int(self.fprm.ratio_num), int(self.fprm.ratio_den)
         # (mutual matching: the forward direction keeps the prefilter -- a row that fails the ratio test is dropped whatever its
-        #  reverse neighbour is; the reverse direction needs every row's exact nearest neighbour and runs without it)
-        self.prefilter = bool(prefilter)
+        #  reverse neighbour is; the reverse direction needs every row's exact nearest neighbour: a full kNN table without it)
+        self.rev_prm = _lib.MatchParams()
         B, cap, dev = self.B, self.cap, self.dev
         self.knn = torch.empty((B, cap, 4), dtype=torch.int32, device=dev)       # sweep records, then the compacted rows per block
         self.blk_count = torch.empty(B * (cap // 256), dtype=torch.int32, device=dev)
-        self.fused = impl in ("auto", "tcgen05")                                  # refinement + filter in one pass (no kNN table)
         self.knn_rev = torch.empty((B, cap, 4), dtype=torch.int32, device=dev) if self.mutual else None
-        # Two-stream pipeline (fused path): the sweep of batch k + 1 runs on the caller's stream while batch k is refined, filtered and
+        # Two-stream pipeline: the sweep of batch k + 1 runs on the caller's stream while batch k is refined, filtered and
         # verified on ``post_stream``.  The sweep is one persistent 352-thread CTA per SM and leaves registers / shared memory / issue slots
         # for one refinement CTA beside it, so the L1-bound refinement hides under the tensor-bound sweep (4.9 % on a four-batch job,
         # profiles/r02_overlap_proto.log).  Scratch and reverse tables are double-buffered for it (second copies made on first use).
-        self.overlap = self.fused and bool(overlap)
+        self.overlap = bool(overlap)
         self.post_stream = torch.cuda.Stream(device=dev) if self.overlap else None
         self._scratch = [(self.knn, self.blk_count, self.knn_rev)]
         self._consumed = [None, None]                                            # event: the post stage has finished with scratch[i]
-        self._ev_sweep = torch.cuda.Event()
         # optional stages after RANSAC-F (SURVEY.md 8f ranks 2 and 4)
         self.homography = bool(homography)
         self.h_ratio = None if h_stop_ratio is None else float(h_stop_ratio)
@@ -151,13 +190,18 @@ class HotPathPlan:
         if intrinsics is not None:
             self.intr = torch.as_tensor(intrinsics_rows(intrinsics, bank.max_images)).to(dev)
         self.dist = float(distance_thresh)
-        self.sets = [_OutSet(B, cap, dev, self.homography, self.intr is not None)]   # the second set is created on the first multi-batch job
+        self.outputs = outputs(self.homography, self.intr is not None)
+        self.sets = [_OutSet(B, cap, dev, self.outputs)]                        # the second set is created on the first multi-batch job
         self.cur = self.sets[0]
         self._n_launched = 0
         self.copy_stream = torch.cuda.Stream(device=dev)
-        # pinned host results of a job
+        # pinned host results of a job: every row array, every per-pair array but n_matches (the host has it from the offsets)
+        self._host_rows = [o for o in self.outputs if o.per == "row"]
+        self._host_pairs = [o for o in self.outputs if o.per == "pair" and o.name != "n_matches"]
+        self._row_bytes = sum(o.nbytes for o in self._host_rows)
+        self._pair_bytes = sum(o.nbytes for o in self._host_pairs)
+        self.host = {}
         self._rows_cap = self._pairs_cap = 0
-        self.matches_h = self.mask_h = self.F_h = self.ninl_h = self.iters_h = None
         self.job_rows = self.job_pairs = self.job_d2h = 0
         self.job_counts = []
 
@@ -176,11 +220,6 @@ class HotPathPlan:
             return o
         L, st, bank = _lib.lib(), _lib.current_stream_ptr(self.dev), self.bank
         cur = torch.cuda.current_stream(self.dev)
-        if self.prefilter:
-            # the sweep marks rows that cannot pass the ratio test; the refinement skips them (they read as "no match")
-            self.mprm.prefilter_mode = self.fprm.ratio_mode
-            self.mprm.prefilter_ratio = self.fprm.ratio
-            self.mprm.prefilter_num, self.mprm.prefilter_den = int(self.fprm.ratio_num), int(self.fprm.ratio_den)
         slot = (self._n_launched - 1) % 2 if self.overlap else 0
         if slot >= len(self._scratch):                # second scratch set of the two-stream pipeline, on first use
             B, cap = self.B, self.cap
@@ -188,78 +227,61 @@ class HotPathPlan:
                                   torch.empty(B * (cap // 256), dtype=torch.int32, device=self.dev),
                                   torch.empty((B, cap, 4), dtype=torch.int32, device=self.dev) if self.mutual else None))
         knn, blk_count, knn_rev = self._scratch[slot]
-        if self.overlap and self._consumed[slot] is not None:
+        if self._consumed[slot] is not None:
             cur.wait_event(self._consumed[slot])      # the batch that used this scratch two launches ago has been refined and gathered
-        if not self.fused:
-            _lib.check(L.sfm_match_knn2(bank.handle, _lib.ptr(pairs_d), P, C.byref(self.mprm), _lib.ptr(knn), st),
-                       "sfm_match_knn2")
         if self.mutual:
             if pairs_rev_d is None:
                 pairs_rev_d = pairs_d.flip(1).contiguous()
-            plain = _lib.MatchParams()
-            plain.impl = self.mprm.impl
-            _lib.check(L.sfm_match_knn2(bank.handle, _lib.ptr(pairs_rev_d), P, C.byref(plain), _lib.ptr(knn_rev), st),
+            _lib.check(L.sfm_match_knn2(bank.handle, _lib.ptr(pairs_rev_d), P, C.byref(self.rev_prm), _lib.ptr(knn_rev), st),
                        "sfm_match_knn2 (reverse)")
+        timing = SWEEP_EVENTS is not None                                                  # bench.py: in-situ duration of the sweep launches
+        if timing:
+            t0 = torch.cuda.Event(enable_timing=True)
+            t0.record(cur)
+        _lib.check(L.sfm_match_knn2(bank.handle, _lib.ptr(pairs_d), P, C.byref(self.mprm), _lib.ptr(knn), st), "sfm_match_knn2 (sweep)")
+        ev_sweep = torch.cuda.Event(enable_timing=timing)
+        ev_sweep.record(cur)
+        if timing:
+            SWEEP_EVENTS.append((t0, ev_sweep, P))
         if self.overlap:
-            sw = _lib.MatchParams()
-            sw.impl, sw.grid, sw.sweep_only = self.mprm.impl, self.mprm.grid, 4          # the sweep alone: candidate records into the scratch
-            sw.prefilter_mode, sw.prefilter_ratio = self.mprm.prefilter_mode, self.mprm.prefilter_ratio
-            sw.prefilter_num, sw.prefilter_den = self.mprm.prefilter_num, self.mprm.prefilter_den
-            timing = SWEEP_EVENTS is not None                                              # bench.py: in-situ duration of the sweep launches
-            if timing:
-                t0 = torch.cuda.Event(enable_timing=True)
-                t0.record(cur)
-            _lib.check(L.sfm_match_knn2(bank.handle, _lib.ptr(pairs_d), P, C.byref(sw), _lib.ptr(knn), st), "sfm_match_knn2 (sweep)")
-            self._ev_sweep = torch.cuda.Event(enable_timing=timing)
-            self._ev_sweep.record(cur)
-            if timing:
-                SWEEP_EVENTS.append((t0, self._ev_sweep, P))
             cur = self.post_stream                    # everything below is enqueued behind the sweep on the second stream
-            cur.wait_event(self._ev_sweep)
+            cur.wait_event(ev_sweep)
             st = C.c_void_p(cur.cuda_stream)
         with torch.cuda.stream(cur):
             self._launch_post(o, pairs_d, pair_id_d, P, knn, blk_count, knn_rev, cur, st, slot)
         return o
 
     def _launch_post(self, o, pairs_d, pair_id_d, P, knn, blk_count, knn_rev, cur, st, slot):
-        """Refinement + filter (or the filter alone on the kNN-table path), RANSAC-F and the optional stages of one batch on ``cur``."""
+        """Refinement + filter, RANSAC-F and the optional stages of one batch on ``cur``."""
         L, bank = _lib.lib(), self.bank
         if o.copy_pending:                            # result copies of the batch that used this set last
             cur.wait_event(o.ev_copied)
             o.copy_pending = False
+        # refinement + ratio / mutual filter in one pass -> offsets -> gather (the kNN table is never written)
+        _lib.check(L.sfm_refine_filter_packed(bank.handle, _lib.ptr(pairs_d), P, C.byref(self.fprm), _lib.ptr(knn_rev), _lib.ptr(knn),
+                                              _lib.ptr(blk_count), _lib.ptr(o.n_matches), _lib.ptr(o.offsets), _lib.ptr(o.matches),
+                                              _lib.ptr(o.corr), st), "sfm_refine_filter_packed")
         if self.overlap:
-            _lib.check(L.sfm_refine_filter_packed(bank.handle, _lib.ptr(pairs_d), P, C.byref(self.fprm), _lib.ptr(knn_rev), _lib.ptr(knn),
-                                                  _lib.ptr(blk_count), _lib.ptr(o.counts), _lib.ptr(o.offsets), _lib.ptr(o.matches), _lib.ptr(o.corr), st),
-                       "sfm_refine_filter_packed")
             ev = torch.cuda.Event()
             ev.record(cur)
             self._consumed[slot] = ev
-        elif self.fused:
-            # sweep -> refinement + ratio / mutual filter in one pass -> offsets -> gather (the kNN table is never written)
-            _lib.check(L.sfm_match_pairs_packed(bank.handle, _lib.ptr(pairs_d), P, C.byref(self.mprm), C.byref(self.fprm), _lib.ptr(knn_rev),
-                                                _lib.ptr(knn), _lib.ptr(blk_count), _lib.ptr(o.counts), _lib.ptr(o.offsets),
-                                                _lib.ptr(o.matches), _lib.ptr(o.corr), st), "sfm_match_pairs_packed")
-        else:
-            _lib.check(L.sfm_filter_matches_packed(bank.handle, _lib.ptr(pairs_d), P, _lib.ptr(knn), _lib.ptr(knn_rev),
-                                                   C.byref(self.fprm), _lib.ptr(o.counts), _lib.ptr(o.offsets),
-                                                   _lib.ptr(o.matches), _lib.ptr(o.corr), st), "sfm_filter_matches_packed")
         o.ev_filter.record(cur)
         _lib.check(L.sfm_ransac_f_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), P, self.cap, _lib.ptr(pair_id_d), None,
-                                         C.byref(self.rprm), _lib.ptr(o.F), _lib.ptr(o.ninl), _lib.ptr(o.mask),
+                                         C.byref(self.rprm), _lib.ptr(o.F), _lib.ptr(o.n_inliers), _lib.ptr(o.inlier),
                                          _lib.ptr(o.iters), st), "sfm_ransac_f_packed")
         if self.homography:
             # the scene graph only asks whether H explains more than h_ratio of what F explains: sampling may stop once a
             # homography with that support would have been found (general pairs: 32 hypotheses instead of max_iters)
-            tgt = None if self.h_ratio is None else h_stop_target(o.ninl[:P], self.h_ratio)
+            tgt = None if self.h_ratio is None else h_stop_target(o.n_inliers[:P], self.h_ratio)
             _lib.check(L.sfm_ransac_h_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), P, self.cap, _lib.ptr(pair_id_d), None, _lib.ptr(tgt),
-                                             C.byref(self.hprm), _lib.ptr(o.H), _lib.ptr(o.ninl_h), _lib.ptr(o.mask_h), None, st),
+                                             C.byref(self.hprm), _lib.ptr(o.H), _lib.ptr(o.n_inliers_h), _lib.ptr(o.inlier_h), None, st),
                        "sfm_ransac_h_packed")
         if self.intr is not None:
             pl = pairs_d.long()
             cam = torch.cat([self.intr[pl[:, 0]], self.intr[pl[:, 1]]], dim=1).contiguous()      # [P, 8] per-pair camera rows
-            _lib.check(L.sfm_two_view_pose_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), P, _lib.ptr(o.mask), _lib.ptr(o.F),
-                                                  _lib.ptr(cam), self.dist, _lib.ptr(o.R), _lib.ptr(o.t), None, _lib.ptr(o.ngood),
-                                                  _lib.ptr(o.pmask), _lib.ptr(o.X), st), "sfm_two_view_pose_packed")
+            _lib.check(L.sfm_two_view_pose_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), P, _lib.ptr(o.inlier), _lib.ptr(o.F),
+                                                  _lib.ptr(cam), self.dist, _lib.ptr(o.R), _lib.ptr(o.t), None, _lib.ptr(o.n_pose),
+                                                  _lib.ptr(o.in_front), _lib.ptr(o.points3d), st), "sfm_two_view_pose_packed")
         o.ev_done.record(cur)
 
     def result_stream(self):
@@ -269,7 +291,7 @@ class HotPathPlan:
     def ensure_sets(self, n: int) -> None:
         """Multi-batch jobs rotate over two output sets, three when the rows go to a sink (created on first use)."""
         while len(self.sets) < n:
-            self.sets.append(_OutSet(self.B, self.cap, self.dev, self.homography, self.intr is not None))
+            self.sets.append(_OutSet(self.B, self.cap, self.dev, self.outputs))
 
     def rerun_ransac(self) -> None:
         """Verification stage alone on the packed correspondences of the last batch (bench.py times it in isolation)."""
@@ -277,7 +299,7 @@ class HotPathPlan:
         if o.P == 0:
             return
         _lib.check(_lib.lib().sfm_ransac_f_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), o.P, self.cap, _lib.ptr(o.pair_id), None,
-                                                  C.byref(self.rprm), _lib.ptr(o.F), _lib.ptr(o.ninl), _lib.ptr(o.mask),
+                                                  C.byref(self.rprm), _lib.ptr(o.F), _lib.ptr(o.n_inliers), _lib.ptr(o.inlier),
                                                   _lib.ptr(o.iters), _lib.current_stream_ptr(self.dev)), "sfm_ransac_f_packed")
 
     # ------------------------------------------------------------------ host results of a job
@@ -285,16 +307,7 @@ class HotPathPlan:
         """Start collecting host results for a job of ``n_pairs`` pairs (any number of batches)."""
         if n_pairs > self._pairs_cap:
             self._pairs_cap = n_pairs
-            self.F_h = torch.zeros((n_pairs, 3, 3), dtype=torch.float64).pin_memory()
-            self.ninl_h = torch.zeros(n_pairs, dtype=torch.int32).pin_memory()
-            self.iters_h = torch.zeros(n_pairs, dtype=torch.int32).pin_memory()
-            if self.homography:
-                self.H_h = torch.zeros((n_pairs, 3, 3), dtype=torch.float64).pin_memory()
-                self.ninlh_h = torch.zeros(n_pairs, dtype=torch.int32).pin_memory()
-            if self.intr is not None:
-                self.R_h = torch.zeros((n_pairs, 3, 3), dtype=torch.float64).pin_memory()
-                self.t_h = torch.zeros((n_pairs, 3), dtype=torch.float64).pin_memory()
-                self.ngood_h = torch.zeros(n_pairs, dtype=torch.int32).pin_memory()
+            self.host.update({o.name: o.empty(n_pairs, pin_memory=True) for o in self._host_pairs})
         self.job_rows = self.job_pairs = self.job_d2h = 0
         self.job_counts = []
 
@@ -302,22 +315,24 @@ class HotPathPlan:
         if rows <= self._rows_cap:
             return
         new_cap = max(rows, expect_total, 2 * self._rows_cap, 1 << 16)
-        m = torch.empty((new_cap, 3), dtype=torch.int32).pin_memory()
-        k = torch.empty(new_cap, dtype=torch.uint8).pin_memory()
-        kh = torch.empty(new_cap, dtype=torch.uint8).pin_memory() if self.homography else None
-        kp = torch.empty(new_cap, dtype=torch.uint8).pin_memory() if self.intr is not None else None
-        x = torch.empty((new_cap, 3), dtype=torch.float32).pin_memory() if self.intr is not None else None
+        grown = {o.name: o.empty(new_cap, pin_memory=True) for o in self._host_rows}
         if self.job_rows:                             # a job in progress outgrew the buffer: keep what has arrived
             self.copy_stream.synchronize()
-            m[: self.job_rows] = self.matches_h[: self.job_rows]
-            k[: self.job_rows] = self.mask_h[: self.job_rows]
-            if kh is not None:
-                kh[: self.job_rows] = self.maskh_h[: self.job_rows]
-            if kp is not None:
-                kp[: self.job_rows] = self.pmask_h[: self.job_rows]
-                x[: self.job_rows] = self.X_h[: self.job_rows]
-        self.matches_h, self.mask_h, self._rows_cap = m, k, new_cap
-        self.maskh_h, self.pmask_h, self.X_h = kh, kp, x
+            for name, h in grown.items():
+                h[: self.job_rows] = self.host[name][: self.job_rows]
+        self.host.update(grown)
+        self._rows_cap = new_cap
+
+    def _offsets(self, out: _OutSet) -> np.ndarray:
+        """Batch ``out``'s packed offsets on the host: the only host wait, until its filter has finished (RANSAC keeps the GPU
+        busy meanwhile)."""
+        P, cs = out.P, self.copy_stream
+        with torch.cuda.stream(cs):
+            cs.wait_event(out.ev_filter)
+            out.offsets_h[: P + 1].copy_(out.offsets[: P + 1], non_blocking=True)
+            out.ev_offsets.record(cs)
+        out.ev_offsets.synchronize()
+        return out.offsets_h[: P + 1].numpy()
 
     def fetch_begin(self, out: _OutSet, pairs_left_after: int = 0) -> None:
         """Enqueue the device -> pinned-host copies of batch ``out`` on the side stream, appending to the job's arrays.
@@ -326,45 +341,26 @@ class HotPathPlan:
         P = out.P
         if P == 0:
             return
-        cs = self.copy_stream
-        with torch.cuda.stream(cs):
-            cs.wait_event(out.ev_filter)
-            out.offsets_h[: P + 1].copy_(out.offsets[: P + 1], non_blocking=True)
-            out.ev_offsets.record(cs)
-        out.ev_offsets.synchronize()                  # filter finished; RANSAC keeps the GPU busy meanwhile
-        off = out.offsets_h[: P + 1].numpy()
+        off = self._offsets(out)
         total = int(off[P])
         r0, p0 = self.job_rows, self.job_pairs
         per_pair = (r0 + total) / max(p0 + P, 1)
         self._ensure_rows(r0 + total, int(1.1 * per_pair * (p0 + P + pairs_left_after)) + 1024)
+        cs = self.copy_stream
         with torch.cuda.stream(cs):
-            if total:
-                self.matches_h[r0: r0 + total].copy_(out.matches[:total], non_blocking=True)
-            cs.wait_event(out.ev_done)
-            if total:
-                self.mask_h[r0: r0 + total].copy_(out.mask[:total], non_blocking=True)
-            self.F_h[p0: p0 + P].copy_(out.F[:P], non_blocking=True)
-            self.ninl_h[p0: p0 + P].copy_(out.ninl[:P], non_blocking=True)
-            self.iters_h[p0: p0 + P].copy_(out.iters[:P], non_blocking=True)
-            if self.homography:
-                if total:
-                    self.maskh_h[r0: r0 + total].copy_(out.mask_h[:total], non_blocking=True)
-                self.H_h[p0: p0 + P].copy_(out.H[:P], non_blocking=True)
-                self.ninlh_h[p0: p0 + P].copy_(out.ninl_h[:P], non_blocking=True)
-                self.job_d2h += total + P * 76
-            if self.intr is not None:
-                if total:
-                    self.pmask_h[r0: r0 + total].copy_(out.pmask[:total], non_blocking=True)
-                    self.X_h[r0: r0 + total].copy_(out.X[:total], non_blocking=True)
-                self.R_h[p0: p0 + P].copy_(out.R[:P], non_blocking=True)
-                self.t_h[p0: p0 + P].copy_(out.t[:P], non_blocking=True)
-                self.ngood_h[p0: p0 + P].copy_(out.ngood[:P], non_blocking=True)
-                self.job_d2h += total * 13 + P * 100
+            for ready, ev in (("filter", None), ("done", out.ev_done)):
+                if ev is not None:
+                    cs.wait_event(ev)
+                for o in self._host_rows:
+                    if o.ready == ready and total:
+                        self.host[o.name][r0: r0 + total].copy_(getattr(out, o.name)[:total], non_blocking=True)
+            for o in self._host_pairs:
+                self.host[o.name][p0: p0 + P].copy_(getattr(out, o.name)[:P], non_blocking=True)
             out.ev_copied.record(cs)
         out.copy_pending = True
         self.job_counts.append(np.diff(off).astype(np.int32))
         self.job_rows, self.job_pairs = r0 + total, p0 + P
-        self.job_d2h += 4 * (P + 1) + total * 13 + P * (72 + 4 + 4)
+        self.job_d2h += 4 * (P + 1) + total * self._row_bytes + P * self._pair_bytes
 
     def push_begin(self, out: _OutSet, sink: RowSink) -> None:
         """Device-side twin of ``fetch_begin``: append batch ``out``'s packed rows to ``sink`` (local or peer memory) with
@@ -374,36 +370,29 @@ class HotPathPlan:
         P = out.P
         if P == 0:
             return
-        L, cs = _lib.lib(), self.copy_stream
-        with torch.cuda.stream(cs):
-            cs.wait_event(out.ev_filter)
-            out.offsets_h[: P + 1].copy_(out.offsets[: P + 1], non_blocking=True)
-            out.ev_offsets.record(cs)
-        out.ev_offsets.synchronize()
-        total = int(out.offsets_h[P])
+        total = int(self._offsets(out)[P])
         r0 = sink.rows
         if r0 + total > sink.cap_rows:
             raise _lib.SfmError(f"row sink overflow: {r0 + total} rows exceed the region's capacity {sink.cap_rows}")
-        src = {"matches": out.matches, "inlier": out.mask, "inlier_h": out.mask_h, "in_front": out.pmask, "points3d": out.X}
+        L, cs = _lib.lib(), self.copy_stream
         st = C.c_void_p(cs.cuda_stream)
         if sink.ready_event is not None:              # the consumer of the previous job's rows has finished with the region
             cs.wait_event(sink.ready_event)
             sink.ready_event = None
-        early = [n for n in sink.fields if n == "matches"]
-        late = [n for n in sink.fields if n != "matches"]
-        for group, ev in ((early, None), (late, out.ev_done)):
+        for ready, ev in (("filter", None), ("done", out.ev_done)):
             if ev is not None:
                 cs.wait_event(ev)
-            for name in group:
-                rb = RowSink.ROW_BYTES[name]
-                if src[name] is None:
+            for name in sink.fields:
+                if OUTPUTS[name].ready != ready:
+                    continue
+                src = getattr(out, name, None)
+                if src is None:
                     raise ValueError(f"the plan does not produce {name!r} (request the stage that does)")
+                rb = RowSink.ROW_BYTES[name]
                 if total:
-                    _lib.check(L.sfm_copy_async(C.c_void_p(sink.fields[name] + r0 * rb), _lib.ptr(src[name]), total * rb, st),
+                    _lib.check(L.sfm_copy_async(C.c_void_p(sink.fields[name] + r0 * rb), _lib.ptr(src), total * rb, st),
                                "sfm_copy_async")
                     sink.bytes += total * rb
-        if not late:
-            cs.wait_event(out.ev_done)
         out.ev_copied.record(cs)
         out.copy_pending = True
         sink.rows, sink.pairs = r0 + total, sink.pairs + P
@@ -415,18 +404,8 @@ class HotPathPlan:
         n_matches = np.concatenate(self.job_counts) if self.job_counts else np.zeros(0, np.int32)
         offsets = np.zeros(P + 1, np.int64)
         np.cumsum(n_matches, out=offsets[1:])
-        if P == 0:
-            return {"n_matches": n_matches, "offsets": offsets, "matches": np.zeros((0, 3), np.int32), "inlier": np.zeros(0, np.uint8),
-                    "F": np.zeros((0, 3, 3)), "n_inliers": np.zeros(0, np.int32), "iters": np.zeros(0, np.int32)}
-        out = {"n_matches": n_matches, "offsets": offsets,
-               "matches": self.matches_h[:rows].numpy() if rows else np.zeros((0, 3), np.int32),
-               "inlier": self.mask_h[:rows].numpy() if rows else np.zeros(0, np.uint8),
-               "F": self.F_h[:P].numpy(), "n_inliers": self.ninl_h[:P].numpy(), "iters": self.iters_h[:P].numpy()}
-        if self.homography:
-            out.update(H=self.H_h[:P].numpy(), n_inliers_h=self.ninlh_h[:P].numpy(),
-                       inlier_h=self.maskh_h[:rows].numpy() if rows else np.zeros(0, np.uint8))
-        if self.intr is not None:
-            out.update(R=self.R_h[:P].numpy(), t=self.t_h[:P].numpy(), n_pose=self.ngood_h[:P].numpy(),
-                       in_front=self.pmask_h[:rows].numpy() if rows else np.zeros(0, np.uint8),
-                       points3d=self.X_h[:rows].numpy() if rows else np.zeros((0, 3), np.float32))
+        out = {"n_matches": n_matches, "offsets": offsets}
+        for o in self._host_rows + self._host_pairs:
+            n = rows if o.per == "row" else P
+            out[o.name] = self.host[o.name][:n].numpy() if n else o.empty(0).numpy()
         return out

@@ -19,7 +19,7 @@ pairs = synth.exhaustive_pairs(n_img)
 bank = sfm_b200.DescriptorBank(n_img, 8192)
 bank.put(0, sc.desc, xy=sc.xy)
 R = dict(thr=3.0, confidence=0.99, max_iters=2000, solver="8pt", score="sym_epipolar", lo=False, seed=1)
-plan = sfm_b200.get_plan(bank, min(2048, len(pairs)), ratio=0.75, ratio_mode="cv2_f32", mutual=False, impl="auto", min_inliers=0,
+plan = sfm_b200.get_plan(bank, min(2048, len(pairs)), ratio=0.75, ratio_mode="cv2_f32", mutual=False, min_inliers=0,
                          prefilter=True, overlap=False, **R)        # stages timed one by one on one stream
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 L, dev = _lib.lib(), bank.device
