@@ -4,30 +4,18 @@
 // code/pipeline.py:60) with the conventions of cv2.findFundamentalMat(FM_RANSAC): x2^T F x1 = 0,
 // F[8] normalised to 1, uint8 inlier mask, inlier iff max(d1^2, d2^2) <= thr^2 (SURVEY.md A.4).
 //
-// One CTA (256 threads) per image pair.  Correspondences are staged once into shared memory as
-// float4 (x1,y1,x2,y2).  Hypotheses are processed in batches of 32, 32, 64, then 128 (ransac_batch):
-//   solve   A: 8 lanes per minimal sample (one matrix row per lane, in registers): Hartley normalisation and the
-//              Gauss-Jordan null space with complete pivoting (fp64, pivot search / row broadcast by shuffles)
-//           B: one thread per sample: rank-2 projection (8-point) or cubic in the pencil (7-point, <= 3 models)
-//   score   one warp per group of 4 models: every lane streams correspondences with 128-bit shared
-//           loads and scores all 4 models (fp32, division-free), lane counts reduced with shuffles
-//   select  strict-greater argmax in (hypothesis, root) order, then the adaptive stop rule
-// followed by an optional LO step (normalised 8-point refit on the inliers, fixed-order fp64
-// reductions) and the final mask.  Every floating-point operation is IEEE basic arithmetic in a fixed
-// order (explicit fma only), so masks and counts are bit-identical to oracle/ransac_f.c, which tests/
-// use as the checker.
+// The kernel body is ransac_driver (ransac_common.cuh).  This file supplies the fundamental-matrix model:
+//   solve   A: one epipolar row per lane, 9 - m null vectors (m = 7 or 8 sample points)
+//           B: rank-2 projection (8-point) or cubic in the pencil (7-point, <= 3 models)
+//   score   symmetric epipolar distance (cv2) or Sampson
+//   LO      normalised 8-point refit on the inliers, rank 2 enforced
+// Every floating-point operation is IEEE basic arithmetic in a fixed order (explicit fma only), so masks and counts are
+// bit-identical to oracle/ransac_f.c, which tests/ use as the checker.
 #include <math.h>
-
-#include <type_traits>
 
 #include "ransac_common.cuh"
 
 namespace sfm {
-
-constexpr int kBatch = 128;
-constexpr int kMaxModels = kBatch * 3;
-constexpr int kLoRounds = 2;
-constexpr int kGroup = 4;
 
 __device__ double det3(const double* r0, const double* r1, const double* r2)
 {
@@ -143,45 +131,15 @@ __device__ int solve_cubic(double c3, double c2, double c1, double c0, double* r
 template <int M>
 static __device__ __forceinline__ bool solve_null_space(const Pts& pts, const int* idx, int sl, unsigned gmask, double* out)
 {
-    double x1[M], y1[M], x2[M], y2[M];
-#pragma unroll
-    for (int k = 0; k < M; ++k) {
-        const float4 c = pts[idx[k]];
-        x1[k] = (double)c.x; y1[k] = (double)c.y; x2[k] = (double)c.z; y2[k] = (double)c.w;
-    }
     Norm2d n1, n2;
-    double sx = 0.0, sy = 0.0, tx = 0.0, ty = 0.0;
-#pragma unroll
-    for (int k = 0; k < M; ++k) { sx += x1[k]; sy += y1[k]; tx += x2[k]; ty += y2[k]; }
-    const double inv = 1.0 / (double)M;
-    n1.cx = sx * inv; n1.cy = sy * inv; n2.cx = tx * inv; n2.cy = ty * inv;
-    double d1 = 0.0, d2 = 0.0;
-#pragma unroll
-    for (int k = 0; k < M; ++k) {
-        const double ax = x1[k] - n1.cx, ay = y1[k] - n1.cy;
-        const double bx = x2[k] - n2.cx, by = y2[k] - n2.cy;
-        d1 += sqrt(ax * ax + ay * ay);
-        d2 += sqrt(bx * bx + by * by);
-    }
-    d1 *= inv; d2 *= inv;
-    if (!(d1 > 1e-9) || !(d2 > 1e-9)) return false;
-    n1.s = 1.4142135623730951 / d1;
-    n2.s = 1.4142135623730951 / d2;
-    double mx1 = x1[0], my1 = y1[0], mx2 = x2[0], my2 = y2[0];            // this lane's sample point
-#pragma unroll
-    for (int k = 1; k < M; ++k)
-        if (sl == k) { mx1 = x1[k]; my1 = y1[k]; mx2 = x2[k]; my2 = y2[k]; }
-    const double u1 = (mx1 - n1.cx) * n1.s, v1 = (my1 - n1.cy) * n1.s;
-    const double u2 = (mx2 - n2.cx) * n2.s, v2 = (my2 - n2.cy) * n2.s;
+    double u1, v1, u2, v2;                                                 // this lane's sample point
+    if (!hartley_sample<M>(pts, idx, sl, n1, n2, u1, v1, u2, v2)) return false;
     double a[9] = {u2 * u1, u2 * v1, u2, v2 * u1, v2 * v1, v2, u1, v1, 1.0};
     CoopGJ st;
     if (!coop_gauss_jordan<M>(a, sl, gmask, 1e-12, st)) return false;
 #pragma unroll
     for (int c = 0; c < 9 - M; ++c) coop_null_vector<M>(a, sl, st, c, out + 9 * c);
-    if (sl == 0) {
-        out[18] = n1.s; out[19] = n1.cx; out[20] = n1.cy;
-        out[21] = n2.s; out[22] = n2.cx; out[23] = n2.cy;
-    }
+    if (sl == 0) store_norms(out, n1, n2);
     return true;
 }
 
@@ -191,8 +149,7 @@ static __device__ int models_from_null_space(const double* in, int m, double* Fo
     double N[2][9];
     for (int i = 0; i < 9; ++i) { N[0][i] = in[i]; N[1][i] = in[9 + i]; }
     Norm2d n1, n2;
-    n1.s = in[18]; n1.cx = in[19]; n1.cy = in[20];
-    n2.s = in[21]; n2.cx = in[22]; n2.cy = in[23];
+    load_norms(in, n1, n2);
     if (m == 8) {
         double Fh[9];
         for (int i = 0; i < 9; ++i) Fh[i] = N[0][i];
@@ -234,304 +191,68 @@ __device__ __forceinline__ bool is_inlier(const float (&F)[9], const float4 c, f
     return n2 <= lim;
 }
 
-struct RansacSmem {
-    double modelD[kMaxModels * 9];
-    double bestF[9];
-    double trialF[9];
-    double wsum[kRansacThreads / 32];
-    float modelF[kMaxModels * 9];
-    int nm[kBatch];
-    int list[kMaxModels];
-    int cnt[kMaxModels];
-    int total, best, stop, ok;
-};
+struct FundamentalModel {
+    static constexpr const char* kName = "sfm_ransac_f";
+    static constexpr int kMaxSample = 8, kRoots = 3, kLoMin = 8;           // LO needs 8 inliers for the 7-point solver too
+    static constexpr bool kSampleInPhaseB = false;
 
-__device__ int block_count_inliers(const double* Fd, const Pts& pts, int M, float thr2, int score,
-                                   uint8_t* __restrict__ mask, int* scratch)
-{
-    float F[9];
-    for (int i = 0; i < 9; ++i) F[i] = (float)Fd[i];
-    int n = 0;
-    for (int i = threadIdx.x; i < M; i += kRansacThreads) {
-        const bool in = is_inlier(F, pts[i], thr2, score);
-        if (mask) mask[i] = (uint8_t)in;
-        n += in;
+    static int check(const sfm_ransac_params& prm)
+    {
+        SFM_REQUIRE(prm.solver == SFM_SOLVER_7PT || prm.solver == SFM_SOLVER_8PT, "solver must be 7 or 8, got %d", prm.solver);
+        SFM_REQUIRE(prm.score == SFM_SCORE_SYM_EPIPOLAR || prm.score == SFM_SCORE_SAMPSON, "unknown score %d", prm.score);
+        return SFM_OK;
     }
-    for (int off = 16; off >= 1; off >>= 1) n += __shfl_down_sync(0xffffffffu, n, off);
-    __syncthreads();
-    if (threadIdx.x == 0) *scratch = 0;
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) atomicAdd(scratch, n);
-    __syncthreads();
-    return *scratch;
-}
+    static __device__ __forceinline__ int sample_size(const sfm_ransac_params& prm) { return prm.solver; }
+    static __device__ __forceinline__ bool null_space(const Pts& pts, const int* idx, int m, int sl, unsigned gmask, double* out)
+    {
+        return (m == 8) ? solve_null_space<8>(pts, idx, sl, gmask, out) : solve_null_space<7>(pts, idx, sl, gmask, out);
+    }
+    static __device__ __forceinline__ int models(const double* in, int m, const Pts&, const int*, double* out)
+    {
+        return models_from_null_space(in, m, out);
+    }
+    static __device__ __forceinline__ bool inlier(const float (&F)[9], const float4 c, float thr2, int score)
+    {
+        return is_inlier(F, c, thr2, score);
+    }
+    // one epipolar row r per inlier: r (x) r
+    static __device__ __forceinline__ void lo_rows(double (&acc)[45], double u1, double v1, double u2, double v2)
+    {
+        const double r[9] = {u2 * u1, u2 * v1, u2, v2 * u1, v2 * v1, v2, u1, v1, 1.0};
+        int e = 0;
+#pragma unroll
+        for (int a = 0; a < 9; ++a)
+#pragma unroll
+            for (int b = a; b < 9; ++b) acc[e++] += r[a] * r[b];
+    }
+    static __device__ __forceinline__ int refit(double* Fh, Norm2d n1, Norm2d n2, double* F)
+    {
+        enforce_rank2(Fh);
+        return denormalise(Fh, n1, n2, F);
+    }
+};
 
 __global__ void __launch_bounds__(kRansacThreads, 2) ransac_f_kernel(
     const float* __restrict__ corr, int corr_stride, const int32_t* __restrict__ count, const int32_t* __restrict__ offsets,
-    const uint32_t* __restrict__ pair_id, const uint32_t* __restrict__ samples, sfm_ransac_params prm, int pts_cap,
-    double* __restrict__ out_F, int32_t* __restrict__ out_ninl, uint8_t* __restrict__ out_mask, int32_t* __restrict__ out_iters)
+    const uint32_t* __restrict__ pair_id, const uint32_t* __restrict__ samples, const int32_t* __restrict__ /* stop_target */,
+    sfm_ransac_params prm, int pts_cap, double* __restrict__ out_F, int32_t* __restrict__ out_ninl, uint8_t* __restrict__ out_mask,
+    int32_t* __restrict__ out_iters)
 {
-    extern __shared__ __align__(16) uint8_t smem_raw[];
-    RansacSmem& S = *reinterpret_cast<RansacSmem*>(smem_raw);
-    float4* spts = reinterpret_cast<float4*>(smem_raw + ((sizeof(RansacSmem) + 15) & ~(size_t)15));
-
-    const int p = blockIdx.x;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    // strided layout: pair p owns rows [p * corr_stride, +count[p]); packed layout: rows [offsets[p], offsets[p+1])
-    const long long base = offsets ? (long long)offsets[p] : (long long)p * corr_stride;
-    const int M = offsets ? (offsets[p + 1] - offsets[p]) : min(count[p], corr_stride);
-    const int m = prm.solver;
-    const float thr2 = prm.threshold * prm.threshold;
-    uint8_t* mask = out_mask + base;
-    const float4* gpts = reinterpret_cast<const float4*>(corr) + base;
-
-    for (int i = tid; i < (offsets ? M : corr_stride); i += kRansacThreads) mask[i] = 0;
-    if (tid < 9) out_F[(long long)p * 9 + tid] = 0.0;
-    if (tid == 0) { out_ninl[p] = 0; if (out_iters) out_iters[p] = 0; S.best = 0; S.stop = 0; }
-    if (M < m) return;
-
-    for (int i = tid; i < min(M, pts_cap); i += kRansacThreads) spts[i] = gpts[i];
-    const Pts pts{spts, gpts, pts_cap};
-    const uint32_t pid = pair_id ? pair_id[p] : (uint32_t)p;
-    __syncthreads();
-
-    int done = 0;
-    while (done < prm.max_iters) {
-        const int nb = min(ransac_batch(done), prm.max_iters - done);
-        // ---- solve, phase A: 8 lanes per hypothesis, 32 hypotheses per round -> null spaces in shared memory (S.modelD)
-        {
-            const int sl = tid & 7;
-            const unsigned gmask = 0xFFu << (lane & 24);
-            for (int h = tid >> 3; h < kBatch; h += kRansacThreads / 8) {
-                bool ok = false;
-                if (h < nb) {
-                    int idx[8];
-                    if (samples) {
-                        for (int k = 0; k < m; ++k) idx[k] = (int)(samples[(size_t)(done + h) * 8 + k] % (uint32_t)M);
-                    } else {
-                        draw_sample(prm.seed, pid, (uint32_t)(done + h), m, M, idx);
-                    }
-                    double* out = S.modelD + h * 24;
-                    ok = (m == 8) ? solve_null_space<8>(pts, idx, sl, gmask, out) : solve_null_space<7>(pts, idx, sl, gmask, out);
-                }
-                if (sl == 0) S.nm[h] = ok ? 1 : 0;
-            }
-        }
-        __syncthreads();
-        // ---- solve, phase B: one thread per hypothesis finishes its models in registers, then all of them are published
-        {
-            double Fm[27];
-            int n = 0;
-            if (tid < kBatch && S.nm[tid]) n = models_from_null_space(S.modelD + tid * 24, m, Fm);
-            __syncthreads();
-            if (tid < kBatch) {
-                for (int r = 0; r < n; ++r)
-                    for (int i = 0; i < 9; ++i) {
-                        S.modelD[(tid * 3 + r) * 9 + i] = Fm[9 * r + i];
-                        S.modelF[(tid * 3 + r) * 9 + i] = (float)Fm[9 * r + i];
-                    }
-                S.nm[tid] = n;
-            }
-        }
-        __syncthreads();
-        if (tid < kBatch) {
-            int off = 0;
-            for (int j = 0; j < tid; ++j) off += S.nm[j];
-            for (int r = 0; r < S.nm[tid]; ++r) S.list[off + r] = tid * 3 + r;
-            if (tid == kBatch - 1) S.total = off + S.nm[tid];
-        }
-        __syncthreads();
-        // ---- score: a warp takes 4 models at a time and streams every correspondence once for all of them
-        const int total = S.total;
-        for (int g = warp * kGroup; g < total; g += (kRansacThreads / 32) * kGroup) {
-            float F[kGroup][9];
-            int c[kGroup];
-#pragma unroll
-            for (int j = 0; j < kGroup; ++j) {
-                const int slot = S.list[min(g + j, total - 1)];
-#pragma unroll
-                for (int i = 0; i < 9; ++i) F[j][i] = S.modelF[slot * 9 + i];
-                c[j] = 0;
-            }
-            // the next correspondence is loaded before the current one is scored: the shared-memory latency hides behind
-            // the ~100 arithmetic instructions of the four models
-            float4 nx = pts[min(lane, M - 1)];
-            // exact bail-out: once none of the four models can still EXCEED the best count of the earlier batches (their
-            // counts so far + every correspondence not yet seen), the rest of the stream is skipped.  The partial counts stay
-            // <= that best, so the strict-greater selection -- and therefore the result -- is unchanged.
-            const int best_prev = S.best;
-            const bool can_bail = best_prev * 4 > M;
-            auto stream = [&](auto bail_c) {
-                constexpr bool kBail = decltype(bail_c)::value;
-                int next_check = lane + 32 * kBailEvery;
-                for (int i = lane; i < M; i += 32) {
-                    const float4 pt = nx;
-                    nx = pts[min(i + 32, M - 1)];
-#pragma unroll
-                    for (int j = 0; j < kGroup; ++j) c[j] += is_inlier(F[j], pt, thr2, prm.score);
-                    if (kBail && i + 32 == next_check) {
-                        next_check += 32 * kBailEvery;
-                        const int left = M - (i - lane + 32);               // correspondences no lane has looked at yet
-                        if (left <= 0) return;                               // (uniform: every lane was active in this iteration iff left >= 0)
-                        int top = 0;
-#pragma unroll
-                        for (int j = 0; j < kGroup; ++j) {
-                            int v = c[j];
-                            for (int off = 16; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-                            top = max(top, v);
-                        }
-                        if (top + left <= best_prev) return;
-                    }
-                }
-            };
-            if (can_bail) stream(std::true_type{}); else stream(std::false_type{});      // no bail-out code in the common first batches
-#pragma unroll
-            for (int j = 0; j < kGroup; ++j) {
-                int v = c[j];
-                for (int off = 16; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-                if (lane == 0 && g + j < total) S.cnt[g + j] = v;
-            }
-        }
-        __syncthreads();
-        // ---- select (strict >, list order = (hypothesis, root) ascending) and stop rule
-        if (tid == 0) {
-            int best = S.best, arg = -1;
-            for (int k = 0; k < total; ++k)
-                if (S.cnt[k] > best) { best = S.cnt[k]; arg = k; }
-            if (arg >= 0) {
-                S.best = best;
-                for (int i = 0; i < 9; ++i) S.bestF[i] = S.modelD[S.list[arg] * 9 + i];
-            }
-            S.stop = should_stop(S.best, M, m, done + nb, prm.confidence) ? 1 : 0;
-        }
-        __syncthreads();
-        done += nb;
-        if (S.stop) break;
-    }
-    if (tid == 0 && out_iters) out_iters[p] = done;
-    if (S.best < m) return;
-
-    int best = block_count_inliers(S.bestF, pts, M, thr2, prm.score, mask, &S.total);
-    if (prm.lo_refit) {
-        for (int round = 0; round < kLoRounds; ++round) {
-            __syncthreads();
-            // moments of the inliers (fixed lane order)
-            double* red_part = S.modelD + 256;   // scratch of the batched reductions: 45 * 8 partials + 45 totals (AtA and the
-            double* red_tot = red_part + 45 * 8;  // eigen-solver's scratch live below 256)
-            double mom[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
-            for (int i = tid; i < M; i += kRansacThreads)
-                if (mask[i]) {
-                    const float4 c = pts[i];
-                    mom[0] += (double)c.x; mom[1] += (double)c.y; mom[2] += (double)c.z; mom[3] += (double)c.w; mom[4] += 1.0;
-                }
-            block_tree_sum_many<5>(mom, red_part, red_tot);
-            if (!(mom[4] >= 8.0)) break;
-            Norm2d n1, n2;
-            const double inv = 1.0 / mom[4];
-            n1.cx = mom[0] * inv; n1.cy = mom[1] * inv; n2.cx = mom[2] * inv; n2.cy = mom[3] * inv;
-            double dd[2] = {0.0, 0.0};
-            for (int i = tid; i < M; i += kRansacThreads)
-                if (mask[i]) {
-                    const float4 c = pts[i];
-                    const double ax = (double)c.x - n1.cx, ay = (double)c.y - n1.cy;
-                    const double bx = (double)c.z - n2.cx, by = (double)c.w - n2.cy;
-                    dd[0] += sqrt(ax * ax + ay * ay);
-                    dd[1] += sqrt(bx * bx + by * by);
-                }
-            block_tree_sum_many<2>(dd, red_part, red_tot);
-            dd[0] *= inv; dd[1] *= inv;
-            if (!(dd[0] > 1e-9) || !(dd[1] > 1e-9)) break;
-            n1.s = 1.4142135623730951 / dd[0];
-            n2.s = 1.4142135623730951 / dd[1];
-            double acc[45];
-#pragma unroll
-            for (int e = 0; e < 45; ++e) acc[e] = 0.0;
-            for (int i = tid; i < M; i += kRansacThreads)
-                if (mask[i]) {
-                    const float4 c = pts[i];
-                    const double u1 = ((double)c.x - n1.cx) * n1.s, v1 = ((double)c.y - n1.cy) * n1.s;
-                    const double u2 = ((double)c.z - n2.cx) * n2.s, v2 = ((double)c.w - n2.cy) * n2.s;
-                    const double r[9] = {u2 * u1, u2 * v1, u2, v2 * u1, v2 * v1, v2, u1, v1, 1.0};
-                    int e = 0;
-#pragma unroll
-                    for (int a = 0; a < 9; ++a)
-#pragma unroll
-                        for (int b = a; b < 9; ++b) acc[e++] += r[a] * r[b];
-                }
-            double* AtA = S.modelD;              // 81 doubles; the eigen-solver's scratch follows
-            block_tree_sum_many<45>(acc, red_part, red_tot);
-            if (tid == 0) {
-                int e = 0;
-                for (int a = 0; a < 9; ++a)
-                    for (int b = a; b < 9; ++b) { AtA[a * 9 + b] = acc[e]; AtA[b * 9 + a] = acc[e]; ++e; }
-            }
-            __syncthreads();
-            if (tid == 0) {
-                double Fh[9];
-                S.ok = smallest_eigvec9(AtA, S.modelD + 81, Fh);
-                if (S.ok) {
-                    enforce_rank2(Fh);
-                    S.ok = denormalise(Fh, n1, n2, S.trialF);
-                }
-            }
-            __syncthreads();
-            if (!S.ok) break;
-            const int cnt = block_count_inliers(S.trialF, pts, M, thr2, prm.score, nullptr, &S.total);
-            if (cnt <= best) break;
-            best = cnt;
-            if (tid < 9) S.bestF[tid] = S.trialF[tid];
-            __syncthreads();
-            block_count_inliers(S.bestF, pts, M, thr2, prm.score, mask, &S.total);
-        }
-    }
-    __syncthreads();
-    if (prm.min_inliers > 0 && best < prm.min_inliers) {
-        for (int i = tid; i < M; i += kRansacThreads) mask[i] = 0;
-        return;
-    }
-    if (tid == 0) {
-        // cv2 convention F[2,2] == 1.0 exactly: divide (x / x == 1), never multiply by a reciprocal
-        const double s = (fabs(S.bestF[8]) > 1.1920928955078125e-07) ? S.bestF[8] : 1.0;
-        for (int i = 0; i < 9; ++i) out_F[(long long)p * 9 + i] = S.bestF[i] / s;
-        out_ninl[p] = best;
-    }
+    ransac_driver<FundamentalModel>(corr, corr_stride, count, offsets, pair_id, samples, nullptr, prm, pts_cap, out_F, out_ninl,
+                                    out_mask, out_iters);
 }
 
 }  // namespace sfm
 
 using namespace sfm;
 
-static int launch_ransac(const float* corr, int corr_stride, const int32_t* count, const int32_t* offsets, int n_pairs,
-                         const uint32_t* pair_id, const uint32_t* samples, const sfm_ransac_params* prm, double* out_F,
-                         int32_t* out_ninl, uint8_t* out_mask, int32_t* out_iters, void* stream)
-{
-    SFM_REQUIRE(corr && (count || offsets) && prm && out_F && out_ninl && out_mask, "sfm_ransac_f: NULL argument");
-    SFM_REQUIRE(prm->solver == SFM_SOLVER_7PT || prm->solver == SFM_SOLVER_8PT, "solver must be 7 or 8, got %d", prm->solver);
-    SFM_REQUIRE(prm->score == SFM_SCORE_SYM_EPIPOLAR || prm->score == SFM_SCORE_SAMPSON, "unknown score %d", prm->score);
-    SFM_REQUIRE(prm->max_iters > 0 && prm->threshold > 0.f, "max_iters and threshold must be positive");
-    SFM_REQUIRE(corr_stride > 0 && n_pairs >= 0, "bad sizes");
-    SFM_REQUIRE(((uintptr_t)corr & 15) == 0, "corr must be 16-byte aligned");
-    if (n_pairs == 0) return SFM_OK;
-    // up to kPtsCap correspondences per pair live in shared memory (2 CTAs per SM); wider pairs read the tail through L1/L2
-    constexpr int kPtsCap = 4096;
-    const int pts_cap = corr_stride < kPtsCap ? corr_stride : kPtsCap;
-    const size_t fixed = (sizeof(RansacSmem) + 15) & ~(size_t)15;
-    const size_t smem = fixed + (size_t)pts_cap * 16;
-    static SmemAttrTable attr;                               // per device; these entry points run on the caller's current device
-    SFM_CUDA_CHECK(ensure_dyn_smem(ransac_f_kernel, smem, current_device(), attr));
-    ransac_f_kernel<<<n_pairs, kRansacThreads, smem, (cudaStream_t)stream>>>(corr, corr_stride, count, offsets, pair_id, samples, *prm,
-                                                                            pts_cap, out_F, out_ninl, out_mask, out_iters);
-    SFM_CUDA_CHECK(cudaGetLastError());
-    count_launch();
-    return SFM_OK;
-}
-
 extern "C" int sfm_ransac_f_batch(const float* corr, int corr_stride, const int32_t* count, int n_pairs, const uint32_t* pair_id,
                                   const uint32_t* samples, const sfm_ransac_params* prm, double* out_F, int32_t* out_ninl,
                                   uint8_t* out_mask, int32_t* out_iters, void* stream)
 {
     SFM_REQUIRE(count != nullptr, "sfm_ransac_f_batch: NULL argument");
-    return launch_ransac(corr, corr_stride, count, nullptr, n_pairs, pair_id, samples, prm, out_F, out_ninl, out_mask, out_iters, stream);
+    return launch_ransac<FundamentalModel>(ransac_f_kernel, corr, corr_stride, count, nullptr, n_pairs, pair_id, samples, nullptr, prm,
+                                           out_F, out_ninl, out_mask, out_iters, stream);
 }
 
 extern "C" int sfm_ransac_f_packed(const float* corr, const int32_t* offsets, int n_pairs, int max_count, const uint32_t* pair_id,
@@ -539,5 +260,6 @@ extern "C" int sfm_ransac_f_packed(const float* corr, const int32_t* offsets, in
                                    uint8_t* out_mask, int32_t* out_iters, void* stream)
 {
     SFM_REQUIRE(offsets != nullptr, "sfm_ransac_f_packed: NULL argument");
-    return launch_ransac(corr, max_count, nullptr, offsets, n_pairs, pair_id, samples, prm, out_F, out_ninl, out_mask, out_iters, stream);
+    return launch_ransac<FundamentalModel>(ransac_f_kernel, corr, max_count, nullptr, offsets, n_pairs, pair_id, samples, nullptr, prm,
+                                           out_F, out_ninl, out_mask, out_iters, stream);
 }

@@ -5,24 +5,16 @@
 // H-vs-F inlier ratio classifies the pair for the scene graph.  Conventions follow cv2.findHomography(RANSAC):
 // x2 ~ H x1, H[8] normalised to 1, uint8 inlier mask, inlier iff |proj(H x1) - x2|^2 <= thr^2.
 //
-// Same scaffolding as ransac_f.cu: one CTA (256 threads) per image pair, correspondences staged in shared memory as
-// float4, hypotheses in batches of 32, 32, 64, then 128:
-//   solve   A: 8 lanes per 4-point sample (one row of the 8x9 DLT system per lane, in registers): Hartley
-//              normalisation, Gauss-Jordan null space with complete pivoting (fp64, shuffles)
-//           B: one thread per sample: denormalise; the sample points must keep the sign of the projective depth
-//   score   one warp per group of 4 models, 128-bit shared loads, fp32, division-free
-//   select  strict-greater argmax in hypothesis order, adaptive stop
-// then an optional LO step (normalised DLT on the inliers, fixed-order fp64 reductions, 9x9 Jacobi) and the final mask.
+// The kernel body is ransac_driver (ransac_common.cuh), shared with RANSAC-F.  This file supplies the homography model:
+//   solve   A: 4-point sample, lane r holds row r of the 8 x 9 DLT system (point r / 2, x- or y-equation), one null vector
+//           B: denormalise; the sample points must keep the sign of the projective depth (needs the sample again)
+//   score   forward transfer error
+//   stop    the caller's optional stop target (stop_target)
+//   LO      normalised DLT on the inliers, two rows per inlier
 // Bit-identical to oracle/ransac_h.c.
-#include <type_traits>
-
 #include "ransac_common.cuh"
 
 namespace sfm {
-
-constexpr int kHBatch = 128;
-constexpr int kHGroup = 4;
-constexpr int kHLoRounds = 2;
 
 // H = T2^-1 Hn T1 with T = [s 0 -s*cx; 0 s -s*cy; 0 0 1], scaled to unit Frobenius norm
 static __device__ int denormalise_h(const double* Hn, Norm2d n1, Norm2d n2, double* H)
@@ -54,36 +46,9 @@ static __device__ int denormalise_h(const double* Hn, Norm2d n1, Norm2d n2, doub
 // it cooperatively; out[0..8] = null vector (normalised frame), out[18..23] = n1, n2.
 static __device__ __forceinline__ bool solve_h_null_space(const Pts& pts, const int* idx, int sl, unsigned gmask, double* out)
 {
-    double x1[4], y1[4], x2[4], y2[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const float4 c = pts[idx[k]];
-        x1[k] = (double)c.x; y1[k] = (double)c.y; x2[k] = (double)c.z; y2[k] = (double)c.w;
-    }
     Norm2d n1, n2;
-    double sx = 0.0, sy = 0.0, tx = 0.0, ty = 0.0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) { sx += x1[k]; sy += y1[k]; tx += x2[k]; ty += y2[k]; }
-    n1.cx = sx * 0.25; n1.cy = sy * 0.25; n2.cx = tx * 0.25; n2.cy = ty * 0.25;
-    double d1 = 0.0, d2 = 0.0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const double ax = x1[k] - n1.cx, ay = y1[k] - n1.cy;
-        const double bx = x2[k] - n2.cx, by = y2[k] - n2.cy;
-        d1 += sqrt(ax * ax + ay * ay);
-        d2 += sqrt(bx * bx + by * by);
-    }
-    d1 *= 0.25; d2 *= 0.25;
-    if (!(d1 > 1e-9) || !(d2 > 1e-9)) return false;
-    n1.s = 1.4142135623730951 / d1;
-    n2.s = 1.4142135623730951 / d2;
-    const int pt = sl >> 1;
-    double mx1 = x1[0], my1 = y1[0], mx2 = x2[0], my2 = y2[0];
-#pragma unroll
-    for (int k = 1; k < 4; ++k)
-        if (pt == k) { mx1 = x1[k]; my1 = y1[k]; mx2 = x2[k]; my2 = y2[k]; }
-    const double u1 = (mx1 - n1.cx) * n1.s, v1 = (my1 - n1.cy) * n1.s;
-    const double u2 = (mx2 - n2.cx) * n2.s, v2 = (my2 - n2.cy) * n2.s;
+    double u1, v1, u2, v2;                    // (the 0.25 of the 4-point mean is 1.0 / 4, bit for bit)
+    if (!hartley_sample<4>(pts, idx, sl >> 1, n1, n2, u1, v1, u2, v2)) return false;
     double a[9];
     if (sl & 1) {
         a[0] = 0.0; a[1] = 0.0; a[2] = 0.0; a[3] = u1; a[4] = v1; a[5] = 1.0;
@@ -95,10 +60,7 @@ static __device__ __forceinline__ bool solve_h_null_space(const Pts& pts, const 
     CoopGJ st;
     if (!coop_gauss_jordan<8>(a, sl, gmask, 1e-10, st)) return false;
     coop_null_vector<8>(a, sl, st, 0, out);
-    if (sl == 0) {
-        out[18] = n1.s; out[19] = n1.cx; out[20] = n1.cy;
-        out[21] = n2.s; out[22] = n2.cx; out[23] = n2.cy;
-    }
+    if (sl == 0) store_norms(out, n1, n2);
     return true;
 }
 
@@ -109,8 +71,7 @@ static __device__ int model_from_null_space_h(const double* in, const Pts& pts, 
     double Hn[9];
     for (int i = 0; i < 9; ++i) Hn[i] = in[i];
     Norm2d n1, n2;
-    n1.s = in[18]; n1.cx = in[19]; n1.cy = in[20];
-    n2.s = in[21]; n2.cx = in[22]; n2.cy = in[23];
+    load_norms(in, n1, n2);
     if (!denormalise_h(Hn, n1, n2, Hout)) return 0;
     int pos = 0, neg = 0;
     for (int k = 0; k < 4; ++k) {
@@ -136,307 +97,64 @@ static __device__ __forceinline__ bool is_inlier_h(const float (&H)[9], const fl
     return e2 <= lim && lim > 0.f;
 }
 
-struct RansacHSmem {
-    double nbuf[kHBatch * 24];        // phase A -> B: null vector + the two normalisations per hypothesis
-    double modelD[kHBatch * 9];       // also the 81 + 81 doubles of the LO eigen-problem
-    double bestH[9];
-    double trialH[9];
-    double wsum[kRansacThreads / 32];
-    float modelF[kHBatch * 9];
-    int nm[kHBatch];
-    int list[kHBatch];
-    int cnt[kHBatch];
-    int total, best, stop, ok;
-};
+struct HomographyModel {
+    static constexpr const char* kName = "sfm_ransac_h";
+    static constexpr int kMaxSample = 4, kRoots = 1, kLoMin = 4;
+    static constexpr bool kSampleInPhaseB = true;                          // the orientation check reads the sample points
 
-static __device__ int block_count_inliers_h(const double* Hd, const Pts& pts, int M, float thr2, uint8_t* __restrict__ mask, int* scratch)
-{
-    float H[9];
-    for (int i = 0; i < 9; ++i) H[i] = (float)Hd[i];
-    int n = 0;
-    for (int i = threadIdx.x; i < M; i += kRansacThreads) {
-        const bool in = is_inlier_h(H, pts[i], thr2);
-        if (mask) mask[i] = (uint8_t)in;
-        n += in;
+    static int check(const sfm_ransac_params&) { return SFM_OK; }          // solver and score are not used
+    static __device__ __forceinline__ int sample_size(const sfm_ransac_params&) { return 4; }
+    static __device__ __forceinline__ bool null_space(const Pts& pts, const int* idx, int, int sl, unsigned gmask, double* out)
+    {
+        return solve_h_null_space(pts, idx, sl, gmask, out);
     }
-    for (int off = 16; off >= 1; off >>= 1) n += __shfl_down_sync(0xffffffffu, n, off);
-    __syncthreads();
-    if (threadIdx.x == 0) *scratch = 0;
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) atomicAdd(scratch, n);
-    __syncthreads();
-    return *scratch;
-}
+    static __device__ __forceinline__ int models(const double* in, int, const Pts& pts, const int* idx, double* out)
+    {
+        return model_from_null_space_h(in, pts, idx, out);
+    }
+    static __device__ __forceinline__ bool inlier(const float (&H)[9], const float4 c, float thr2, int)
+    {
+        return is_inlier_h(H, c, thr2);
+    }
+    // the two DLT rows of each inlier
+    static __device__ __forceinline__ void lo_rows(double (&acc)[45], double u1, double v1, double u2, double v2)
+    {
+        const double ra[9] = {u1, v1, 1.0, 0.0, 0.0, 0.0, -(u2 * u1), -(u2 * v1), -u2};
+        const double rb[9] = {0.0, 0.0, 0.0, u1, v1, 1.0, -(v2 * u1), -(v2 * v1), -v2};
+        int e = 0;
+#pragma unroll
+        for (int a = 0; a < 9; ++a)
+#pragma unroll
+            for (int b = a; b < 9; ++b) {
+                acc[e] += ra[a] * ra[b];
+                acc[e] += rb[a] * rb[b];
+                ++e;
+            }
+    }
+    static __device__ __forceinline__ int refit(double* Hn, Norm2d n1, Norm2d n2, double* H) { return denormalise_h(Hn, n1, n2, H); }
+};
 
 __global__ void __launch_bounds__(kRansacThreads, 2) ransac_h_kernel(
     const float* __restrict__ corr, int corr_stride, const int32_t* __restrict__ count, const int32_t* __restrict__ offsets,
     const uint32_t* __restrict__ pair_id, const uint32_t* __restrict__ samples, const int32_t* __restrict__ stop_target,
-    sfm_ransac_params prm, int pts_cap, double* __restrict__ out_H, int32_t* __restrict__ out_ninl, uint8_t* __restrict__ out_mask, int32_t* __restrict__ out_iters)
+    sfm_ransac_params prm, int pts_cap, double* __restrict__ out_H, int32_t* __restrict__ out_ninl, uint8_t* __restrict__ out_mask,
+    int32_t* __restrict__ out_iters)
 {
-    extern __shared__ __align__(16) uint8_t smem_raw[];
-    RansacHSmem& S = *reinterpret_cast<RansacHSmem*>(smem_raw);
-    float4* spts = reinterpret_cast<float4*>(smem_raw + ((sizeof(RansacHSmem) + 15) & ~(size_t)15));
-
-    const int p = blockIdx.x;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const long long base = offsets ? (long long)offsets[p] : (long long)p * corr_stride;
-    const int M = offsets ? (offsets[p + 1] - offsets[p]) : min(count[p], corr_stride);
-    const float thr2 = prm.threshold * prm.threshold;
-    uint8_t* mask = out_mask + base;
-    const float4* gpts = reinterpret_cast<const float4*>(corr) + base;
-
-    for (int i = tid; i < (offsets ? M : corr_stride); i += kRansacThreads) mask[i] = 0;
-    if (tid < 9) out_H[(long long)p * 9 + tid] = 0.0;
-    if (tid == 0) { out_ninl[p] = 0; if (out_iters) out_iters[p] = 0; S.best = 0; S.stop = 0; }
-    if (M < 4) return;
-
-    for (int i = tid; i < min(M, pts_cap); i += kRansacThreads) spts[i] = gpts[i];
-    const Pts pts{spts, gpts, pts_cap};
-    const uint32_t pid = pair_id ? pair_id[p] : (uint32_t)p;
-    const int target = stop_target ? min(max(stop_target[p], 0), M) : 0;
-    __syncthreads();
-
-    int done = 0;
-    while (done < prm.max_iters) {
-        const int nb = min(ransac_batch(done), prm.max_iters - done);
-        // ---- solve, phase A: 8 lanes per hypothesis -> null vectors in shared memory (S.modelD, 24 doubles each)
-        {
-            const int sl = tid & 7;
-            const unsigned gmask = 0xFFu << (lane & 24);
-            for (int h = tid >> 3; h < kHBatch; h += kRansacThreads / 8) {
-                bool ok = false;
-                if (h < nb) {
-                    int idx[4];
-                    if (samples) {
-                        for (int k = 0; k < 4; ++k) idx[k] = (int)(samples[(size_t)(done + h) * 8 + k] % (uint32_t)M);
-                    } else {
-                        draw_sample(prm.seed, pid, (uint32_t)(done + h), 4, M, idx);
-                    }
-                    ok = solve_h_null_space(pts, idx, sl, gmask, S.nbuf + h * 24);
-                }
-                if (sl == 0) S.nm[h] = ok ? 1 : 0;
-            }
-        }
-        __syncthreads();
-        // ---- solve, phase B: one thread per hypothesis
-        if (tid < kHBatch) {
-            int n = 0;
-            if (S.nm[tid]) {
-                int idx[4];
-                if (samples) {
-                    for (int k = 0; k < 4; ++k) idx[k] = (int)(samples[(size_t)(done + tid) * 8 + k] % (uint32_t)M);
-                } else {
-                    draw_sample(prm.seed, pid, (uint32_t)(done + tid), 4, M, idx);
-                }
-                double Hm[9];
-                n = model_from_null_space_h(S.nbuf + tid * 24, pts, idx, Hm);
-                if (n)
-                    for (int i = 0; i < 9; ++i) {
-                        S.modelD[tid * 9 + i] = Hm[i];
-                        S.modelF[tid * 9 + i] = (float)Hm[i];
-                    }
-            }
-            S.nm[tid] = n;
-        }
-        __syncthreads();
-        if (tid < kHBatch) {
-            int off = 0;
-            for (int j = 0; j < tid; ++j) off += S.nm[j];
-            if (S.nm[tid]) S.list[off] = tid;
-            if (tid == kHBatch - 1) S.total = off + S.nm[tid];
-        }
-        __syncthreads();
-        const int total = S.total;
-        for (int g = warp * kHGroup; g < total; g += (kRansacThreads / 32) * kHGroup) {
-            float H[kHGroup][9];
-            int c[kHGroup];
-#pragma unroll
-            for (int j = 0; j < kHGroup; ++j) {
-                const int slot = S.list[min(g + j, total - 1)];
-#pragma unroll
-                for (int i = 0; i < 9; ++i) H[j][i] = S.modelF[slot * 9 + i];
-                c[j] = 0;
-            }
-            // the next correspondence is loaded before the current one is scored: the shared-memory latency hides behind
-            // the ~100 arithmetic instructions of the four models
-            float4 nx = pts[min(lane, M - 1)];
-            // exact bail-out: once none of the four models can still EXCEED the best count of the earlier batches (their
-            // counts so far + every correspondence not yet seen), the rest of the stream is skipped.  The partial counts stay
-            // <= that best, so the strict-greater selection -- and therefore the result -- is unchanged.
-            const int best_prev = S.best;
-            const bool can_bail = best_prev * 4 > M;
-            auto stream = [&](auto bail_c) {
-                constexpr bool kBail = decltype(bail_c)::value;
-                int next_check = lane + 32 * kBailEvery;
-                for (int i = lane; i < M; i += 32) {
-                    const float4 pt = nx;
-                    nx = pts[min(i + 32, M - 1)];
-#pragma unroll
-                    for (int j = 0; j < kHGroup; ++j) c[j] += is_inlier_h(H[j], pt, thr2);
-                    if (kBail && i + 32 == next_check) {
-                        next_check += 32 * kBailEvery;
-                        const int left = M - (i - lane + 32);               // correspondences no lane has looked at yet
-                        if (left <= 0) return;                               // (uniform: every lane was active in this iteration iff left >= 0)
-                        int top = 0;
-#pragma unroll
-                        for (int j = 0; j < kHGroup; ++j) {
-                            int v = c[j];
-                            for (int off = 16; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-                            top = max(top, v);
-                        }
-                        if (top + left <= best_prev) return;
-                    }
-                }
-            };
-            if (can_bail) stream(std::true_type{}); else stream(std::false_type{});      // no bail-out code in the common first batches
-#pragma unroll
-            for (int j = 0; j < kHGroup; ++j) {
-                int v = c[j];
-                for (int off = 16; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-                if (lane == 0 && g + j < total) S.cnt[g + j] = v;
-            }
-        }
-        __syncthreads();
-        if (tid == 0) {
-            int best = S.best, arg = -1;
-            for (int k = 0; k < total; ++k)
-                if (S.cnt[k] > best) { best = S.cnt[k]; arg = k; }
-            if (arg >= 0) {
-                S.best = best;
-                for (int i = 0; i < 9; ++i) S.bestH[i] = S.modelD[S.list[arg] * 9 + i];
-            }
-            // stop_target: the caller only needs to know whether H can reach that support (scene-graph test n_H > r * n_F):
-            // sampling ends once a model with max(best, target) inliers would have been found with the requested confidence
-            S.stop = should_stop(max(S.best, target), M, 4, done + nb, prm.confidence) ? 1 : 0;
-        }
-        __syncthreads();
-        done += nb;
-        if (S.stop) break;
-    }
-    if (tid == 0 && out_iters) out_iters[p] = done;
-    if (S.best < 4) return;
-
-    int best = block_count_inliers_h(S.bestH, pts, M, thr2, mask, &S.total);
-    if (prm.lo_refit) {
-        for (int round = 0; round < kHLoRounds; ++round) {
-            __syncthreads();
-            double* red_part = S.modelD + 256;   // scratch of the batched reductions: 45 * 8 partials + 45 totals (AtA and the
-            double* red_tot = red_part + 45 * 8;  // eigen-solver's scratch live below 256)
-            double mom[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
-            for (int i = tid; i < M; i += kRansacThreads)
-                if (mask[i]) {
-                    const float4 c = pts[i];
-                    mom[0] += (double)c.x; mom[1] += (double)c.y; mom[2] += (double)c.z; mom[3] += (double)c.w; mom[4] += 1.0;
-                }
-            block_tree_sum_many<5>(mom, red_part, red_tot);
-            if (!(mom[4] >= 4.0)) break;
-            Norm2d n1, n2;
-            const double inv = 1.0 / mom[4];
-            n1.cx = mom[0] * inv; n1.cy = mom[1] * inv; n2.cx = mom[2] * inv; n2.cy = mom[3] * inv;
-            double dd[2] = {0.0, 0.0};
-            for (int i = tid; i < M; i += kRansacThreads)
-                if (mask[i]) {
-                    const float4 c = pts[i];
-                    const double ax = (double)c.x - n1.cx, ay = (double)c.y - n1.cy;
-                    const double bx = (double)c.z - n2.cx, by = (double)c.w - n2.cy;
-                    dd[0] += sqrt(ax * ax + ay * ay);
-                    dd[1] += sqrt(bx * bx + by * by);
-                }
-            block_tree_sum_many<2>(dd, red_part, red_tot);
-            dd[0] *= inv; dd[1] *= inv;
-            if (!(dd[0] > 1e-9) || !(dd[1] > 1e-9)) break;
-            n1.s = 1.4142135623730951 / dd[0];
-            n2.s = 1.4142135623730951 / dd[1];
-            double acc[45];
-#pragma unroll
-            for (int e = 0; e < 45; ++e) acc[e] = 0.0;
-            for (int i = tid; i < M; i += kRansacThreads)
-                if (mask[i]) {
-                    const float4 c = pts[i];
-                    const double u1 = ((double)c.x - n1.cx) * n1.s, v1 = ((double)c.y - n1.cy) * n1.s;
-                    const double u2 = ((double)c.z - n2.cx) * n2.s, v2 = ((double)c.w - n2.cy) * n2.s;
-                    const double ra[9] = {u1, v1, 1.0, 0.0, 0.0, 0.0, -(u2 * u1), -(u2 * v1), -u2};
-                    const double rb[9] = {0.0, 0.0, 0.0, u1, v1, 1.0, -(v2 * u1), -(v2 * v1), -v2};
-                    int e = 0;
-#pragma unroll
-                    for (int a = 0; a < 9; ++a)
-#pragma unroll
-                        for (int b = a; b < 9; ++b) {
-                            acc[e] += ra[a] * ra[b];
-                            acc[e] += rb[a] * rb[b];
-                            ++e;
-                        }
-                }
-            double* AtA = S.modelD;              // 81 doubles; the eigen-solver's scratch follows
-            block_tree_sum_many<45>(acc, red_part, red_tot);
-            if (tid == 0) {
-                int e = 0;
-                for (int a = 0; a < 9; ++a)
-                    for (int b = a; b < 9; ++b) { AtA[a * 9 + b] = acc[e]; AtA[b * 9 + a] = acc[e]; ++e; }
-            }
-            __syncthreads();
-            if (tid == 0) {
-                double Hn[9];
-                S.ok = smallest_eigvec9(AtA, S.modelD + 81, Hn);
-                if (S.ok) S.ok = denormalise_h(Hn, n1, n2, S.trialH);
-            }
-            __syncthreads();
-            if (!S.ok) break;
-            const int cnt = block_count_inliers_h(S.trialH, pts, M, thr2, nullptr, &S.total);
-            if (cnt <= best) break;
-            best = cnt;
-            if (tid < 9) S.bestH[tid] = S.trialH[tid];
-            __syncthreads();
-            block_count_inliers_h(S.bestH, pts, M, thr2, mask, &S.total);
-        }
-    }
-    __syncthreads();
-    if (prm.min_inliers > 0 && best < prm.min_inliers) {
-        for (int i = tid; i < M; i += kRansacThreads) mask[i] = 0;
-        return;
-    }
-    if (tid == 0) {
-        // cv2 convention H[2,2] == 1.0 exactly: divide, never multiply by a reciprocal
-        const double s = (fabs(S.bestH[8]) > 1.1920928955078125e-07) ? S.bestH[8] : 1.0;
-        for (int i = 0; i < 9; ++i) out_H[(long long)p * 9 + i] = S.bestH[i] / s;
-        out_ninl[p] = best;
-    }
+    ransac_driver<HomographyModel>(corr, corr_stride, count, offsets, pair_id, samples, stop_target, prm, pts_cap, out_H, out_ninl,
+                                   out_mask, out_iters);
 }
 
 }  // namespace sfm
 
 using namespace sfm;
 
-static int launch_ransac_h(const float* corr, int corr_stride, const int32_t* count, const int32_t* offsets, int n_pairs,
-                           const uint32_t* pair_id, const uint32_t* samples, const int32_t* stop_target,
-                           const sfm_ransac_params* prm, double* out_H, int32_t* out_ninl, uint8_t* out_mask, int32_t* out_iters,
-                           void* stream)
-{
-    SFM_REQUIRE(corr && (count || offsets) && prm && out_H && out_ninl && out_mask, "sfm_ransac_h: NULL argument");
-    SFM_REQUIRE(prm->max_iters > 0 && prm->threshold > 0.f, "max_iters and threshold must be positive");
-    SFM_REQUIRE(corr_stride > 0 && n_pairs >= 0, "bad sizes");
-    SFM_REQUIRE(((uintptr_t)corr & 15) == 0, "corr must be 16-byte aligned");
-    if (n_pairs == 0) return SFM_OK;
-    constexpr int kPtsCap = 4096;
-    const int pts_cap = corr_stride < kPtsCap ? corr_stride : kPtsCap;
-    const size_t fixed = (sizeof(RansacHSmem) + 15) & ~(size_t)15;
-    const size_t smem = fixed + (size_t)pts_cap * 16;
-    static SmemAttrTable attr;                               // per device; these entry points run on the caller's current device
-    SFM_CUDA_CHECK(ensure_dyn_smem(ransac_h_kernel, smem, current_device(), attr));
-    ransac_h_kernel<<<n_pairs, kRansacThreads, smem, (cudaStream_t)stream>>>(corr, corr_stride, count, offsets, pair_id, samples,
-                                                                            stop_target, *prm, pts_cap, out_H, out_ninl, out_mask, out_iters);
-    SFM_CUDA_CHECK(cudaGetLastError());
-    count_launch();
-    return SFM_OK;
-}
-
 extern "C" int sfm_ransac_h_batch(const float* corr, int corr_stride, const int32_t* count, int n_pairs, const uint32_t* pair_id,
                                   const uint32_t* samples, const int32_t* stop_target, const sfm_ransac_params* prm, double* out_H,
                                   int32_t* out_ninl, uint8_t* out_mask, int32_t* out_iters, void* stream)
 {
     SFM_REQUIRE(count != nullptr, "sfm_ransac_h_batch: NULL argument");
-    return launch_ransac_h(corr, corr_stride, count, nullptr, n_pairs, pair_id, samples, stop_target, prm, out_H, out_ninl, out_mask,
-                           out_iters, stream);
+    return launch_ransac<HomographyModel>(ransac_h_kernel, corr, corr_stride, count, nullptr, n_pairs, pair_id, samples, stop_target, prm,
+                                          out_H, out_ninl, out_mask, out_iters, stream);
 }
 
 extern "C" int sfm_ransac_h_packed(const float* corr, const int32_t* offsets, int n_pairs, int max_count, const uint32_t* pair_id,
@@ -444,6 +162,6 @@ extern "C" int sfm_ransac_h_packed(const float* corr, const int32_t* offsets, in
                                    int32_t* out_ninl, uint8_t* out_mask, int32_t* out_iters, void* stream)
 {
     SFM_REQUIRE(offsets != nullptr, "sfm_ransac_h_packed: NULL argument");
-    return launch_ransac_h(corr, max_count, nullptr, offsets, n_pairs, pair_id, samples, stop_target, prm, out_H, out_ninl, out_mask,
-                           out_iters, stream);
+    return launch_ransac<HomographyModel>(ransac_h_kernel, corr, max_count, nullptr, offsets, n_pairs, pair_id, samples, stop_target, prm,
+                                          out_H, out_ninl, out_mask, out_iters, stream);
 }

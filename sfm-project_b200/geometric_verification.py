@@ -31,30 +31,13 @@ def verify_pairs(points1, points2, *, thr=3.0, confidence=0.99, max_iters=2000, 
                  lo=False, seed=0, min_inliers=0):
     """Batched verification.  ``points1[k]``, ``points2[k]`` are the [M_k,2] matched pixel coordinates of pair k.
     Returns a list of ``(F or None, mask uint8 [M_k,1])``."""
-    if len(points1) != len(points2):
-        raise ValueError("points1 and points2 must have the same number of pairs")
-    P = len(points1)
-    if P == 0:
+    if len(points1) == len(points2) == 0:
         return []
-    p1 = [_as_points(p, "pts1") for p in points1]
-    p2 = [_as_points(p, "pts2") for p in points2]
-    for a, b in zip(p1, p2):
-        if len(a) != len(b):
-            raise ValueError("pts1 and pts2 must have the same number of points")
-    cap = max(16, max(len(a) for a in p1))
-    corr = np.zeros((P, cap, 4), np.float32)
-    counts = np.zeros(P, np.int32)
-    for k, (a, b) in enumerate(zip(p1, p2)):
-        corr[k, : len(a), :2], corr[k, : len(a), 2:] = a, b
-        counts[k] = len(a)
-    vb = _sfm.verify_corr(torch.from_numpy(corr).cuda(), torch.from_numpy(counts), thr=thr, confidence=confidence,
-                          max_iters=max_iters, solver=solver, score=score, lo=lo, seed=seed, min_inliers=min_inliers)
+    corr, counts_t, counts = _corr_batch(points1, points2)
+    vb = _sfm.verify_corr(corr, counts_t, thr=thr, confidence=confidence, max_iters=max_iters, solver=solver, score=score, lo=lo,
+                          seed=seed, min_inliers=min_inliers)
     F, ninl, mask = vb.F.cpu().numpy(), vb.n_inliers.cpu().numpy(), vb.mask.cpu().numpy()
-    out = []
-    for k in range(P):
-        m = mask[k, : counts[k]].reshape(-1, 1).copy()
-        out.append((F[k].copy() if ninl[k] > 0 else None, m))
-    return out
+    return [(F[k].copy() if ninl[k] > 0 else None, mask[k, : counts[k]].reshape(-1, 1).copy()) for k in range(len(counts))]
 
 
 def verify_pair(pts1, pts2, *, thr=3.0, confidence=0.99, max_iters=2000, solver="7pt", score="sym_epipolar", lo=False,

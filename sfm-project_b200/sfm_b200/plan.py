@@ -266,9 +266,7 @@ class HotPathPlan:
             ev.record(cur)
             self._consumed[slot] = ev
         o.ev_filter.record(cur)
-        _lib.check(L.sfm_ransac_f_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), P, self.cap, _lib.ptr(pair_id_d), None,
-                                         C.byref(self.rprm), _lib.ptr(o.F), _lib.ptr(o.n_inliers), _lib.ptr(o.inlier),
-                                         _lib.ptr(o.iters), st), "sfm_ransac_f_packed")
+        self._ransac_f(o, st)
         if self.homography:
             # the scene graph only asks whether H explains more than h_ratio of what F explains: sampling may stop once a
             # homography with that support would have been found (general pairs: 32 hypotheses instead of max_iters)
@@ -295,12 +293,14 @@ class HotPathPlan:
 
     def rerun_ransac(self) -> None:
         """Verification stage alone on the packed correspondences of the last batch (bench.py times it in isolation)."""
-        o = self.cur
-        if o.P == 0:
-            return
+        if self.cur.P:
+            self._ransac_f(self.cur, _lib.current_stream_ptr(self.dev))
+
+    def _ransac_f(self, o, st) -> None:
+        """RANSAC-F on the packed correspondences of output set ``o`` (its ``P`` pairs), enqueued on stream ``st``."""
         _lib.check(_lib.lib().sfm_ransac_f_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), o.P, self.cap, _lib.ptr(o.pair_id), None,
                                                   C.byref(self.rprm), _lib.ptr(o.F), _lib.ptr(o.n_inliers), _lib.ptr(o.inlier),
-                                                  _lib.ptr(o.iters), _lib.current_stream_ptr(self.dev)), "sfm_ransac_f_packed")
+                                                  _lib.ptr(o.iters), st), "sfm_ransac_f_packed")
 
     # ------------------------------------------------------------------ host results of a job
     def job_begin(self, n_pairs: int) -> None:

@@ -39,15 +39,14 @@ def ransac_params(*, thr=3.0, confidence=0.99, max_iters=2000, solver="7pt", sco
     return p
 
 
-def verify_corr(corr: torch.Tensor, counts: torch.Tensor, *, pair_id=None, samples=None, **kw) -> VerifyBatch:
-    """corr float32 [P, cap, 4] (x1,y1,x2,y2) on the GPU, counts int32 [P]."""
+def _run(entry: str, corr: torch.Tensor, counts: torch.Tensor, prm, pair_id, samples, *stop_target) -> VerifyBatch:
+    """One call of ``sfm_ransac_f_batch`` or, with a ``stop_target`` argument (None or [P]), ``sfm_ransac_h_batch``."""
     if corr.dtype != torch.float32 or corr.dim() != 3 or corr.shape[2] != 4 or not corr.is_cuda:
         raise ValueError("corr must be a CUDA float32 tensor [P, cap, 4]")
     corr = corr.contiguous()
     counts = counts.to(device=corr.device, dtype=torch.int32).contiguous()
     P, cap, dev = corr.shape[0], corr.shape[1], corr.device
-    prm = ransac_params(**kw)
-    F = torch.zeros((P, 3, 3), dtype=torch.float64, device=dev)
+    model = torch.zeros((P, 3, 3), dtype=torch.float64, device=dev)
     ninl = torch.zeros(P, dtype=torch.int32, device=dev)
     mask = torch.zeros((P, cap), dtype=torch.uint8, device=dev)
     iters = torch.zeros(P, dtype=torch.int32, device=dev)
@@ -58,14 +57,22 @@ def verify_corr(corr: torch.Tensor, counts: torch.Tensor, *, pair_id=None, sampl
         if s.shape != (prm.max_iters, 8):
             raise ValueError(f"samples must be [max_iters, 8], got {s.shape}")
         smp = torch.from_numpy(s.view(np.int32)).to(dev)
+    tgt = [None if t is None else torch.as_tensor(t).to(device=dev, dtype=torch.int32).contiguous() for t in stop_target]
+    if any(t is not None and tuple(t.shape) != (P,) for t in tgt):
+        raise ValueError("stop_target must be [P]")
     if P:
         _lib.check(
-            _lib.lib().sfm_ransac_f_batch(_lib.ptr(corr), cap, _lib.ptr(counts), P, _lib.ptr(pid), _lib.ptr(smp), C.byref(prm),
-                                          _lib.ptr(F), _lib.ptr(ninl), _lib.ptr(mask), _lib.ptr(iters),
-                                          _lib.current_stream_ptr(dev)),
-            "sfm_ransac_f_batch",
+            getattr(_lib.lib(), entry)(_lib.ptr(corr), cap, _lib.ptr(counts), P, _lib.ptr(pid), _lib.ptr(smp), *map(_lib.ptr, tgt),
+                                       C.byref(prm), _lib.ptr(model), _lib.ptr(ninl), _lib.ptr(mask), _lib.ptr(iters),
+                                       _lib.current_stream_ptr(dev)),
+            entry,
         )
-    return VerifyBatch(F, ninl, mask, iters)
+    return VerifyBatch(model, ninl, mask, iters)
+
+
+def verify_corr(corr: torch.Tensor, counts: torch.Tensor, *, pair_id=None, samples=None, **kw) -> VerifyBatch:
+    """corr float32 [P, cap, 4] (x1,y1,x2,y2) on the GPU, counts int32 [P]."""
+    return _run("sfm_ransac_f_batch", corr, counts, ransac_params(**kw), pair_id, samples)
 
 
 def h_stop_target(n_inliers_f, ratio: float):
@@ -85,34 +92,8 @@ def verify_h_corr(corr: torch.Tensor, counts: torch.Tensor, *, pair_id=None, sam
     """Batched RANSAC homography on the same buffers as ``verify_corr`` (C ABI: sfm_ransac_h_batch); conventions of
     ``cv2.findHomography(RANSAC)``.  ``VerifyBatch.F`` holds H (x2 ~ H x1, H[2,2] == 1).  ``stop_target`` (int32 [P], e.g.
     0.8 * the pair's F inliers) ends sampling once a model with that support would have been found (see include/sfm_b200.h)."""
-    if corr.dtype != torch.float32 or corr.dim() != 3 or corr.shape[2] != 4 or not corr.is_cuda:
-        raise ValueError("corr must be a CUDA float32 tensor [P, cap, 4]")
-    corr = corr.contiguous()
-    counts = counts.to(device=corr.device, dtype=torch.int32).contiguous()
-    P, cap, dev = corr.shape[0], corr.shape[1], corr.device
     prm = ransac_params(thr=thr, confidence=confidence, max_iters=max_iters, solver="8pt", lo=lo, seed=seed, min_inliers=min_inliers)
-    H = torch.zeros((P, 3, 3), dtype=torch.float64, device=dev)
-    ninl = torch.zeros(P, dtype=torch.int32, device=dev)
-    mask = torch.zeros((P, cap), dtype=torch.uint8, device=dev)
-    iters = torch.zeros(P, dtype=torch.int32, device=dev)
-    pid = None if pair_id is None else torch.as_tensor(np.asarray(pair_id, np.int64).astype(np.uint32).view(np.int32)).to(dev)
-    smp = None
-    if samples is not None:
-        s = np.ascontiguousarray(samples, np.uint32)
-        if s.shape != (prm.max_iters, 8):
-            raise ValueError(f"samples must be [max_iters, 8], got {s.shape}")
-        smp = torch.from_numpy(s.view(np.int32)).to(dev)
-    tgt = None if stop_target is None else torch.as_tensor(stop_target).to(device=dev, dtype=torch.int32).contiguous()
-    if tgt is not None and tuple(tgt.shape) != (P,):
-        raise ValueError("stop_target must be [P]")
-    if P:
-        _lib.check(
-            _lib.lib().sfm_ransac_h_batch(_lib.ptr(corr), cap, _lib.ptr(counts), P, _lib.ptr(pid), _lib.ptr(smp), _lib.ptr(tgt), C.byref(prm),
-                                          _lib.ptr(H), _lib.ptr(ninl), _lib.ptr(mask), _lib.ptr(iters),
-                                          _lib.current_stream_ptr(dev)),
-            "sfm_ransac_h_batch",
-        )
-    return VerifyBatch(H, ninl, mask, iters)
+    return _run("sfm_ransac_h_batch", corr, counts, prm, pair_id, samples, stop_target)
 
 
 @dataclass

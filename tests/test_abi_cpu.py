@@ -56,6 +56,38 @@ def test_argument_errors_are_reported_without_a_gpu():
     with pytest.raises(sfm_b200.SfmError):
         sfm_b200._lib.check(-1, "unit-test")
 
+    # RANSAC-F / RANSAC-H launchers: every rejection returns before any CUDA call.  Pointers are fake and never read.
+    from sfm_b200.ransac import ransac_params
+
+    def ransac(entry, corr=0x1000, size=64, n_pairs=1, null=None, **fields):
+        prm = ransac_params(solver="8pt")
+        for k, v in fields.items():
+            setattr(prm, k, v)
+        a = {"corr": corr, "idx": 0x2000, "prm": C.byref(prm), "out": 0x3000, "ninl": 0x4000, "mask": 0x5000}
+        if null:
+            a[null] = None
+        head = [a["corr"], size, a["idx"], n_pairs] if entry.endswith("_batch") else [a["corr"], a["idx"], n_pairs, size]
+        opt = [None] * (3 if "_h_" in entry else 2)            # pair_id, samples (, stop_target)
+        rc = getattr(L, entry)(*head, *opt, a["prm"], a["out"], a["ninl"], a["mask"], None, None)
+        return rc, L.sfm_last_error().decode()
+
+    for entry in ("sfm_ransac_f_batch", "sfm_ransac_f_packed", "sfm_ransac_h_batch", "sfm_ransac_h_packed"):
+        model = entry.rsplit("_", 1)[0]
+        assert ransac(entry, null="idx") == (-1, f"{entry}: NULL argument")
+        for null in ("corr", "prm", "out", "ninl", "mask"):
+            assert ransac(entry, null=null) == (-1, f"{model}: NULL argument"), (entry, null)
+        assert ransac(entry, max_iters=0) == (-1, "max_iters and threshold must be positive")
+        assert ransac(entry, threshold=0.0) == (-1, "max_iters and threshold must be positive")
+        assert ransac(entry, size=0) == (-1, "bad sizes")
+        assert ransac(entry, n_pairs=-1) == (-1, "bad sizes")
+        assert ransac(entry, corr=0x1004) == (-1, "corr must be 16-byte aligned")
+        assert ransac(entry, n_pairs=0)[0] == 0
+        if model == "sfm_ransac_f":
+            assert ransac(entry, solver=5) == (-1, "solver must be 7 or 8, got 5")
+            assert ransac(entry, score=2) == (-1, "unknown score 2")
+        else:                                                  # RANSAC-H ignores both fields
+            assert ransac(entry, n_pairs=0, solver=5, score=2)[0] == 0
+
 
 def test_no_cpu_fallback_without_cuda(monkeypatch):
     import torch
