@@ -1,4 +1,6 @@
-/* ransac_common.h -- helpers shared by the CPU oracles (ransac_f.c, ransac_h.c, pose.c).
+/* ransac_common.h -- helpers shared by the CPU oracles (ransac_f.c, ransac_h.c, pose.c), and the RANSAC driver that
+ * runs RANSAC-F and RANSAC-H.  Each of those two supplies only an oracle_model (see below), as the kernels supply a
+ * Model policy to ransac_driver.
  *
  * TEST INFRASTRUCTURE ONLY (see ransac_f.c).  Operation for operation the same as
  * sfm-project_b200/csrc/ransac_common.cuh; built with -ffp-contract=off.
@@ -42,6 +44,18 @@ static __attribute__((unused)) void draw_sample(uint64_t seed, uint32_t pair, ui
             if (!dup) break;
         }
         idx[k] = v;
+    }
+}
+
+/* The m correspondence indices of hypothesis hyp: the caller's samples rows ([max_iters, 8], reduced mod M) or drawn.
+ * Kernel twin: hypothesis_sample. */
+static __attribute__((unused)) void hypothesis_sample(const uint32_t* samples, uint64_t seed, uint32_t pair, int hyp, int m,
+                                                      int M, int* idx)
+{
+    if (samples) {
+        for (int k = 0; k < m; ++k) idx[k] = (int)(samples[(size_t)hyp * 8 + k] % (uint32_t)M);
+    } else {
+        draw_sample(seed, pair, (uint32_t)hyp, m, M, idx);
     }
 }
 
@@ -162,5 +176,236 @@ static __attribute__((unused)) int smallest_eigvec9(const double* A, double* xou
     }
     for (int i = 0; i < 9; ++i) xout[i] = x[i];
     return 1;
+}
+
+/* ------------------------------------------------------------ the RANSAC driver */
+/* The rows (1 or 2) that one Hartley-normalised correspondence adds to a model's linear system, in the minimal solver
+ * and in the LO refit */
+typedef int (*model_rows_fn)(double u1, double v1, double u2, double v2, double (*r)[9]);
+/* fp32 inlier predicate of a model rounded to float */
+typedef int (*inlier_fn)(const float* model, const float* c, float thr2, int score);
+
+/* What RANSAC-F and RANSAC-H supply to oracle_ransac_driver; the kernel twin is the Model policy of ransac_driver. */
+typedef struct {
+    int (*sample_size)(const sfm_ransac_params* prm);              /* m; 0 when prm names no solver of this model */
+    int (*solve)(const float* corr, const int* idx, int m, double* out);   /* up to 3 unit-norm models; returns their number */
+    inlier_fn inlier;
+    model_rows_fn rows;
+    int lo_min;                                                    /* fewest inliers the LO refit runs on */
+    int (*refit)(double* h, norm2d n1, norm2d n2, double* out);    /* model from the smallest eigenvector h; 0 if unusable */
+} oracle_model;
+
+/* Hartley normalisation (n1, n2) of the m-point sample idx, then the null space of the n rows (at most 8) that `rows`
+ * makes from its points, by Gauss-Jordan elimination with complete pivoting: 9 - n vectors in N.  Returns 9 - n; 0 when
+ * the points of either image coincide or a pivot is not above tol.  Kernel twins: hartley_sample and coop_gauss_jordan. */
+static __attribute__((unused)) int hartley_null_space(const float* corr, const int* idx, int m, model_rows_fn rows, double tol,
+                                                      norm2d* n1, norm2d* n2, double N[2][9])
+{
+    double x1[8], y1[8], x2[8], y2[8];
+    for (int k = 0; k < m; ++k) {
+        const float* c = corr + 4 * (size_t)idx[k];
+        x1[k] = (double)c[0]; y1[k] = (double)c[1];
+        x2[k] = (double)c[2]; y2[k] = (double)c[3];
+    }
+    {
+        double sx = 0.0, sy = 0.0, tx = 0.0, ty = 0.0;
+        for (int k = 0; k < m; ++k) { sx += x1[k]; sy += y1[k]; tx += x2[k]; ty += y2[k]; }
+        double inv = 1.0 / (double)m;
+        n1->cx = sx * inv; n1->cy = sy * inv; n2->cx = tx * inv; n2->cy = ty * inv;
+        double d1 = 0.0, d2 = 0.0;
+        for (int k = 0; k < m; ++k) {
+            double ax = x1[k] - n1->cx, ay = y1[k] - n1->cy;
+            double bx = x2[k] - n2->cx, by = y2[k] - n2->cy;
+            d1 += sqrt(ax * ax + ay * ay);
+            d2 += sqrt(bx * bx + by * by);
+        }
+        d1 *= inv; d2 *= inv;
+        if (!(d1 > 1e-9) || !(d2 > 1e-9)) return 0;
+        n1->s = 1.4142135623730951 / d1;
+        n2->s = 1.4142135623730951 / d2;
+    }
+    double A[8][9];
+    int n = 0;
+    for (int k = 0; k < m; ++k) {
+        double u1 = (x1[k] - n1->cx) * n1->s, v1 = (y1[k] - n1->cy) * n1->s;
+        double u2 = (x2[k] - n2->cx) * n2->s, v2 = (y2[k] - n2->cy) * n2->s;
+        n += rows(u1, v1, u2, v2, A + n);
+    }
+    int perm[9];
+    for (int j = 0; j < 9; ++j) perm[j] = j;
+    for (int k = 0; k < n; ++k) {
+        int pi = k, pj = k;
+        double best = -1.0;
+        for (int i = k; i < n; ++i)
+            for (int j = k; j < 9; ++j) {
+                double v = fabs(A[i][j]);
+                if (v > best) { best = v; pi = i; pj = j; }
+            }
+        if (!(best > tol)) return 0;
+        if (pi != k)
+            for (int j = 0; j < 9; ++j) { double t = A[k][j]; A[k][j] = A[pi][j]; A[pi][j] = t; }
+        if (pj != k) {
+            for (int i = 0; i < n; ++i) { double t = A[i][k]; A[i][k] = A[i][pj]; A[i][pj] = t; }
+            int t = perm[k]; perm[k] = perm[pj]; perm[pj] = t;
+        }
+        double inv = 1.0 / A[k][k];
+        for (int j = k; j < 9; ++j) A[k][j] *= inv;
+        for (int i = 0; i < n; ++i) {
+            if (i == k) continue;
+            double f = A[i][k];
+            for (int j = k; j < 9; ++j) A[i][j] -= f * A[k][j];
+        }
+    }
+    for (int c = 0; c < 9 - n; ++c) {
+        for (int j = 0; j < 9; ++j) N[c][j] = 0.0;
+        N[c][perm[n + c]] = 1.0;
+        for (int k = 0; k < n; ++k) N[c][perm[k]] = -A[k][n + c];
+    }
+    return 9 - n;
+}
+
+/* Inliers of a model after rounding it to float; mask may be NULL.  Kernel twin: block_count_inliers. */
+static __attribute__((unused)) int count_inliers(inlier_fn inlier, const double* model, const float* corr, int M, float thr2,
+                                                 int score, uint8_t* mask)
+{
+    float Mf[9];
+    for (int i = 0; i < 9; ++i) Mf[i] = (float)model[i];
+    int n = 0;
+    for (int i = 0; i < M; ++i) {
+        int in = inlier(Mf, corr + 4 * (size_t)i, thr2, score);
+        if (mask) mask[i] = (uint8_t)in;
+        n += in;
+    }
+    return n;
+}
+
+/* LO: Hartley-normalised least-squares refit on the inliers in mask -- moments, mean distances and the 9 x 9 normal
+ * matrix of the model's rows, each summed over SFM_RANSAC_LANES lanes and lane_tree, then its smallest eigenvector.
+ * Kernel twin: the LO step of ransac_driver. */
+static __attribute__((unused)) int lo_refit(const oracle_model* mdl, const float* corr, int M, const uint8_t* mask, double* out)
+{
+    double part[SFM_RANSAC_LANES];
+    double mom[5];
+    for (int q = 0; q < 5; ++q) {
+        for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
+            double s = 0.0;
+            for (int i = t; i < M; i += SFM_RANSAC_LANES)
+                if (mask[i]) s += (q == 4) ? 1.0 : (double)corr[4 * (size_t)i + q];
+            part[t] = s;
+        }
+        mom[q] = lane_tree(part);
+    }
+    if (!(mom[4] >= (double)mdl->lo_min)) return 0;
+    norm2d n1, n2;
+    double inv = 1.0 / mom[4];
+    n1.cx = mom[0] * inv; n1.cy = mom[1] * inv; n2.cx = mom[2] * inv; n2.cy = mom[3] * inv;
+    double dd[2];
+    for (int q = 0; q < 2; ++q) {
+        double cx = q ? n2.cx : n1.cx, cy = q ? n2.cy : n1.cy;
+        for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
+            double s = 0.0;
+            for (int i = t; i < M; i += SFM_RANSAC_LANES)
+                if (mask[i]) {
+                    double ax = (double)corr[4 * (size_t)i + 2 * q] - cx;
+                    double ay = (double)corr[4 * (size_t)i + 2 * q + 1] - cy;
+                    s += sqrt(ax * ax + ay * ay);
+                }
+            part[t] = s;
+        }
+        dd[q] = lane_tree(part) * inv;
+    }
+    if (!(dd[0] > 1e-9) || !(dd[1] > 1e-9)) return 0;
+    n1.s = 1.4142135623730951 / dd[0];
+    n2.s = 1.4142135623730951 / dd[1];
+    double AtA[81];
+    for (int a = 0; a < 9; ++a)
+        for (int b = a; b < 9; ++b) {
+            for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
+                double s = 0.0;
+                for (int i = t; i < M; i += SFM_RANSAC_LANES)
+                    if (mask[i]) {
+                        const float* c = corr + 4 * (size_t)i;
+                        double u1 = ((double)c[0] - n1.cx) * n1.s, v1 = ((double)c[1] - n1.cy) * n1.s;
+                        double u2 = ((double)c[2] - n2.cx) * n2.s, v2 = ((double)c[3] - n2.cy) * n2.s;
+                        double r[2][9];
+                        int nr = mdl->rows(u1, v1, u2, v2, r);
+                        for (int j = 0; j < nr; ++j) s += r[j][a] * r[j][b];
+                    }
+                part[t] = s;
+            }
+            double v = lane_tree(part);
+            AtA[a * 9 + b] = v;
+            AtA[b * 9 + a] = v;
+        }
+    double h[9];
+    if (!smallest_eigvec9(AtA, h)) return 0;
+    return mdl->refit(h, n1, n2, out);
+}
+
+/* One RANSAC run on the M correspondences corr (x1, y1, x2, y2): hypotheses in batches of ransac_batch, strict-greater
+ * selection in (hypothesis, root) order, the stop rule on max(best, stop_target clamped to [0, M]), the final mask, the
+ * LO rounds and the min_inliers rule.  out_mask and out_iters may be NULL.  The model is divided by its element [8]
+ * (cv2's convention).  Kernel twin: ransac_driver. */
+static __attribute__((unused)) int oracle_ransac_driver(const oracle_model* mdl, const float* corr, int M,
+                                                        const sfm_ransac_params* prm, uint32_t pair_id, const uint32_t* samples,
+                                                        int stop_target, double* out_model, int32_t* out_ninl,
+                                                        uint8_t* out_mask, int32_t* out_iters)
+{
+    const int m = mdl->sample_size(prm);
+    const float thr2 = prm->threshold * prm->threshold;
+    for (int i = 0; i < 9; ++i) out_model[i] = 0.0;
+    if (out_mask) memset(out_mask, 0, (size_t)(M > 0 ? M : 0));
+    *out_ninl = 0;
+    if (out_iters) *out_iters = 0;
+    if (m == 0 || M < m) return 0;
+
+    double bestM[9];
+    int best = 0, done = 0;
+    while (done < prm->max_iters) {
+        int nb = prm->max_iters - done;
+        if (nb > ransac_batch(done)) nb = ransac_batch(done);
+        for (int h = 0; h < nb; ++h) {
+            int idx[8];
+            hypothesis_sample(samples, prm->seed, pair_id, done + h, m, M, idx);
+            double Mm[27];
+            int nm = mdl->solve(corr, idx, m, Mm);
+            for (int r = 0; r < nm; ++r) {
+                int cnt = count_inliers(mdl->inlier, Mm + 9 * r, corr, M, thr2, prm->score, NULL);
+                if (cnt > best) { best = cnt; memcpy(bestM, Mm + 9 * r, sizeof bestM); }
+            }
+        }
+        done += nb;
+        int target = stop_target < 0 ? 0 : (stop_target > M ? M : stop_target);
+        if (should_stop(best > target ? best : target, M, m, done, prm->confidence)) break;
+    }
+    if (out_iters) *out_iters = done;
+    if (best < m) return 0;
+
+    uint8_t* mask = out_mask ? out_mask : (uint8_t*)malloc((size_t)M);
+    best = count_inliers(mdl->inlier, bestM, corr, M, thr2, prm->score, mask);
+    if (prm->lo_refit) {
+        uint8_t* trial = (uint8_t*)malloc((size_t)M);
+        for (int round = 0; round < SFM_LO_ROUNDS; ++round) {
+            double Mr[9];
+            if (!lo_refit(mdl, corr, M, mask, Mr)) break;
+            int cnt = count_inliers(mdl->inlier, Mr, corr, M, thr2, prm->score, trial);
+            if (cnt <= best) break;
+            best = cnt;
+            memcpy(bestM, Mr, sizeof bestM);
+            memcpy(mask, trial, (size_t)M);
+        }
+        free(trial);
+    }
+    if (prm->min_inliers > 0 && best < prm->min_inliers) {
+        memset(mask, 0, (size_t)M);
+        if (!out_mask) free(mask);
+        return 0;
+    }
+    if (!out_mask) free(mask);
+    /* cv2 convention model[2,2] == 1.0 exactly: divide (x / x == 1), never multiply by a reciprocal */
+    const double s = (fabs(bestM[8]) > 1.1920928955078125e-07) ? bestM[8] : 1.0;
+    for (int i = 0; i < 9; ++i) out_model[i] = bestM[i] / s;
+    *out_ninl = best;
+    return 0;
 }
 #endif

@@ -135,80 +135,29 @@ static int solve_cubic(double c3, double c2, double c1, double c0, double* roots
     return n;
 }
 
+/* The epipolar row of one normalised correspondence: x2^T F x1 = 0 */
+static int rows_f(double u1, double v1, double u2, double v2, double (*r)[9])
+{
+    r[0][0] = u2 * u1; r[0][1] = u2 * v1; r[0][2] = u2;
+    r[0][3] = v2 * u1; r[0][4] = v2 * v1; r[0][5] = v2;
+    r[0][6] = u1;      r[0][7] = v1;      r[0][8] = 1.0;
+    return 1;
+}
+
+/* F from a null vector of the normalised system: the 8-point model, and the LO refit's */
+static int refit_f(double* Fh, norm2d n1, norm2d n2, double* F)
+{
+    enforce_rank2(Fh);
+    return denormalise(Fh, n1, n2, F);
+}
+
 /* Minimal solver: m = 7 or 8 sample points -> up to 3 unit-norm F (row-major). */
 static int solve_minimal(const float* corr, const int* idx, int m, double* Fout)
 {
-    double x1[8], y1[8], x2[8], y2[8];
-    for (int k = 0; k < m; ++k) {
-        const float* c = corr + 4 * (size_t)idx[k];
-        x1[k] = (double)c[0]; y1[k] = (double)c[1];
-        x2[k] = (double)c[2]; y2[k] = (double)c[3];
-    }
     norm2d n1, n2;
-    {
-        double sx = 0.0, sy = 0.0, tx = 0.0, ty = 0.0;
-        for (int k = 0; k < m; ++k) { sx += x1[k]; sy += y1[k]; tx += x2[k]; ty += y2[k]; }
-        double inv = 1.0 / (double)m;
-        n1.cx = sx * inv; n1.cy = sy * inv; n2.cx = tx * inv; n2.cy = ty * inv;
-        double d1 = 0.0, d2 = 0.0;
-        for (int k = 0; k < m; ++k) {
-            double ax = x1[k] - n1.cx, ay = y1[k] - n1.cy;
-            double bx = x2[k] - n2.cx, by = y2[k] - n2.cy;
-            d1 += sqrt(ax * ax + ay * ay);
-            d2 += sqrt(bx * bx + by * by);
-        }
-        d1 *= inv; d2 *= inv;
-        if (!(d1 > 1e-9) || !(d2 > 1e-9)) return 0;
-        n1.s = 1.4142135623730951 / d1;
-        n2.s = 1.4142135623730951 / d2;
-    }
-    double A[8][9];
-    for (int k = 0; k < m; ++k) {
-        double u1 = (x1[k] - n1.cx) * n1.s, v1 = (y1[k] - n1.cy) * n1.s;
-        double u2 = (x2[k] - n2.cx) * n2.s, v2 = (y2[k] - n2.cy) * n2.s;
-        A[k][0] = u2 * u1; A[k][1] = u2 * v1; A[k][2] = u2;
-        A[k][3] = v2 * u1; A[k][4] = v2 * v1; A[k][5] = v2;
-        A[k][6] = u1;      A[k][7] = v1;      A[k][8] = 1.0;
-    }
-    /* Gauss-Jordan with complete pivoting */
-    int perm[9];
-    for (int j = 0; j < 9; ++j) perm[j] = j;
-    for (int k = 0; k < m; ++k) {
-        int pi = k, pj = k;
-        double best = -1.0;
-        for (int i = k; i < m; ++i)
-            for (int j = k; j < 9; ++j) {
-                double v = fabs(A[i][j]);
-                if (v > best) { best = v; pi = i; pj = j; }
-            }
-        if (!(best > 1e-12)) return 0;
-        if (pi != k)
-            for (int j = 0; j < 9; ++j) { double t = A[k][j]; A[k][j] = A[pi][j]; A[pi][j] = t; }
-        if (pj != k) {
-            for (int i = 0; i < m; ++i) { double t = A[i][k]; A[i][k] = A[i][pj]; A[i][pj] = t; }
-            int t = perm[k]; perm[k] = perm[pj]; perm[pj] = t;
-        }
-        double inv = 1.0 / A[k][k];
-        for (int j = k; j < 9; ++j) A[k][j] *= inv;
-        for (int i = 0; i < m; ++i) {
-            if (i == k) continue;
-            double f = A[i][k];
-            for (int j = k; j < 9; ++j) A[i][j] -= f * A[k][j];
-        }
-    }
     double N[2][9];
-    int nfree = 9 - m;
-    for (int c = 0; c < nfree; ++c) {
-        for (int j = 0; j < 9; ++j) N[c][j] = 0.0;
-        N[c][perm[m + c]] = 1.0;
-        for (int k = 0; k < m; ++k) N[c][perm[k]] = -A[k][m + c];
-    }
-    if (m == 8) {
-        double Fh[9];
-        for (int i = 0; i < 9; ++i) Fh[i] = N[0][i];
-        enforce_rank2(Fh);
-        return denormalise(Fh, n1, n2, Fout);
-    }
+    if (!hartley_null_space(corr, idx, m, rows_f, 1e-12, &n1, &n2, N)) return 0;
+    if (m == 8) return refit_f(N[0], n1, n2, Fout);
     /* 7 point: det(l*F1 + F2) = 0 */
     const double* F1 = N[0];
     const double* F2 = N[1];
@@ -246,147 +195,17 @@ static int is_inlier(const float* Ff, const float* c, float thr2, int score)
     return n2 <= lim;
 }
 
-static int count_inliers(const double* F, const float* corr, int M, float thr2, int score, uint8_t* mask)
-{
-    float Ff[9];
-    for (int i = 0; i < 9; ++i) Ff[i] = (float)F[i];
-    int n = 0;
-    for (int i = 0; i < M; ++i) {
-        int in = is_inlier(Ff, corr + 4 * (size_t)i, thr2, score);
-        if (mask) mask[i] = (uint8_t)in;
-        n += in;
-    }
-    return n;
-}
-
-/* -------------------------------------------------------------- LO refit */
-static int lo_refit(const float* corr, int M, const uint8_t* mask, double* F)
-{
-    double part[SFM_RANSAC_LANES];
-    double mom[5];
-    for (int q = 0; q < 5; ++q) {
-        for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
-            double s = 0.0;
-            for (int i = t; i < M; i += SFM_RANSAC_LANES)
-                if (mask[i]) s += (q == 4) ? 1.0 : (double)corr[4 * (size_t)i + q];
-            part[t] = s;
-        }
-        mom[q] = lane_tree(part);
-    }
-    if (!(mom[4] >= 8.0)) return 0;
-    norm2d n1, n2;
-    double inv = 1.0 / mom[4];
-    n1.cx = mom[0] * inv; n1.cy = mom[1] * inv; n2.cx = mom[2] * inv; n2.cy = mom[3] * inv;
-    double dd[2];
-    for (int q = 0; q < 2; ++q) {
-        double cx = q ? n2.cx : n1.cx, cy = q ? n2.cy : n1.cy;
-        for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
-            double s = 0.0;
-            for (int i = t; i < M; i += SFM_RANSAC_LANES)
-                if (mask[i]) {
-                    double ax = (double)corr[4 * (size_t)i + 2 * q] - cx;
-                    double ay = (double)corr[4 * (size_t)i + 2 * q + 1] - cy;
-                    s += sqrt(ax * ax + ay * ay);
-                }
-            part[t] = s;
-        }
-        dd[q] = lane_tree(part) * inv;
-    }
-    if (!(dd[0] > 1e-9) || !(dd[1] > 1e-9)) return 0;
-    n1.s = 1.4142135623730951 / dd[0];
-    n2.s = 1.4142135623730951 / dd[1];
-    double AtA[81];
-    for (int a = 0; a < 9; ++a)
-        for (int b = a; b < 9; ++b) {
-            for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
-                double s = 0.0;
-                for (int i = t; i < M; i += SFM_RANSAC_LANES)
-                    if (mask[i]) {
-                        const float* c = corr + 4 * (size_t)i;
-                        double u1 = ((double)c[0] - n1.cx) * n1.s, v1 = ((double)c[1] - n1.cy) * n1.s;
-                        double u2 = ((double)c[2] - n2.cx) * n2.s, v2 = ((double)c[3] - n2.cy) * n2.s;
-                        double r[9] = {u2 * u1, u2 * v1, u2, v2 * u1, v2 * v1, v2, u1, v1, 1.0};
-                        s += r[a] * r[b];
-                    }
-                part[t] = s;
-            }
-            double v = lane_tree(part);
-            AtA[a * 9 + b] = v;
-            AtA[b * 9 + a] = v;
-        }
-    double Fh[9];
-    if (!smallest_eigvec9(AtA, Fh)) return 0;
-    enforce_rank2(Fh);
-    return denormalise(Fh, n1, n2, F);
-}
-
 /* --------------------------------------------------------------- driver */
+static int sample_size_f(const sfm_ransac_params* prm) { return (prm->solver == 7 || prm->solver == 8) ? prm->solver : 0; }
+
+/* LO needs 8 inliers for the 7-point solver too */
+static const oracle_model kFundamental = {sample_size_f, solve_minimal, is_inlier, rows_f, 8, refit_f};
+
 int sfm_oracle_ransac_f(const float* corr, int M, const sfm_ransac_params* prm, uint32_t pair_id,
                         const uint32_t* samples, double* out_F, int32_t* out_ninl,
                         uint8_t* out_mask, int32_t* out_iters)
 {
-    const int m = prm->solver;
-    const float thr2 = prm->threshold * prm->threshold;
-    for (int i = 0; i < 9; ++i) out_F[i] = 0.0;
-    if (out_mask) memset(out_mask, 0, (size_t)(M > 0 ? M : 0));
-    *out_ninl = 0;
-    if (out_iters) *out_iters = 0;
-    if ((m != 7 && m != 8) || M < m) return 0;
-
-    double bestF[9];
-    int best = 0, done = 0;
-    while (done < prm->max_iters) {
-        int nb = prm->max_iters - done;
-        if (nb > ransac_batch(done)) nb = ransac_batch(done);
-        for (int h = 0; h < nb; ++h) {
-            int idx[8];
-            if (samples) {
-                for (int k = 0; k < m; ++k) {
-                    uint32_t v = samples[(size_t)(done + h) * 8 + k];
-                    idx[k] = (int)(v % (uint32_t)M);
-                }
-            } else {
-                draw_sample(prm->seed, pair_id, (uint32_t)(done + h), m, M, idx);
-            }
-            double Fm[27];
-            int nm = solve_minimal(corr, idx, m, Fm);
-            for (int r = 0; r < nm; ++r) {
-                int cnt = count_inliers(Fm + 9 * r, corr, M, thr2, prm->score, NULL);
-                if (cnt > best) { best = cnt; memcpy(bestF, Fm + 9 * r, sizeof bestF); }
-            }
-        }
-        done += nb;
-        if (should_stop(best, M, m, done, prm->confidence)) break;
-    }
-    if (out_iters) *out_iters = done;
-    if (best < m) return 0;
-
-    uint8_t* mask = out_mask ? out_mask : (uint8_t*)malloc((size_t)M);
-    best = count_inliers(bestF, corr, M, thr2, prm->score, mask);
-    if (prm->lo_refit) {
-        uint8_t* trial = (uint8_t*)malloc((size_t)M);
-        for (int round = 0; round < SFM_LO_ROUNDS; ++round) {
-            double Fr[9];
-            if (!lo_refit(corr, M, mask, Fr)) break;
-            int cnt = count_inliers(Fr, corr, M, thr2, prm->score, trial);
-            if (cnt <= best) break;
-            best = cnt;
-            memcpy(bestF, Fr, sizeof bestF);
-            memcpy(mask, trial, (size_t)M);
-        }
-        free(trial);
-    }
-    if (prm->min_inliers > 0 && best < prm->min_inliers) {
-        memset(mask, 0, (size_t)M);
-        if (!out_mask) free(mask);
-        return 0;
-    }
-    if (!out_mask) free(mask);
-    /* cv2 convention F[2,2] == 1.0 exactly: divide (x / x == 1), never multiply by a reciprocal */
-    const double s = (fabs(bestF[8]) > 1.1920928955078125e-07) ? bestF[8] : 1.0;
-    for (int i = 0; i < 9; ++i) out_F[i] = bestF[i] / s;
-    *out_ninl = best;
-    return 0;
+    return oracle_ransac_driver(&kFundamental, corr, M, prm, pair_id, samples, 0, out_F, out_ninl, out_mask, out_iters);
 }
 
 /* Expose the pieces so tests can pin them individually. */
@@ -399,7 +218,7 @@ int sfm_oracle_solve_minimal(const float* corr, const int32_t* idx, int m, doubl
 
 int sfm_oracle_count_inliers(const double* F, const float* corr, int M, float thr, int score, uint8_t* mask)
 {
-    return count_inliers(F, corr, M, thr * thr, score, mask);
+    return count_inliers(is_inlier, F, corr, M, thr * thr, score, mask);
 }
 
 void sfm_oracle_draw_sample(uint64_t seed, uint32_t pair, uint32_t hyp, int m, int M, int32_t* idx)

@@ -42,81 +42,36 @@ static int denormalise_h(const double* Hn, norm2d n1, norm2d n2, double* H)
     return 1;
 }
 
-static int solve_h4(const float* corr, const int* idx, double* Hout)
+/* The two DLT rows of one normalised correspondence: x2 ~ H x1 */
+static int rows_h(double u1, double v1, double u2, double v2, double (*r)[9])
 {
-    double x1[4], y1[4], x2[4], y2[4];
-    for (int k = 0; k < 4; ++k) {
-        const float* c = corr + 4 * (size_t)idx[k];
-        x1[k] = (double)c[0]; y1[k] = (double)c[1]; x2[k] = (double)c[2]; y2[k] = (double)c[3];
-    }
+    double* r0 = r[0];
+    double* r1 = r[1];
+    r0[0] = u1;  r0[1] = v1;  r0[2] = 1.0; r0[3] = 0.0; r0[4] = 0.0; r0[5] = 0.0;
+    r0[6] = -(u2 * u1); r0[7] = -(u2 * v1); r0[8] = -u2;
+    r1[0] = 0.0; r1[1] = 0.0; r1[2] = 0.0; r1[3] = u1;  r1[4] = v1;  r1[5] = 1.0;
+    r1[6] = -(v2 * u1); r1[7] = -(v2 * v1); r1[8] = -v2;
+    return 2;
+}
+
+static int solve_h4(const float* corr, const int* idx, int m, double* Hout)
+{
     norm2d n1, n2;
-    {
-        double sx = 0.0, sy = 0.0, tx = 0.0, ty = 0.0;
-        for (int k = 0; k < 4; ++k) { sx += x1[k]; sy += y1[k]; tx += x2[k]; ty += y2[k]; }
-        n1.cx = sx * 0.25; n1.cy = sy * 0.25; n2.cx = tx * 0.25; n2.cy = ty * 0.25;
-        double d1 = 0.0, d2 = 0.0;
-        for (int k = 0; k < 4; ++k) {
-            double ax = x1[k] - n1.cx, ay = y1[k] - n1.cy;
-            double bx = x2[k] - n2.cx, by = y2[k] - n2.cy;
-            d1 += sqrt(ax * ax + ay * ay);
-            d2 += sqrt(bx * bx + by * by);
-        }
-        d1 *= 0.25; d2 *= 0.25;
-        if (!(d1 > 1e-9) || !(d2 > 1e-9)) return 0;
-        n1.s = 1.4142135623730951 / d1;
-        n2.s = 1.4142135623730951 / d2;
-    }
-    double A[8][9];
-    for (int k = 0; k < 4; ++k) {
-        double u1 = (x1[k] - n1.cx) * n1.s, v1 = (y1[k] - n1.cy) * n1.s;
-        double u2 = (x2[k] - n2.cx) * n2.s, v2 = (y2[k] - n2.cy) * n2.s;
-        double* r0 = A[2 * k];
-        double* r1 = A[2 * k + 1];
-        r0[0] = u1;  r0[1] = v1;  r0[2] = 1.0; r0[3] = 0.0; r0[4] = 0.0; r0[5] = 0.0;
-        r0[6] = -(u2 * u1); r0[7] = -(u2 * v1); r0[8] = -u2;
-        r1[0] = 0.0; r1[1] = 0.0; r1[2] = 0.0; r1[3] = u1;  r1[4] = v1;  r1[5] = 1.0;
-        r1[6] = -(v2 * u1); r1[7] = -(v2 * v1); r1[8] = -v2;
-    }
-    int perm[9];
-    for (int j = 0; j < 9; ++j) perm[j] = j;
-    for (int k = 0; k < 8; ++k) {
-        int pi = k, pj = k;
-        double best = -1.0;
-        for (int i = k; i < 8; ++i)
-            for (int j = k; j < 9; ++j) {
-                double v = fabs(A[i][j]);
-                if (v > best) { best = v; pi = i; pj = j; }
-            }
-        if (!(best > 1e-10)) return 0;
-        if (pi != k)
-            for (int j = 0; j < 9; ++j) { double t = A[k][j]; A[k][j] = A[pi][j]; A[pi][j] = t; }
-        if (pj != k) {
-            for (int i = 0; i < 8; ++i) { double t = A[i][k]; A[i][k] = A[i][pj]; A[i][pj] = t; }
-            int t = perm[k]; perm[k] = perm[pj]; perm[pj] = t;
-        }
-        double inv = 1.0 / A[k][k];
-        for (int j = k; j < 9; ++j) A[k][j] *= inv;
-        for (int i = 0; i < 8; ++i) {
-            if (i == k) continue;
-            double f = A[i][k];
-            for (int j = k; j < 9; ++j) A[i][j] -= f * A[k][j];
-        }
-    }
-    double Hn[9];
-    for (int j = 0; j < 9; ++j) Hn[j] = 0.0;
-    Hn[perm[8]] = 1.0;
-    for (int k = 0; k < 8; ++k) Hn[perm[k]] = -A[k][8];
-    if (!denormalise_h(Hn, n1, n2, Hout)) return 0;
+    double N[2][9];
+    if (!hartley_null_space(corr, idx, 4, rows_h, 1e-10, &n1, &n2, N)) return 0;
+    if (!denormalise_h(N[0], n1, n2, Hout)) return 0;
+    /* the sample points map with w of one sign */
     int pos = 0, neg = 0;
     for (int k = 0; k < 4; ++k) {
-        double w = Hout[6] * x1[k] + Hout[7] * y1[k] + Hout[8];
+        const float* c = corr + 4 * (size_t)idx[k];
+        double w = Hout[6] * (double)c[0] + Hout[7] * (double)c[1] + Hout[8];
         pos += (w > 0.0);
         neg += (w < 0.0);
     }
     return (pos == 4 || neg == 4) ? 1 : 0;
 }
 
-static int is_inlier_h(const float* H, const float* c, float thr2)
+static int is_inlier_h(const float* H, const float* c, float thr2, int score)
 {
     float X = fmaf(H[0], c[0], fmaf(H[1], c[1], H[2]));
     float Y = fmaf(H[3], c[0], fmaf(H[4], c[1], H[5]));
@@ -129,150 +84,27 @@ static int is_inlier_h(const float* H, const float* c, float thr2)
     return e2 <= lim && lim > 0.f;
 }
 
-static int count_inliers_h(const double* H, const float* corr, int M, float thr2, uint8_t* mask)
-{
-    float Hf[9];
-    for (int i = 0; i < 9; ++i) Hf[i] = (float)H[i];
-    int n = 0;
-    for (int i = 0; i < M; ++i) {
-        int in = is_inlier_h(Hf, corr + 4 * (size_t)i, thr2);
-        if (mask) mask[i] = (uint8_t)in;
-        n += in;
-    }
-    return n;
-}
+static int refit_h(double* Hn, norm2d n1, norm2d n2, double* H) { return denormalise_h(Hn, n1, n2, H); }
 
-static int lo_refit_h(const float* corr, int M, const uint8_t* mask, double* H)
-{
-    double part[SFM_RANSAC_LANES];
-    double mom[5];
-    for (int q = 0; q < 5; ++q) {
-        for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
-            double s = 0.0;
-            for (int i = t; i < M; i += SFM_RANSAC_LANES)
-                if (mask[i]) s += (q == 4) ? 1.0 : (double)corr[4 * (size_t)i + q];
-            part[t] = s;
-        }
-        mom[q] = lane_tree(part);
-    }
-    if (!(mom[4] >= 4.0)) return 0;
-    norm2d n1, n2;
-    double inv = 1.0 / mom[4];
-    n1.cx = mom[0] * inv; n1.cy = mom[1] * inv; n2.cx = mom[2] * inv; n2.cy = mom[3] * inv;
-    double dd[2];
-    for (int q = 0; q < 2; ++q) {
-        double cx = q ? n2.cx : n1.cx, cy = q ? n2.cy : n1.cy;
-        for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
-            double s = 0.0;
-            for (int i = t; i < M; i += SFM_RANSAC_LANES)
-                if (mask[i]) {
-                    double ax = (double)corr[4 * (size_t)i + 2 * q] - cx;
-                    double ay = (double)corr[4 * (size_t)i + 2 * q + 1] - cy;
-                    s += sqrt(ax * ax + ay * ay);
-                }
-            part[t] = s;
-        }
-        dd[q] = lane_tree(part) * inv;
-    }
-    if (!(dd[0] > 1e-9) || !(dd[1] > 1e-9)) return 0;
-    n1.s = 1.4142135623730951 / dd[0];
-    n2.s = 1.4142135623730951 / dd[1];
-    double AtA[81];
-    for (int a = 0; a < 9; ++a)
-        for (int b = a; b < 9; ++b) {
-            for (int t = 0; t < SFM_RANSAC_LANES; ++t) {
-                double s = 0.0;
-                for (int i = t; i < M; i += SFM_RANSAC_LANES)
-                    if (mask[i]) {
-                        const float* c = corr + 4 * (size_t)i;
-                        double u1 = ((double)c[0] - n1.cx) * n1.s, v1 = ((double)c[1] - n1.cy) * n1.s;
-                        double u2 = ((double)c[2] - n2.cx) * n2.s, v2 = ((double)c[3] - n2.cy) * n2.s;
-                        double ra[9] = {u1, v1, 1.0, 0.0, 0.0, 0.0, -(u2 * u1), -(u2 * v1), -u2};
-                        double rb[9] = {0.0, 0.0, 0.0, u1, v1, 1.0, -(v2 * u1), -(v2 * v1), -v2};
-                        s += ra[a] * ra[b];
-                        s += rb[a] * rb[b];
-                    }
-                part[t] = s;
-            }
-            double v = lane_tree(part);
-            AtA[a * 9 + b] = v;
-            AtA[b * 9 + a] = v;
-        }
-    double Hn[9];
-    if (!smallest_eigvec9(AtA, Hn)) return 0;
-    return denormalise_h(Hn, n1, n2, H);
-}
+static int sample_size_h(const sfm_ransac_params* prm) { return 4; }
+
+static const oracle_model kHomography = {sample_size_h, solve_h4, is_inlier_h, rows_h, 4, refit_h};
 
 int sfm_oracle_ransac_h(const float* corr, int M, const sfm_ransac_params* prm, uint32_t pair_id,
                         const uint32_t* samples, int stop_target, double* out_H, int32_t* out_ninl,
                         uint8_t* out_mask, int32_t* out_iters)
 {
-    const float thr2 = prm->threshold * prm->threshold;
-    for (int i = 0; i < 9; ++i) out_H[i] = 0.0;
-    if (out_mask) memset(out_mask, 0, (size_t)(M > 0 ? M : 0));
-    *out_ninl = 0;
-    if (out_iters) *out_iters = 0;
-    if (M < 4) return 0;
-
-    double bestH[9];
-    int best = 0, done = 0;
-    while (done < prm->max_iters) {
-        int nb = prm->max_iters - done;
-        if (nb > ransac_batch(done)) nb = ransac_batch(done);
-        for (int h = 0; h < nb; ++h) {
-            int idx[4];
-            if (samples) {
-                for (int k = 0; k < 4; ++k) idx[k] = (int)(samples[(size_t)(done + h) * 8 + k] % (uint32_t)M);
-            } else {
-                draw_sample(prm->seed, pair_id, (uint32_t)(done + h), 4, M, idx);
-            }
-            double Hm[9];
-            if (!solve_h4(corr, idx, Hm)) continue;
-            int cnt = count_inliers_h(Hm, corr, M, thr2, NULL);
-            if (cnt > best) { best = cnt; memcpy(bestH, Hm, sizeof bestH); }
-        }
-        done += nb;
-        int target = stop_target < 0 ? 0 : (stop_target > M ? M : stop_target);
-        if (should_stop(best > target ? best : target, M, 4, done, prm->confidence)) break;
-    }
-    if (out_iters) *out_iters = done;
-    if (best < 4) return 0;
-
-    uint8_t* mask = out_mask ? out_mask : (uint8_t*)malloc((size_t)M);
-    best = count_inliers_h(bestH, corr, M, thr2, mask);
-    if (prm->lo_refit) {
-        uint8_t* trial = (uint8_t*)malloc((size_t)M);
-        for (int round = 0; round < SFM_LO_ROUNDS; ++round) {
-            double Hr[9];
-            if (!lo_refit_h(corr, M, mask, Hr)) break;
-            int cnt = count_inliers_h(Hr, corr, M, thr2, trial);
-            if (cnt <= best) break;
-            best = cnt;
-            memcpy(bestH, Hr, sizeof bestH);
-            memcpy(mask, trial, (size_t)M);
-        }
-        free(trial);
-    }
-    if (prm->min_inliers > 0 && best < prm->min_inliers) {
-        memset(mask, 0, (size_t)M);
-        if (!out_mask) free(mask);
-        return 0;
-    }
-    if (!out_mask) free(mask);
-    const double s = (fabs(bestH[8]) > 1.1920928955078125e-07) ? bestH[8] : 1.0;
-    for (int i = 0; i < 9; ++i) out_H[i] = bestH[i] / s;
-    *out_ninl = best;
-    return 0;
+    return oracle_ransac_driver(&kHomography, corr, M, prm, pair_id, samples, stop_target, out_H, out_ninl, out_mask, out_iters);
 }
 
 int sfm_oracle_solve_h4(const float* corr, const int32_t* idx, double* Hout)
 {
     int id[4];
     for (int k = 0; k < 4; ++k) id[k] = idx[k];
-    return solve_h4(corr, id, Hout);
+    return solve_h4(corr, id, 4, Hout);
 }
 
 int sfm_oracle_count_inliers_h(const double* H, const float* corr, int M, float thr, uint8_t* mask)
 {
-    return count_inliers_h(H, corr, M, thr * thr, mask);
+    return count_inliers(is_inlier_h, H, corr, M, thr * thr, 0, mask);
 }

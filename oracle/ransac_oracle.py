@@ -46,9 +46,10 @@ def lib():
     global _lib
     if _lib is None:
         _lib = C.CDLL(build())
-        _lib.sfm_oracle_ransac_f.restype = C.c_int
-        _lib.sfm_oracle_solve_minimal.restype = C.c_int
-        _lib.sfm_oracle_count_inliers.restype = C.c_int
+        for name in ("ransac_f", "ransac_h", "solve_minimal", "solve_h4", "count_inliers", "count_inliers_h",
+                     "smallest_eigvec9", "two_view_pose", "triangulate"):
+            getattr(_lib, "sfm_oracle_" + name).restype = C.c_int
+        _lib.sfm_oracle_draw_sample.restype = None
     return _lib
 
 
@@ -64,26 +65,26 @@ def _corr(pts1, pts2):
     return np.ascontiguousarray(c, np.float32)
 
 
-def ransac_f(pts1, pts2, *, pair_id=0, samples=None, **kw):
-    """Returns (F float64[3,3] or None, mask uint8[M], n_inliers, iters)."""
+def _ransac(entry, pts1, pts2, prm, pair_id, samples, *stop_target):
+    """Runs sfm_oracle_ransac_f or sfm_oracle_ransac_h (which also takes stop_target)."""
     corr = _corr(pts1, pts2)
     M = corr.shape[0]
-    prm = make_params(**kw)
-    F = np.zeros(9, np.float64)
+    model = np.zeros(9, np.float64)
     mask = np.zeros(max(M, 1), np.uint8)
-    ninl = C.c_int32(0)
-    iters = C.c_int32(0)
+    ninl, iters = C.c_int32(0), C.c_int32(0)
     sp = None
     if samples is not None:
         samples = np.ascontiguousarray(samples, np.uint32)
         assert samples.shape == (prm.max_iters, 8)
         sp = samples.ctypes.data_as(C.c_void_p)
-    lib().sfm_oracle_ransac_f(
-        corr.ctypes.data_as(C.c_void_p), C.c_int(M), C.byref(prm), C.c_uint32(pair_id), sp,
-        F.ctypes.data_as(C.c_void_p), C.byref(ninl), mask.ctypes.data_as(C.c_void_p), C.byref(iters),
-    )
-    Fm = F.reshape(3, 3) if ninl.value > 0 else None
-    return Fm, mask[:M], int(ninl.value), int(iters.value)
+    entry(corr.ctypes.data_as(C.c_void_p), C.c_int(M), C.byref(prm), C.c_uint32(pair_id), sp, *stop_target,
+          model.ctypes.data_as(C.c_void_p), C.byref(ninl), mask.ctypes.data_as(C.c_void_p), C.byref(iters))
+    return (model.reshape(3, 3) if ninl.value > 0 else None), mask[:M], int(ninl.value), int(iters.value)
+
+
+def ransac_f(pts1, pts2, *, pair_id=0, samples=None, **kw):
+    """Returns (F float64[3,3] or None, mask uint8[M], n_inliers, iters)."""
+    return _ransac(lib().sfm_oracle_ransac_f, pts1, pts2, make_params(**kw), pair_id, samples)
 
 
 def solve_minimal(pts1, pts2, idx):
@@ -146,31 +147,15 @@ def iou(a, b) -> float:
 def ransac_h(pts1, pts2, *, pair_id=0, samples=None, thr=3.0, max_iters=2000, confidence=0.995, seed=0, lo=False, min_inliers=0,
              stop_target=0):
     """Returns (H float64[3,3] or None, mask uint8[M], n_inliers, iters)."""
-    corr = _corr(pts1, pts2)
-    M = corr.shape[0]
     prm = make_params(solver=8, thr=thr, max_iters=max_iters, confidence=confidence, seed=seed, lo=lo, min_inliers=min_inliers)
-    H = np.zeros(9, np.float64)
-    mask = np.zeros(max(M, 1), np.uint8)
-    ninl, iters = C.c_int32(0), C.c_int32(0)
-    sp = None
-    if samples is not None:
-        samples = np.ascontiguousarray(samples, np.uint32)
-        assert samples.shape == (prm.max_iters, 8)
-        sp = samples.ctypes.data_as(C.c_void_p)
-    L = lib()
-    L.sfm_oracle_ransac_h.restype = C.c_int
-    L.sfm_oracle_ransac_h(corr.ctypes.data_as(C.c_void_p), C.c_int(M), C.byref(prm), C.c_uint32(pair_id), sp, C.c_int(int(stop_target)),
-                          H.ctypes.data_as(C.c_void_p), C.byref(ninl), mask.ctypes.data_as(C.c_void_p), C.byref(iters))
-    return (H.reshape(3, 3) if ninl.value > 0 else None), mask[:M], int(ninl.value), int(iters.value)
+    return _ransac(lib().sfm_oracle_ransac_h, pts1, pts2, prm, pair_id, samples, C.c_int(int(stop_target)))
 
 
 def solve_h4(pts1, pts2, idx):
     corr = _corr(pts1, pts2)
     idx = np.ascontiguousarray(idx, np.int32)
     out = np.zeros(9, np.float64)
-    L = lib()
-    L.sfm_oracle_solve_h4.restype = C.c_int
-    ok = L.sfm_oracle_solve_h4(corr.ctypes.data_as(C.c_void_p), idx.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p))
+    ok = lib().sfm_oracle_solve_h4(corr.ctypes.data_as(C.c_void_p), idx.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p))
     return out.reshape(3, 3) if ok else None
 
 
@@ -198,10 +183,8 @@ def two_view_pose(pts1, pts2, F, cam, *, mask=None, distance_thresh=50.0):
         mask = np.ascontiguousarray(np.asarray(mask).ravel(), np.uint8)
         assert mask.shape[0] == M
         mp = mask.ctypes.data_as(C.c_void_p)
-    L = lib()
-    L.sfm_oracle_two_view_pose.restype = C.c_int
-    n = L.sfm_oracle_two_view_pose(corr.ctypes.data_as(C.c_void_p), C.c_int(M), mp, F.ctypes.data_as(C.c_void_p),
-                                   cam.ctypes.data_as(C.c_void_p), C.c_double(distance_thresh), R.ctypes.data_as(C.c_void_p),
-                                   t.ctypes.data_as(C.c_void_p), E.ctypes.data_as(C.c_void_p), omask.ctypes.data_as(C.c_void_p),
-                                   X.ctypes.data_as(C.c_void_p))
+    n = lib().sfm_oracle_two_view_pose(corr.ctypes.data_as(C.c_void_p), C.c_int(M), mp, F.ctypes.data_as(C.c_void_p),
+                                       cam.ctypes.data_as(C.c_void_p), C.c_double(distance_thresh), R.ctypes.data_as(C.c_void_p),
+                                       t.ctypes.data_as(C.c_void_p), E.ctypes.data_as(C.c_void_p), omask.ctypes.data_as(C.c_void_p),
+                                       X.ctypes.data_as(C.c_void_p))
     return int(n), R.reshape(3, 3), t, E.reshape(3, 3), omask[:M], X[:M]
