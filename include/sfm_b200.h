@@ -343,6 +343,51 @@ int sfm_orb_retain_best(const float* response_host, int n, int n_points, int32_t
 int sfm_orb_harris_angle(const uint8_t* img, int w, int h, int pitch, const int32_t* xy, const int32_t* sel, int n,
                          int32_t* out_xy, float* out_resp, float* out_angle, void* stream);
 
+/* ------------------------------------------------------------- feature tracks (f5)
+ * The output of correspondence search (Schoenberger & Frahm 2016, §2.1) that registration and multi-view triangulation
+ * read: the reference's empty code/3d_reconstruction.py (imported at code/pipeline.py:4) would build it from the
+ * `pair_matches` list of code/pipeline.py:43-47.  A track is a connected component of the graph whose nodes are
+ * n = image * S + feature (S = features per image, n_images * S < 2^31) and whose edges are the used match rows.
+ *
+ *   pairs      int32 [n_pairs, 2]   (i, j) per pair
+ *   row_start  int64 [n_pairs]      pair p owns rows [row_start[p], row_start[p] + n_rows[p]) of rows / row_flag
+ *   n_rows     int32 [n_pairs]
+ *   rows       int32 [., 3]         (q, t, d2): the edge (i*S + q, j*S + t); d2 is not read
+ *   row_flag   uint8 [.] or NULL    a row is used only when its flag is non-zero (NULL = every row)
+ *   n_inliers  int32 [n_pairs] or NULL   pairs with n_inliers[p] < params->min_pair_inliers contribute no row
+ * A row that would be used but has q or t outside [0, S) (or whose pair names an image outside [0, n_images)) is counted in
+ * counts[4] and not used.
+ *
+ * Candidates are the connected components of the used edges.  A candidate holding two features of one image is
+ * conflicting (counts[2]) and dropped unless keep_conflicts; then a candidate of fewer than min_length observations is
+ * dropped (counts[3]).  Kept tracks are numbered in ascending order of their smallest node, observations ascend by node:
+ * the output depends only on the SET of used edges (not on row / pair order, duplicates or both-direction rows).
+ *
+ *   sfm_tracks_workspace_bytes  size of the caller-owned device workspace (256-byte aligned)
+ *   sfm_tracks_init             start a job (one launch)
+ *   sfm_tracks_hook             add the used rows of a batch of pairs (one launch; any number of calls per job)
+ *   sfm_tracks_finalize         write the tracks (14 launches; the state stays valid for more hooks and another finalize):
+ *       track_of int32 [n_images, S]        track id of every feature, -1 = none
+ *       offsets  int64 [>= n_nodes/2 + 1]   track k owns observations [offsets[k], offsets[k+1])
+ *       obs      int32 [>= n_nodes, 2]      (image, feature)
+ *       counts   int64 [5]                  tracks, observations, conflicting candidates, short candidates, invalid rows
+ *     The buffers are sized for the worst case, so nothing waits for the host.
+ */
+typedef struct {
+    int32_t min_pair_inliers;  /* see n_inliers above                             */
+    int32_t min_length;        /* >= 2                                            */
+    int32_t keep_conflicts;    /* 0/1                                             */
+    int32_t reserved[5];
+} sfm_track_params;
+
+int sfm_tracks_workspace_bytes(int n_images, int S, size_t* out_bytes);
+int sfm_tracks_init(int n_images, int S, void* workspace, size_t workspace_bytes, void* stream);
+int sfm_tracks_hook(int n_images, int S, const int32_t* pairs, int n_pairs, const int64_t* row_start, const int32_t* n_rows,
+                    const int32_t* rows, const uint8_t* row_flag, const int32_t* n_inliers, const sfm_track_params* params,
+                    void* workspace, size_t workspace_bytes, void* stream);
+int sfm_tracks_finalize(int n_images, int S, const sfm_track_params* params, void* workspace, size_t workspace_bytes,
+                        int32_t* track_of, int64_t* offsets, int32_t* obs, int64_t* counts, void* stream);
+
 /* ------------------------------------------ result regions in peer memory (multi-GPU gather)
  * Across ranks, the reference's `pair_matches.append(Pair(...))` (code/pipeline.py:43-47) becomes: every rank
  * writes the packed match rows / inlier flags of its pair block straight into a region of the gathering rank's

@@ -123,6 +123,12 @@ __global__ void __launch_bounds__(1024) offsets_scan_kernel(const int32_t* __res
     if (threadIdx.x == 0) offset[n] = carry;
 }
 
+void launch_offsets_scan(const int32_t* cnt, int n, int32_t* offset, cudaStream_t st)
+{
+    offsets_scan_kernel<<<1, 1024, 0, st>>>(cnt, n, offset);
+    count_launch();
+}
+
 // Second half of the fused path: block b of pair p copies its compacted (queryIdx, trainIdx, D1) rows from its slice of the
 // scratch table to their final packed position and gathers the two keypoints of every match.
 __global__ void __launch_bounds__(256) gather_packed_kernel(const int32_t* __restrict__ pairs, const float* __restrict__ xy, int feat_stride,

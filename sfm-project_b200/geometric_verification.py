@@ -168,3 +168,42 @@ def two_view_geometry(pts1, pts2, K1=None, K2=None, *, thr=3.0, confidence=0.99,
         n, R, t, pm, X = recover_pose(F, pts1, pts2, K1, K2, mask=fmask, distance_thresh=distance_thresh)
         out.update(n_pose=n, R=R if n else None, t=t if n else None, in_front=pm, points3d=X)
     return out
+
+
+# ------------------------------------------------------------------ feature tracks (correspondence search output)
+def build_tracks(result, n_images, n_features, *, flags="inlier", min_pair_inliers=15, min_length=2, keep_conflicts=False):
+    """Feature tracks of a matched image set (csrc/tracks.cu): the connected components of the graph whose nodes are
+    ``image * n_features + feature`` and whose edges are the used match rows -- what ``code/3d_reconstruction.py`` (empty;
+    imported at ``code/pipeline.py:4``) would build from ``pair_matches`` for registration and triangulation.
+
+    ``result`` is one of
+      * ``VerifiedPairs.to_host()`` (numpy; uploaded once),
+      * the dict ``sfm_b200.dist.match_and_verify_sharded(gather="full")`` returns on its destination rank (device tensors,
+        used in place),
+      * the reference's ``pair_matches`` list (``Pair`` records whose ``matches`` are ``cv2.DMatch`` lists or int rows, as
+        ``code/pipeline.py:36-47`` or ``sfm_b200.to_reference_pairs`` build it): every match is used, ``flags`` and
+        ``min_pair_inliers`` do not apply.
+    A row is used when its ``flags`` array (``"inlier"``, ``"inlier_h"``, ``"in_front"`` or None = every row) is set and its pair
+    has ``n_inliers >= min_pair_inliers``.  Candidates holding two features of one image are dropped unless ``keep_conflicts``,
+    then those with fewer than ``min_length`` observations.  Returns ``sfm_b200.Tracks`` (device; ``.to_host()`` for numpy)."""
+    from sfm_b200 import tracks as tr
+
+    opts = dict(min_length=min_length, keep_conflicts=keep_conflicts)
+    if isinstance(result, dict) and "row_start" in result:
+        return tr.build_tracks_from_rows(result, n_images, n_features, flags=flags, min_pair_inliers=min_pair_inliers, **opts)
+    if isinstance(result, dict):
+        off = np.asarray(result["offsets"], np.int64)
+        return tr.build_tracks_device(result["pairs"], off[:-1], np.diff(off), result["matches"], tr.flag_rows(result, flags),
+                                      result["n_inliers"], n_images, n_features, min_pair_inliers=min_pair_inliers, **opts)
+    pairs, counts, rows = [], [], []
+    for p in result:
+        m = p.matches
+        r = (np.asarray(m, np.int32).reshape(-1, 3)[:, :2] if isinstance(m, np.ndarray)
+             else np.array([(d.queryIdx, d.trainIdx) for d in m], np.int32).reshape(-1, 2))
+        pairs.append((p.img_inx_1, p.img_inx_2))
+        counts.append(len(r))
+        rows.append(np.concatenate([r, np.zeros((len(r), 1), np.int32)], axis=1))
+    counts = np.asarray(counts, np.int64)
+    start = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64) if len(counts) else np.zeros(0, np.int64)
+    return tr.build_tracks_device(np.asarray(pairs, np.int32).reshape(-1, 2), start, counts,
+                                  np.concatenate(rows) if rows else np.zeros((0, 3), np.int32), None, None, n_images, n_features, **opts)

@@ -31,6 +31,7 @@ EXPORTS = [
     "sfm_ransac_f_batch", "sfm_ransac_f_packed", "sfm_ransac_h_batch", "sfm_ransac_h_packed",
     "sfm_two_view_pose_batch", "sfm_two_view_pose_packed",
     "sfm_orb_resize", "sfm_orb_blur", "sfm_orb_describe", "sfm_orb_fast_detect", "sfm_orb_retain_best", "sfm_orb_harris_angle",
+    "sfm_tracks_workspace_bytes", "sfm_tracks_init", "sfm_tracks_hook", "sfm_tracks_finalize",
     "sfm_peer_alloc", "sfm_peer_open", "sfm_peer_close", "sfm_peer_free", "sfm_copy_async", "sfm_probe_int8_mma", "sfm_debug_tc_tile", "sfm_debug_refine_stats", "sfm_launch_count",
 ]
 
@@ -54,6 +55,11 @@ class RansacParams(C.Structure):
         ("confidence", C.c_double), ("seed", C.c_uint64), ("lo_refit", C.c_int32), ("min_inliers", C.c_int32),
         ("reserved", C.c_int32 * 4),
     ]
+
+
+class TrackParams(C.Structure):
+    _fields_ = [("min_pair_inliers", C.c_int32), ("min_length", C.c_int32), ("keep_conflicts", C.c_int32),
+                ("reserved", C.c_int32 * 5)]
 
 
 class SfmError(RuntimeError):
@@ -103,6 +109,10 @@ def lib():
     L.sfm_orb_fast_detect.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]
     L.sfm_orb_retain_best.argtypes = [vp, i32, i32, vp]
     L.sfm_orb_harris_angle.argtypes = [vp, i32, i32, i32, vp, vp, i32, vp, vp, vp, vp]
+    L.sfm_tracks_workspace_bytes.argtypes = [i32, i32, C.POINTER(sz)]
+    L.sfm_tracks_init.argtypes = [i32, i32, vp, sz, vp]
+    L.sfm_tracks_hook.argtypes = [i32, i32, vp, i32, vp, vp, vp, vp, vp, C.POINTER(TrackParams), vp, sz, vp]
+    L.sfm_tracks_finalize.argtypes = [i32, i32, C.POINTER(TrackParams), vp, sz, vp, vp, vp, vp, vp]
     L.sfm_peer_alloc.argtypes = [i32, sz, C.POINTER(vp), vp]
     L.sfm_peer_open.argtypes = [i32, vp, C.POINTER(vp)]
     L.sfm_peer_close.argtypes = [i32, vp]

@@ -25,6 +25,7 @@ import torch
 import torch.distributed as dist
 
 from .plan import OUTPUTS, RowSink, outputs
+from .tracks import build_tracks_from_rows
 
 
 def world():
@@ -436,14 +437,21 @@ def match_and_verify_sharded(bank, pairs, *, mode: str = "block", dst: int = 0, 
     gather="summaries": n_matches, n_inliers, iters, F (H / n_inliers_h, R / t / n_pose when those stages are requested).
     gather="full"     : additionally the packed rows of every pair: ``matches`` int32 [rows,3] = (queryIdx, trainIdx, squared
                         L2), ``inlier`` uint8 [rows] (``inlier_h`` / ``in_front`` / ``points3d`` with the optional stages) and
-                        ``row_start`` int64 [P]: pair p owns rows ``row_start[p] : row_start[p] + n_matches[p]``.
-    All values are device tensors on ``dst``.  RANSAC streams are keyed by GLOBAL pair index, so every value equals what one
+                        ``row_start`` int64 [P]: pair p owns rows ``row_start[p] : row_start[p] + n_matches[p]``; ``pairs``
+                        (numpy int32 [P,2]) is the pair list.  ``tracks=True`` (with the options of ``match_and_verify``) then builds
+                        the feature tracks of the whole list on ``dst`` from the gathered rows (``out["tracks"]``); the ranks
+                        themselves hook nothing.
+    All values are device tensors on ``dst`` except ``pairs`` (host) and ``transport`` (a string).  RANSAC streams are keyed by GLOBAL pair index, so every value equals what one
     GPU computes for the whole list.  ``events`` (a dict) receives timing events recorded on the current stream: "compute"
     after this rank's last kernel and row copy, "done" after the gather.  Returns (gathered dict or None, local VerifiedPairs)."""
     from .pipeline import match_and_verify
 
     if gather not in ("full", "summaries"):
         raise ValueError("gather must be 'full' or 'summaries'")
+    track_opts = {k: params.pop(k) for k in ("track_flags", "min_pair_inliers", "min_length", "keep_conflicts") if k in params}
+    tracks = bool(params.pop("tracks", False))
+    if tracks and gather != "full":
+        raise ValueError("tracks=True needs gather='full': the tracks are built from the gathered rows")
     rank, ws = world()
     pairs = np.asarray(pairs, np.int32).reshape(-1, 2)
     n_total = len(pairs)
@@ -474,7 +482,12 @@ def match_and_verify_sharded(bank, pairs, *, mode: str = "block", dst: int = 0, 
             for name in region.fields:
                 out[name] = region.full[name]
             out["row_start"] = region.row_starts(out["n_matches"], lay)
+            out["pairs"] = pairs                                         # (host: the caller's list, as passed)
             out["transport"] = region.transport
+            if tracks:
+                opts = dict(track_opts)
+                flags = opts.pop("track_flags", "inlier")
+                out["tracks"] = build_tracks_from_rows(out, max(bank.n_images, 1), bank.max_feats, flags=flags, **opts)
     if events is not None:
         events["done"] = torch.cuda.Event(enable_timing=True)
         events["done"].record()

@@ -16,6 +16,7 @@ import torch
 
 from .bank import DescriptorBank
 from .plan import OUTPUTS, HotPathPlan, RowSink, outputs
+from .tracks import Tracks, build_tracks_device
 
 
 @dataclass
@@ -37,6 +38,7 @@ class VerifiedPairs:
     t: torch.Tensor | None = None            # float64 [P,3]    |t| = 1
     n_pose: torch.Tensor | None = None       # int32 [P]        inliers in front of both cameras
     plan: HotPathPlan | None = field(default=None, repr=False)     # the plan that ran the job (its buffers hold the last batch)
+    tracks: Tracks | None = None             # feature tracks of the job (tracks=True)
 
     def to_host(self, with_matches: bool = True) -> dict:
         """``pairs, n_matches, F, n_inliers, iters`` and, with ``with_matches``, the packed rows
@@ -58,7 +60,8 @@ class VerifiedPairs:
 
 
 _PLAN_KEYS = ("ratio", "ratio_mode", "mutual", "thr", "confidence", "max_iters", "solver", "score", "lo", "seed",
-              "min_inliers", "prefilter", "homography", "distance_thresh", "h_stop_ratio", "overlap")
+              "min_inliers", "prefilter", "homography", "distance_thresh", "h_stop_ratio", "overlap",
+              "tracks", "track_flags", "min_pair_inliers", "min_length", "keep_conflicts")
 
 
 def get_plan(bank: DescriptorBank, batch: int, **params) -> HotPathPlan:
@@ -67,6 +70,9 @@ def get_plan(bank: DescriptorBank, batch: int, **params) -> HotPathPlan:
     params.setdefault("distance_thresh", 50.0)
     params.setdefault("h_stop_ratio", 0.8)
     params.setdefault("overlap", True)
+    if not params.get("tracks"):                    # the track options only matter to a plan that builds tracks
+        for k in ("tracks", "track_flags", "min_pair_inliers", "min_length", "keep_conflicts"):
+            params.pop(k, None)
     intr = params.get("intrinsics")
     key = (int(batch),) + tuple(params.get(k) for k in _PLAN_KEYS) + (None if intr is None else np.asarray(intr, np.float64).tobytes(),)
     cache = bank.__dict__.setdefault("_plans", {})
@@ -82,7 +88,9 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
                      thr=3.0, confidence=0.99, max_iters=2000, solver="7pt", score="sym_epipolar", lo=False, seed=0,
                      min_inliers=0, pair_batch: int = 2048, pair_ids=None, fetch=False,
                      prefilter: bool = True, homography: bool = False, intrinsics=None, distance_thresh: float = 50.0,
-                     h_stop_ratio: float | None = 0.8, sink: RowSink | None = None, overlap: bool = True, _segments=None) -> VerifiedPairs:
+                     h_stop_ratio: float | None = 0.8, sink: RowSink | None = None, overlap: bool = True, tracks: bool = False,
+                     track_flags: str | None = "inlier", min_pair_inliers: int = 15, min_length: int = 2, keep_conflicts: bool = False,
+                     _segments=None) -> VerifiedPairs:
     """Match and verify every pair of ``pairs`` (int32 [P,2], image ids in the bank).
 
     ``pair_ids`` (default 0..P-1) name the RANSAC sample stream of each pair, so a sharded run that passes global
@@ -100,7 +108,14 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
     ``geometric_verification.classify_pairs``; its sampling stops once a homography explaining ``h_stop_ratio`` of the pair's
     F inliers would have been found -- pass ``None`` for the plain stop rule); ``intrinsics`` (one 3x3 K, ``[n_images,3,3]`` or ``[n_images,4]`` rows
     fx fy cx cy) recovers the relative pose of every pair from its F and inliers (``R``, ``t``, ``n_pose``; host rows
-    ``in_front`` and ``points3d`` float32 [rows,3] in the first camera's frame)."""
+    ``in_front`` and ``points3d`` float32 [rows,3] in the first camera's frame).
+
+    ``tracks=True`` also builds the job's feature tracks (``VerifiedPairs.tracks``, see ``sfm_b200.tracks``) on the GPU: each
+    batch's rows are hooked right after its last kernel, so tracks exist with ``fetch=False`` too and no row is kept or moved.
+    A row is used when its ``track_flags`` row array (``"inlier"``, ``"inlier_h"``, ``"in_front"`` or None = every row) is
+    set and its pair has ``n_inliers >= min_pair_inliers``; candidates holding two features of one image are dropped unless
+    ``keep_conflicts``, then those shorter than ``min_length``.  Node numbering uses the bank's ``max_feats`` features per
+    image and its ``n_images`` images."""
     pairs_host = np.ascontiguousarray(np.asarray(pairs.cpu() if isinstance(pairs, torch.Tensor) else pairs, np.int32).reshape(-1, 2))
     P = pairs_host.shape[0]
     if P and (pairs_host.min() < 0 or pairs_host.max() >= bank.n_images):
@@ -115,14 +130,21 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
         host = None
         if fetch:
             host = {"pairs": pairs_host, "offsets": np.zeros(1, np.int64), **{o.name: o.empty(0).numpy() for o in outs}}
-        return VerifiedPairs(pairs=torch.zeros((0, 2), dtype=torch.int32, device=dev), host=host,
+        trk = None
+        if tracks:
+            none = np.zeros(0, np.int32)
+            trk = build_tracks_device(none, none, none, none, None, None, max(bank.n_images, 1), bank.max_feats,
+                                      min_pair_inliers=min_pair_inliers, min_length=min_length, keep_conflicts=keep_conflicts, device=dev)
+        return VerifiedPairs(pairs=torch.zeros((0, 2), dtype=torch.int32, device=dev), host=host, tracks=trk,
                              **{o.name: o.empty(0, device=dev) for o in outs if o.per == "pair"})
     batch = int(min(pair_batch, P))
     if overlap and not _segments and 512 <= P <= batch:
         batch = -(-P // 2)                          # one-batch job: two halves, so that the first half's refinement hides under the second sweep
     plan = get_plan(bank, batch, ratio=ratio, ratio_mode=ratio_mode, mutual=mutual, thr=thr, confidence=confidence,
                     max_iters=max_iters, solver=solver, score=score, lo=lo, seed=seed, min_inliers=min_inliers, prefilter=prefilter,
-                    homography=homography, intrinsics=intrinsics, distance_thresh=distance_thresh, h_stop_ratio=h_stop_ratio, overlap=overlap)
+                    homography=homography, intrinsics=intrinsics, distance_thresh=distance_thresh, h_stop_ratio=h_stop_ratio, overlap=overlap,
+                    tracks=tracks, track_flags=track_flags, min_pair_inliers=min_pair_inliers, min_length=min_length,
+                    keep_conflicts=keep_conflicts)
     # one upload of the whole pair list and its RANSAC stream ids through a pinned staging buffer kept on the bank
     # (allocating pinned memory per call costs ~0.2 ms of idle GPU at the head of every job)
     stage = bank.__dict__.get("_pair_stage")
@@ -140,6 +162,8 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
     pairs_d = stage_d[: 2 * P].view(P, 2)
     ids_d = stage_d[2 * P: 3 * P]
     rev_d = pairs_d.flip(1).contiguous() if mutual else None
+    if plan.tracks is not None:
+        plan.tracks.begin(bank.n_images)              # ordered before every hook: the first sweep follows it on this stream
     # (the full-length result arrays are allocated after the first batch has been enqueued: every host microsecond before
     #  the first kernel is GPU idle time, everything after it hides behind the sweep)
     results = {}
@@ -198,6 +222,7 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
             trace.append(time.perf_counter())
     if plan.overlap:
         torch.cuda.current_stream(dev).wait_stream(plan.post_stream)     # the caller's stream sees every batch's results
+    trk = plan.tracks.finalize() if plan.tracks is not None else None
     host, d2h = None, 0
     if sink is not None:
         plan.ev_kernels = torch.cuda.Event(enable_timing=True)           # diagnostics: the job's last kernel, before its last row copies
@@ -213,7 +238,7 @@ def match_and_verify(bank: DescriptorBank, pairs, *, ratio=0.75, ratio_mode="cv2
             h = {k: v.copy() for k, v in h.items()}
         host = dict(h)
         host["pairs"] = pairs_host
-    return VerifiedPairs(pairs=pairs_d.clone(), host=host, d2h_bytes=d2h, plan=plan, **results)      # (pairs_d is a view of the staging buffer)
+    return VerifiedPairs(pairs=pairs_d.clone(), host=host, d2h_bytes=d2h, plan=plan, tracks=trk, **results)      # (pairs_d is a view of the staging buffer)
 
 
 def match_and_verify_host(desc, xy, pairs, *, bank: DescriptorBank | None = None, n_chunks: int = 3, fetch=True, pair_ids=None, chunk_growth: float = 1.0, **params):

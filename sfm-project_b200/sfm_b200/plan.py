@@ -7,6 +7,7 @@ fixed launch sequence on the caller's stream, and result copies on a side stream
     RANSAC-F on the packed correspondences                       sfm_ransac_f_packed
     [RANSAC-H on the same correspondences]                       sfm_ransac_h_packed            (homography=True)
     [E, (R, t) by cheirality vote, triangulated inliers]         sfm_two_view_pose_packed       (intrinsics given)
+    [union of the batch's used rows into the job's tracks]       sfm_tracks_hook                (tracks=True)
 
 This is the batched body of the reference's pair loop (code/pipeline.py:38-47) plus the verification stage it left
 empty (code/pipeline.py:60-65).  Nothing here computes: every array is produced by lib/libsfm_b200.so.
@@ -24,6 +25,7 @@ from . import _lib
 from .bank import DescriptorBank
 from .matcher import filter_params
 from .ransac import h_stop_target, ransac_params
+from .tracks import FLAG_FIELDS, TrackBuilder
 
 
 def intrinsics_rows(intrinsics, n_images: int) -> np.ndarray:
@@ -148,7 +150,8 @@ class HotPathPlan:
 
     def __init__(self, bank: DescriptorBank, max_pairs: int, *, ratio=0.75, ratio_mode="cv2_f32", mutual=False,
                  thr=3.0, confidence=0.99, max_iters=2000, solver="7pt", score="sym_epipolar", lo=False, seed=0,
-                 min_inliers=0, prefilter=True, homography=False, intrinsics=None, distance_thresh=50.0, h_stop_ratio=0.8, overlap=True):
+                 min_inliers=0, prefilter=True, homography=False, intrinsics=None, distance_thresh=50.0, h_stop_ratio=0.8, overlap=True,
+                 tracks=False, track_flags="inlier", min_pair_inliers=15, min_length=2, keep_conflicts=False):
         if bank.metric != "l2":
             raise ValueError("the verification path needs an L2 bank")
         self.bank, self.B, self.cap, self.dev = bank, int(max_pairs), bank.feat_stride, bank.device
@@ -191,6 +194,15 @@ class HotPathPlan:
             self.intr = torch.as_tensor(intrinsics_rows(intrinsics, bank.max_images)).to(dev)
         self.dist = float(distance_thresh)
         self.outputs = outputs(self.homography, self.intr is not None)
+        # feature tracks of a job (per job, not per pair or row: no entry in OUTPUTS): every batch's rows are hooked on the
+        # stream that verified them, before its output set can be reused; match_and_verify begins and finalizes
+        self.tracks = None
+        if tracks:
+            if track_flags not in FLAG_FIELDS or (track_flags is not None and track_flags not in [o.name for o in self.outputs]):
+                raise ValueError(f"track_flags {track_flags!r} is not a row array of this plan ({[o.name for o in self.outputs if o.per == 'row']})")
+            self.track_flags = track_flags
+            self.tracks = TrackBuilder(bank.max_images, bank.max_feats, dev, min_pair_inliers=min_pair_inliers, min_length=min_length,
+                                       keep_conflicts=keep_conflicts)
         self.sets = [_OutSet(B, cap, dev, self.outputs)]                        # the second set is created on the first multi-batch job
         self.cur = self.sets[0]
         self._n_launched = 0
@@ -280,6 +292,9 @@ class HotPathPlan:
             _lib.check(L.sfm_two_view_pose_packed(_lib.ptr(o.corr), _lib.ptr(o.offsets), P, _lib.ptr(o.inlier), _lib.ptr(o.F),
                                                   _lib.ptr(cam), self.dist, _lib.ptr(o.R), _lib.ptr(o.t), None, _lib.ptr(o.n_pose),
                                                   _lib.ptr(o.in_front), _lib.ptr(o.points3d), st), "sfm_two_view_pose_packed")
+        if self.tracks is not None:
+            self.tracks.hook(pairs_d, o.offsets, o.n_matches, o.matches,
+                             None if self.track_flags is None else getattr(o, self.track_flags), o.n_inliers)
         o.ev_done.record(cur)
 
     def result_stream(self):
