@@ -388,6 +388,60 @@ int sfm_tracks_hook(int n_images, int S, const int32_t* pairs, int n_pairs, cons
 int sfm_tracks_finalize(int n_images, int S, const sfm_track_params* params, void* workspace, size_t workspace_bytes,
                         int32_t* track_of, int64_t* offsets, int32_t* obs, int64_t* counts, void* stream);
 
+/* ------------------------------------------------------------ track triangulation
+ * One 3-D point per feature track from known cameras: what known-pose reconstruction (calibrated rigs, poses from GPS /
+ * IMU) computes, and what incremental registration calls after every image it adds.  Cameras follow x ~ K (R X + t),
+ * X in world coordinates (the two-view step's frame when camera 1 is [I|0]).
+ *
+ *   offsets, obs, track_counts   the tracks exactly as sfm_tracks_finalize writes them; the track count is read from
+ *                                track_counts[0] on the device, clamped to max_tracks (the capacity of offsets - 1 and of
+ *                                the per-track outputs), so nothing waits for the host
+ *   xy         float  [n_images, xy_stride, 2]   keypoint pixel coordinates (a bank's xy section); S <= xy_stride
+ *   cams       double [n_images, 16]             fx fy cx cy, R (row-major), t
+ *   registered uint8  [n_images] or NULL         observations in images with registered[i] == 0 are not used (NULL = all)
+ *
+ * Per track k, over its M usable observations (registered images, in obs order), all in fp64:
+ *   normalised coordinates  x^ = ((double)x - cx) / fx, y^ = ((double)y - cy) / fy
+ *   DLT rows                x^ r3 - r1 and y^ r3 - r2 of [R|t], added serially in row order to the 4 x 4 normal matrix;
+ *                           the point is its eigenvector of the smallest eigenvalue (6 cyclic Jacobi sweeps), divided by
+ *                           w when |w| > 1e-300
+ *   reprojection            p = R X + t; the squared error is ((p0 * (1/p2) - x^) * fx)^2 + ((p1 * (1/p2) - y^) * fy)^2;
+ *                           an observation is an inlier iff p2 > 0 and that error <= max_error^2
+ *   hypotheses              the DLT of observations draw_sample(seed, k, h, 2, M) (the RANSAC kernels' sampler; rows of
+ *                           the earlier observation first), kept iff both depths are > 0 and the cosine of the angle
+ *                           between X - C_a and X - C_b (C = -R^T t) is <= cos(min_angle).  Batches of 32, 32, 64, 128, ...
+ *                           hypotheses, the RANSAC stop rule after each batch, at most max_iters; a hypothesis replaces
+ *                           the best only with strictly more inliers
+ *   refit                   at most 2 rounds of the N-view DLT over the current inliers; kept iff it has at least as many
+ *   status                  0 triangulated, 1 too few views (M < 2), 2 no hypothesis kept, 3 fewer than min_inliers
+ *                           inliers, 4 an observation names an image outside [0, n_images) or a feature outside [0, S)
+ *                           (the track is counted and none of its coordinates are read)
+ * Outputs:
+ *   out_X           double [max_tracks, 3]   zeros unless status 0
+ *   out_n_inliers   int32  [max_tracks]      inliers of the final point (status 0 and 3), else 0
+ *   out_status      uint8  [max_tracks]
+ *   out_obs_inlier  uint8  [obs]             per observation, in obs order (0 unless status 0)
+ *   out_obs_error   float  [obs]             pixel reprojection error of the final point; +inf behind the camera, NaN in
+ *                                            unregistered images and for tracks without a point.  The kernel also uses a
+ *                                            track's slice as scratch for observations beyond the shared-memory stage
+ *   out_counts      int64  [5]               tracks per status
+ * Bit-identical to oracle/triangulate.c.  One launch (after a memset of out_counts).
+ */
+typedef struct {
+    double   max_error;    /* pixels, > 0 (COLMAP's mapper filter default: 4)         */
+    double   min_angle;    /* degrees, in [0, 90) (COLMAP's default: 1.5)             */
+    double   confidence;   /* adaptive stop; >= 1.0 disables it                        */
+    uint64_t seed;
+    int32_t  max_iters;    /* hypothesis budget per track, > 0                         */
+    int32_t  min_inliers;  /* >= 2                                                     */
+    int32_t  reserved[6];
+} sfm_triangulate_params;
+
+int sfm_triangulate_tracks(int n_images, int S, const int64_t* offsets, const int32_t* obs, const int64_t* track_counts,
+                           int64_t max_tracks, const float* xy, int xy_stride, const double* cams, const uint8_t* registered,
+                           const sfm_triangulate_params* params, double* out_X, int32_t* out_n_inliers, uint8_t* out_status,
+                           uint8_t* out_obs_inlier, float* out_obs_error, int64_t* out_counts, void* stream);
+
 /* ------------------------------------------ result regions in peer memory (multi-GPU gather)
  * Across ranks, the reference's `pair_matches.append(Pair(...))` (code/pipeline.py:43-47) becomes: every rank
  * writes the packed match rows / inlier flags of its pair block straight into a region of the gathering rank's

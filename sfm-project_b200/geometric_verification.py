@@ -207,3 +207,49 @@ def build_tracks(result, n_images, n_features, *, flags="inlier", min_pair_inlie
     start = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64) if len(counts) else np.zeros(0, np.int64)
     return tr.build_tracks_device(np.asarray(pairs, np.int32).reshape(-1, 2), start, counts,
                                   np.concatenate(rows) if rows else np.zeros((0, 3), np.int32), None, None, n_images, n_features, **opts)
+
+
+# ------------------------------------------------------------------ track triangulation (tracks + cameras -> points)
+def triangulate_tracks(tracks, keypoints, K, R, t, *, registered=None, max_error=4.0, min_angle=1.5, max_iters=500, confidence=0.999,
+                       seed=0, min_inliers=2):
+    """One world point per feature track from known cameras ``x ~ K (R X + t)`` (csrc/triangulate.cu): two-view DLT
+    hypotheses sampled RANSAC-style, kept when both depths are positive and the rays meet at ``min_angle`` degrees or more,
+    scored by pixel reprojection error (an observation is an inlier within ``max_error`` pixels, in front of its camera), the
+    best refit by an N-view DLT over its inliers.  The defaults of ``max_error`` and ``min_angle`` are COLMAP's mapper filter
+    defaults.
+
+    ``tracks``     ``sfm_b200.Tracks`` (device, e.g. ``match_and_verify(..., tracks=True).tracks``; nothing waits for the host) or
+                   its ``to_host()`` dict
+    ``keypoints``  the ``DescriptorBank`` the tracks were built from (its ``xy`` is read in place) or an [n_images, S, 2] array
+    ``K``          one 3x3 pinhole matrix or [n,3,3]; ``R`` [n,3,3]; ``t`` [n,3] -- camera i observes image i
+    ``registered`` bool / uint8 [n] or None: observations in images whose entry is 0 are not used
+    Returns ``sfm_b200.TrackPoints`` (device; ``.to_host()`` for numpy): ``X``, ``n_inliers``, ``status`` per track (0 triangulated,
+    1 too few views, 2 no model, 3 too few inliers, 4 invalid observation), ``obs_inlier`` and ``obs_error`` per observation."""
+    from sfm_b200 import tracks as tr
+    from sfm_b200 import triangulate as tri
+
+    cams = tri.camera_table(K, R, t)
+    n = cams.shape[0]
+    if isinstance(tracks, dict):
+        dev = torch.device("cuda", torch.cuda.current_device())
+        counts = torch.tensor([tracks[k] for k in tr.COUNT_NAMES], dtype=torch.int64)
+        tracks = tr.Tracks(offsets_buf=torch.as_tensor(np.asarray(tracks["offsets"], np.int64)).to(dev),
+                           obs_buf=torch.as_tensor(np.asarray(tracks["obs"], np.int32).reshape(-1, 2)).to(dev),
+                           track_of_buf=torch.as_tensor(np.asarray(tracks["track_of"], np.int32)).to(dev), counts_dev=counts.to(dev))
+    elif not isinstance(tracks, tr.Tracks):
+        raise TypeError(f"tracks must be sfm_b200.Tracks or its to_host() dict, got {type(tracks).__name__}")
+    dev = tracks.obs_buf.device
+    if isinstance(keypoints, _sfm.DescriptorBank):
+        if keypoints.device != dev:
+            raise ValueError(f"the bank lives on {keypoints.device}, the tracks on {dev}")
+        if n > keypoints.max_images:
+            raise ValueError(f"{n} cameras for a bank of {keypoints.max_images} images")
+        xy, S = keypoints.xy[:n], keypoints.max_feats
+    else:
+        a = np.asarray(keypoints)
+        if a.ndim != 3 or a.shape[2] != 2 or a.shape[0] != n:
+            raise ValueError(f"keypoints must be [{n}, S, 2], got {a.shape}")
+        xy, S = torch.from_numpy(np.ascontiguousarray(a, np.float32)).to(dev), a.shape[1]
+    reg = None if registered is None else (np.asarray(registered).reshape(-1) != 0).astype(np.uint8)
+    return tri.triangulate_tracks_device(tracks, xy, torch.from_numpy(cams).to(dev), reg, S=S, max_error=max_error, min_angle=min_angle,
+                                         max_iters=max_iters, confidence=confidence, seed=seed, min_inliers=min_inliers)

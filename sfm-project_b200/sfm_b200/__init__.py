@@ -12,4 +12,5 @@ from .pipeline import VerifiedPairs, get_plan, match_and_verify, match_and_verif
 from .plan import HotPathPlan  # noqa: F401
 from .ransac import VerifyBatch, verify_corr  # noqa: F401
 from .tracks import Tracks, build_tracks_device  # noqa: F401
+from .triangulate import TrackPoints, triangulate_tracks_device  # noqa: F401
 from .pairs import Pair, blocked_exhaustive_pairs, exhaustive_pairs, ordered_pairs, to_reference_pairs, windowed_pairs  # noqa: F401

@@ -27,12 +27,14 @@ class Scene:
     xy     float32[n_images, n_feats, 2]     keypoint pixel coordinates
     point  int32  [n_images, n_feats]        scene-point id of each feature, -1 = clutter
     P      float64[n_images, 3, 4]           camera matrices K[R|t]
+    X      float64[n_points, 3]              world coordinates of the scene points (``point`` indexes them)
     """
 
     desc: np.ndarray
     xy: np.ndarray
     point: np.ndarray
     P: np.ndarray
+    X: np.ndarray | None = None
 
     @property
     def n_images(self) -> int:
@@ -139,7 +141,7 @@ def make_scene(
         desc[k, s_cl] = sift_like(rng, n_cl, dim)
         xy[k, s_cl, 0] = rng.uniform(0, IMG_W, n_cl).astype(np.float32)
         xy[k, s_cl, 1] = rng.uniform(0, IMG_H, n_cl).astype(np.float32)
-    return Scene(desc=desc, xy=xy, point=point, P=Ps)
+    return Scene(desc=desc, xy=xy, point=point, P=Ps, X=X[:, :3].copy())
 
 
 def exhaustive_pairs(n_images: int) -> np.ndarray:
