@@ -442,6 +442,69 @@ int sfm_triangulate_tracks(int n_images, int S, const int64_t* offsets, const in
                            const sfm_triangulate_params* params, double* out_X, int32_t* out_n_inliers, uint8_t* out_status,
                            uint8_t* out_obs_inlier, float* out_obs_error, int64_t* out_counts, void* stream);
 
+/* ------------------------------------------------------------ absolute pose / registration
+ * A camera pose from 2-D / 3-D correspondences: the step of incremental reconstruction that registers a new image against
+ * the points triangulated so far.  Cameras follow x ~ K (R X + t), as in track triangulation.
+ *
+ * sfm_pnp_gather: the correspondences of n_query images.  For query q, they are the features f of image[q] (f ascending)
+ * whose track k = track_of[image[q] * S + f] satisfies 0 <= k < min(track_counts[0], max_tracks) and point_status[k] == 0:
+ *   track_of, track_counts   as sfm_tracks_finalize writes them (the track count is read on the device)
+ *   point_status, X          uint8 [max_tracks], double [max_tracks, 3]: as sfm_triangulate_tracks writes them
+ *   xy                       float [n_images, xy_stride, 2]   keypoint pixel coordinates; S <= xy_stride
+ * Outputs in the strided layout of sfm_pnp_ransac with stride S (query q owns entries [q * S, q * S + out_count[q])):
+ *   out_xy float [n_query, S, 2], out_X double [n_query, S, 3], out_feature int32 [n_query, S], out_count int32 [n_query].
+ * An image outside [0, n_images) gets out_count 0.  Entries past out_count[q] are not written.  One launch.
+ *
+ * sfm_pnp_ransac: one pose per query from the first count[q] (clamped to stride) correspondences of query q:
+ *   cams    double [n_images, 16]   fx fy cx cy ... (the table track triangulation reads); row image[q] gives the intrinsics
+ *   xy      float  [n_query, stride, 2]   pixel coordinates;  X  double [n_query, stride, 3]   world points
+ * All in fp64 with IEEE basic operations and sqrt only:
+ *   normalised coordinates  x^ = ((double)x - cx) / fx, y^ = ((double)y - cy) / fy
+ *   inlier                  p = R X + t, p2 > 0 and ((p0 * (1/p2) - x^) * fx)^2 + ((p1 * (1/p2) - y^) * fy)^2 <= max_error^2
+ *                           (track triangulation's predicate, so a pose and a point agree on what an inlier is)
+ *   hypotheses              the correspondences draw_sample(seed, image[q], h, 3, M) (the RANSAC kernels' sampler; the
+ *                           image id is the stream id, so a query's bits do not depend on its batch), solved by Lambda Twist
+ *                           P3P (Persson & Nordberg, ECCV 2018): the cubic's root by Newton iterations, the 3 x 3 symmetric
+ *                           eigenproblem by 8 cyclic Jacobi sweeps, at most 5 Gauss-Newton steps on the depths, R from a
+ *                           3 x 3 inverse; up to 4 poses per sample in a fixed root order, a root dropped when a depth is
+ *                           not > 0 or R, t is not finite.  Batches of 32, 32, 64, 128, ... hypotheses, the RANSAC stop rule
+ *                           (m = 3) after each, at most max_iters; a pose replaces the best only with strictly more inliers,
+ *                           in (hypothesis, root) order
+ *   refinement              when refine_iters > 0, at most 2 rounds while the pose has >= 3 inliers: at most refine_iters
+ *                           Gauss-Newton steps on the pixel residuals of the round's inliers (sums over 256 lanes, each lane
+ *                           in correspondence order, then a fixed tree; the 6 x 6 normal equations by Cholesky; the rotation
+ *                           update the normalised quaternion (1, w/2), applied on the left), a step taken only if the cost
+ *                           drops; the round's pose is kept iff it moved and has at least as many inliers
+ *   status                  0 registered, 1 fewer than 3 correspondences, 2 no pose from any sample, 3 fewer inliers than
+ *                           min_inliers or min_inlier_ratio * M, 4 image outside [0, n_images) or a focal length that is not
+ *                           positive and finite (the query is counted and none of its correspondences are read)
+ * Outputs:
+ *   out_pose       double [n_query, 12]      R (row-major), t: drops into cams[image, 4:]; zeros unless status 0
+ *   out_n_inliers  int32  [n_query]          inliers of the final pose (status 0 and 3), else 0
+ *   out_status     uint8  [n_query]
+ *   out_mask       uint8  [n_query, stride]  inlier flags of the final pose (0 unless status 0); used as scratch
+ *   out_iters      int32  [n_query] or NULL  hypotheses drawn
+ *   out_counts     int64  [5]                queries per status
+ * Bit-identical to oracle/pnp.c.  One launch (after a memset of out_counts).
+ */
+typedef struct {
+    double   max_error;         /* pixels, > 0 (COLMAP's IncrementalMapper abs_pose_max_error: 12)                 */
+    double   confidence;        /* adaptive stop; >= 1.0 disables it                                               */
+    uint64_t seed;
+    int32_t  max_iters;         /* hypothesis budget per query, > 0                                                */
+    int32_t  min_inliers;       /* >= 3 (COLMAP's abs_pose_min_num_inliers: 30)                                    */
+    double   min_inlier_ratio;  /* in [0, 1] (COLMAP's abs_pose_min_inlier_ratio: 0.25)                            */
+    int32_t  refine_iters;      /* Gauss-Newton steps per refinement round, in [0, 1000]; 0 = no refinement        */
+    int32_t  reserved[5];
+} sfm_pnp_params;
+
+int sfm_pnp_gather(int n_images, int S, const int32_t* track_of, const int64_t* track_counts, int64_t max_tracks,
+                   const uint8_t* point_status, const double* X, const float* xy, int xy_stride, const int32_t* image, int n_query,
+                   float* out_xy, double* out_X, int32_t* out_feature, int32_t* out_count, void* stream);
+int sfm_pnp_ransac(int n_images, const double* cams, const int32_t* image, int n_query, const float* xy, const double* X, int stride,
+                   const int32_t* count, const sfm_pnp_params* params, double* out_pose, int32_t* out_n_inliers, uint8_t* out_status,
+                   uint8_t* out_mask, int32_t* out_iters, int64_t* out_counts, void* stream);
+
 /* ------------------------------------------ result regions in peer memory (multi-GPU gather)
  * Across ranks, the reference's `pair_matches.append(Pair(...))` (code/pipeline.py:43-47) becomes: every rank
  * writes the packed match rows / inlier flags of its pair block straight into a region of the gathering rank's

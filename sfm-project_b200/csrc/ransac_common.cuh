@@ -287,6 +287,41 @@ static __device__ bool should_stop(int best, int M, int m, int done, double conf
     return res <= (1.0 - confidence);
 }
 
+// A calibrated camera x ~ K (R X + t) with K's focal lengths; the principal point is applied to the observations instead
+// (normalised coordinates x^ = (x - cx) / fx).  Shared by track triangulation (triangulate.cu) and registration (pnp.cu).
+struct Camera {
+    double fx, fy, r[9], t[3];
+};
+
+// One row of a [n, 16] camera table: fx fy cx cy, R (row-major), t
+static __device__ __forceinline__ void load_camera(const double* __restrict__ c, Camera& K)
+{
+    K.fx = __ldg(c + 0);
+    K.fy = __ldg(c + 1);
+#pragma unroll
+    for (int i = 0; i < 9; ++i) K.r[i] = __ldg(c + 4 + i);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) K.t[i] = __ldg(c + 13 + i);
+}
+
+// Squared pixel reprojection error (e2 = +inf behind the camera); inlier iff in front and e2 <= thr2.  A triangulated point
+// and a registered pose agree on what an inlier observation is because both use this predicate.
+static __device__ __forceinline__ bool reproject(const Camera& K, const double* X, double x, double y, double thr2, double& e2)
+{
+    const double p0 = K.r[0] * X[0] + K.r[1] * X[1] + K.r[2] * X[2] + K.t[0];
+    const double p1 = K.r[3] * X[0] + K.r[4] * X[1] + K.r[5] * X[2] + K.t[1];
+    const double p2 = K.r[6] * X[0] + K.r[7] * X[1] + K.r[8] * X[2] + K.t[2];
+    if (!(p2 > 0.0)) {
+        e2 = __longlong_as_double(0x7ff0000000000000ll);
+        return false;
+    }
+    const double iz = 1.0 / p2;
+    const double ex = (p0 * iz - x) * K.fx;
+    const double ey = (p1 * iz - y) * K.fy;
+    e2 = ex * ex + ey * ey;
+    return e2 <= thr2;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Cooperative Gauss-Jordan elimination with complete pivoting: 8 lanes (one aligned octet of a warp) reduce ONE
 // m x 9 system, lane r holding row r in registers (a[0..8], statically indexed).  Value for value the serial

@@ -64,20 +64,6 @@ struct TriTrack {
     }
 };
 
-struct Camera {
-    double fx, fy, r[9], t[3];
-};
-
-static __device__ __forceinline__ void load_camera(const double* __restrict__ c, Camera& K)
-{
-    K.fx = __ldg(c + 0);
-    K.fy = __ldg(c + 1);
-#pragma unroll
-    for (int i = 0; i < 9; ++i) K.r[i] = __ldg(c + 4 + i);
-#pragma unroll
-    for (int i = 0; i < 3; ++i) K.t[i] = __ldg(c + 13 + i);
-}
-
 struct Normal {
     double g[10];                       // upper triangle of the 4 x 4 normal matrix, row by row
 };
@@ -145,23 +131,6 @@ static __device__ __noinline__ Point solve_point(Normal N)
 static __device__ __forceinline__ double depth(const Camera& K, const double* X)
 {
     return K.r[6] * X[0] + K.r[7] * X[1] + K.r[8] * X[2] + K.t[2];
-}
-
-// Squared pixel reprojection error (e2 = +inf behind the camera); inlier iff in front and e2 <= thr2.
-static __device__ __forceinline__ bool reproject(const Camera& K, const double* X, double x, double y, double thr2, double& e2)
-{
-    const double p0 = K.r[0] * X[0] + K.r[1] * X[1] + K.r[2] * X[2] + K.t[0];
-    const double p1 = K.r[3] * X[0] + K.r[4] * X[1] + K.r[5] * X[2] + K.t[1];
-    const double p2 = K.r[6] * X[0] + K.r[7] * X[1] + K.r[8] * X[2] + K.t[2];
-    if (!(p2 > 0.0)) {
-        e2 = __longlong_as_double(0x7ff0000000000000ll);
-        return false;
-    }
-    const double iz = 1.0 / p2;
-    const double ex = (p0 * iz - x) * K.fx;
-    const double ey = (p1 * iz - y) * K.fy;
-    e2 = ex * ex + ey * ey;
-    return e2 <= thr2;
 }
 
 // C = -R^T t

@@ -210,6 +210,35 @@ def build_tracks(result, n_images, n_features, *, flags="inlier", min_pair_inlie
 
 
 # ------------------------------------------------------------------ track triangulation (tracks + cameras -> points)
+def _device_tracks(tracks):
+    """``sfm_b200.Tracks`` as given, or uploaded from its ``to_host()`` dict."""
+    from sfm_b200 import tracks as tr
+
+    if isinstance(tracks, dict):
+        dev = torch.device("cuda", torch.cuda.current_device())
+        counts = torch.tensor([tracks[k] for k in tr.COUNT_NAMES], dtype=torch.int64)
+        return tr.Tracks(offsets_buf=torch.as_tensor(np.asarray(tracks["offsets"], np.int64)).to(dev),
+                         obs_buf=torch.as_tensor(np.asarray(tracks["obs"], np.int32).reshape(-1, 2)).to(dev),
+                         track_of_buf=torch.as_tensor(np.asarray(tracks["track_of"], np.int32)).to(dev), counts_dev=counts.to(dev))
+    if not isinstance(tracks, tr.Tracks):
+        raise TypeError(f"tracks must be sfm_b200.Tracks or its to_host() dict, got {type(tracks).__name__}")
+    return tracks
+
+
+def _keypoints(keypoints, n, dev):
+    """(xy float32 [n, S, 2] on dev, S) of a ``DescriptorBank`` (its xy, in place) or an [n, S, 2] array."""
+    if isinstance(keypoints, _sfm.DescriptorBank):
+        if keypoints.device != dev:
+            raise ValueError(f"the bank lives on {keypoints.device}, the tracks on {dev}")
+        if n > keypoints.max_images:
+            raise ValueError(f"{n} cameras for a bank of {keypoints.max_images} images")
+        return keypoints.xy[:n], keypoints.max_feats
+    a = np.asarray(keypoints)
+    if a.ndim != 3 or a.shape[2] != 2 or a.shape[0] != n:
+        raise ValueError(f"keypoints must be [{n}, S, 2], got {a.shape}")
+    return torch.from_numpy(np.ascontiguousarray(a, np.float32)).to(dev), a.shape[1]
+
+
 def triangulate_tracks(tracks, keypoints, K, R, t, *, registered=None, max_error=4.0, min_angle=1.5, max_iters=500, confidence=0.999,
                        seed=0, min_inliers=2):
     """One world point per feature track from known cameras ``x ~ K (R X + t)`` (csrc/triangulate.cu): two-view DLT
@@ -225,31 +254,87 @@ def triangulate_tracks(tracks, keypoints, K, R, t, *, registered=None, max_error
     ``registered`` bool / uint8 [n] or None: observations in images whose entry is 0 are not used
     Returns ``sfm_b200.TrackPoints`` (device; ``.to_host()`` for numpy): ``X``, ``n_inliers``, ``status`` per track (0 triangulated,
     1 too few views, 2 no model, 3 too few inliers, 4 invalid observation), ``obs_inlier`` and ``obs_error`` per observation."""
-    from sfm_b200 import tracks as tr
     from sfm_b200 import triangulate as tri
 
     cams = tri.camera_table(K, R, t)
     n = cams.shape[0]
-    if isinstance(tracks, dict):
-        dev = torch.device("cuda", torch.cuda.current_device())
-        counts = torch.tensor([tracks[k] for k in tr.COUNT_NAMES], dtype=torch.int64)
-        tracks = tr.Tracks(offsets_buf=torch.as_tensor(np.asarray(tracks["offsets"], np.int64)).to(dev),
-                           obs_buf=torch.as_tensor(np.asarray(tracks["obs"], np.int32).reshape(-1, 2)).to(dev),
-                           track_of_buf=torch.as_tensor(np.asarray(tracks["track_of"], np.int32)).to(dev), counts_dev=counts.to(dev))
-    elif not isinstance(tracks, tr.Tracks):
-        raise TypeError(f"tracks must be sfm_b200.Tracks or its to_host() dict, got {type(tracks).__name__}")
+    tracks = _device_tracks(tracks)
     dev = tracks.obs_buf.device
-    if isinstance(keypoints, _sfm.DescriptorBank):
-        if keypoints.device != dev:
-            raise ValueError(f"the bank lives on {keypoints.device}, the tracks on {dev}")
-        if n > keypoints.max_images:
-            raise ValueError(f"{n} cameras for a bank of {keypoints.max_images} images")
-        xy, S = keypoints.xy[:n], keypoints.max_feats
-    else:
-        a = np.asarray(keypoints)
-        if a.ndim != 3 or a.shape[2] != 2 or a.shape[0] != n:
-            raise ValueError(f"keypoints must be [{n}, S, 2], got {a.shape}")
-        xy, S = torch.from_numpy(np.ascontiguousarray(a, np.float32)).to(dev), a.shape[1]
+    xy, S = _keypoints(keypoints, n, dev)
     reg = None if registered is None else (np.asarray(registered).reshape(-1) != 0).astype(np.uint8)
     return tri.triangulate_tracks_device(tracks, xy, torch.from_numpy(cams).to(dev), reg, S=S, max_error=max_error, min_angle=min_angle,
                                          max_iters=max_iters, confidence=confidence, seed=seed, min_inliers=min_inliers)
+
+
+# ------------------------------------------------------------------ registration (2-D / 3-D correspondences -> camera pose)
+def estimate_absolute_poses(points2d, points3d, K, *, max_error=12.0, confidence=0.9999, max_iters=10000, min_inliers=30,
+                            min_inlier_ratio=0.25, refine_iters=10, seed=0):
+    """Batched ``cv2.solvePnPRansac`` + ``cv2.solvePnPRefineLM`` for calibrated pinhole cameras (csrc/pnp.cu): RANSAC over Lambda
+    Twist P3P samples, an observation an inlier within ``max_error`` pixels in front of the camera, the best pose refined by
+    Gauss-Newton on its inliers.  ``points2d`` / ``points3d`` are lists of [M_k, 2] pixel and [M_k, 3] world arrays, ``K`` one 3x3
+    or [P,3,3].  The defaults of ``max_error``, ``min_inliers`` and ``min_inlier_ratio`` are COLMAP's incremental-mapper ones.
+    Returns a list of ``(n_inliers, R float64[3,3], t float64[3], mask uint8[M_k,1])`` with x ~ K (R X + t); ``n_inliers == 0``
+    means no pose (R and t are then zero)."""
+    from sfm_b200 import pnp
+    from sfm_b200 import triangulate as tri
+
+    P = len(points2d)
+    if len(points3d) != P:
+        raise ValueError(f"{P} point sets of 2-D points, {len(points3d)} of 3-D points")
+    if P == 0:
+        return []
+    p2 = [np.asarray(p, np.float64).reshape(-1, 2) for p in points2d]
+    p3 = [np.asarray(p, np.float64).reshape(-1, 3) for p in points3d]
+    counts = np.array([len(p) for p in p2], np.int32)
+    if any(len(a) != len(b) for a, b in zip(p2, p3)):
+        raise ValueError("every 2-D point set must have as many points as its 3-D set")
+    cams = tri.camera_table(K, np.tile(np.eye(3), (P, 1, 1)), np.zeros((P, 3)))
+    stride = max(int(counts.max()), 1)
+    xy = np.zeros((P, stride, 2), np.float32)
+    X = np.zeros((P, stride, 3), np.float64)
+    for k in range(P):
+        xy[k, : counts[k]] = p2[k]
+        X[k, : counts[k]] = p3[k]
+    dev = torch.device("cuda", torch.cuda.current_device())
+    res = pnp.pnp_ransac_device(torch.from_numpy(xy).to(dev), torch.from_numpy(X).to(dev), torch.from_numpy(counts).to(dev),
+                                torch.from_numpy(cams).to(dev), np.arange(P, dtype=np.int32), max_error=max_error, confidence=confidence,
+                                max_iters=max_iters, min_inliers=min_inliers, min_inlier_ratio=min_inlier_ratio, refine_iters=refine_iters,
+                                seed=seed).to_host()
+    ok = res["status"] == 0
+    return [(int(res["n_inliers"][k]) if ok[k] else 0, res["R"][k].copy(), res["t"][k].copy(), res["mask"][k, : counts[k]].reshape(-1, 1).copy())
+            for k in range(P)]
+
+
+def estimate_absolute_pose(pts2d, pts3d, K, **kw):
+    """Single-set form: ``(n_inliers, R, t, mask)``."""
+    return estimate_absolute_poses([pts2d], [pts3d], K, **kw)[0]
+
+
+def register_images(tracks, points, keypoints, K, R, t, images, *, registered=None, max_error=12.0, confidence=0.9999, max_iters=10000,
+                    min_inliers=30, min_inlier_ratio=0.25, refine_iters=10, seed=0):
+    """Register ``images`` against triangulated tracks (csrc/pnp.cu): the correspondences of image i are its features whose track
+    has a point (``points``, from ``triangulate_tracks``), in feature order; the pose as ``estimate_absolute_poses``.
+
+    ``tracks``, ``keypoints``, ``K``, ``R``, ``t`` as ``triangulate_tracks`` (only the intrinsics of ``images`` are read);
+    ``registered`` None or a bool / uint8 [n] array or tensor, set to 1 in place for every image registered here.  Returns
+    ``sfm_b200.AbsolutePoses`` (device; ``.to_host()`` for numpy): ``R``, ``t``, ``n_inliers``, ``status`` per image (0 registered,
+    1 fewer than 3 points, 2 no model, 3 too few inliers, 4 invalid image), ``mask`` and ``feature`` per correspondence."""
+    from sfm_b200 import pnp
+    from sfm_b200 import triangulate as tri
+
+    cams = tri.camera_table(K, R, t)
+    n = cams.shape[0]
+    tracks = _device_tracks(tracks)
+    dev = tracks.obs_buf.device
+    xy, _ = _keypoints(keypoints, n, dev)
+    res = pnp.register_images_device(tracks, points, xy, torch.from_numpy(cams).to(dev), images, max_error=max_error, confidence=confidence,
+                                     max_iters=max_iters, min_inliers=min_inliers, min_inlier_ratio=min_inlier_ratio,
+                                     refine_iters=refine_iters, seed=seed)
+    if registered is not None:
+        ok = res.status == 0
+        img = res.images.long()[ok]
+        if isinstance(registered, torch.Tensor):
+            registered[img.to(registered.device)] = 1
+        else:
+            registered[img.cpu().numpy()] = 1
+    return res

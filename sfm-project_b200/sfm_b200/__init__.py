@@ -13,4 +13,5 @@ from .plan import HotPathPlan  # noqa: F401
 from .ransac import VerifyBatch, verify_corr  # noqa: F401
 from .tracks import Tracks, build_tracks_device  # noqa: F401
 from .triangulate import TrackPoints, triangulate_tracks_device  # noqa: F401
+from .pnp import AbsolutePoses, pnp_ransac_device, register_images_device  # noqa: F401
 from .pairs import Pair, blocked_exhaustive_pairs, exhaustive_pairs, ordered_pairs, to_reference_pairs, windowed_pairs  # noqa: F401
