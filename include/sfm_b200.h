@@ -402,9 +402,10 @@ int sfm_tracks_finalize(int n_images, int S, const sfm_track_params* params, voi
  *
  * Per track k, over its M usable observations (registered images, in obs order), all in fp64:
  *   normalised coordinates  x^ = ((double)x - cx) / fx, y^ = ((double)y - cy) / fy
- *   DLT rows                x^ r3 - r1 and y^ r3 - r2 of [R|t], added serially in row order to the 4 x 4 normal matrix;
- *                           the point is its eigenvector of the smallest eigenvalue (6 cyclic Jacobi sweeps), divided by
- *                           w when |w| > 1e-300
+ *   DLT rows                (x^ r3 - r1) * fx and (y^ r3 - r2) * fy of [R|t], added serially in row order to the 4 x 4
+ *                           normal matrix; the point is its eigenvector of the smallest eigenvalue (6 cyclic Jacobi
+ *                           sweeps), divided by w when |w| > 1e-300.  The focal lengths make each row a pixel residual
+ *                           times the depth, so the views of different cameras weigh alike
  *   reprojection            p = R X + t; the squared error is ((p0 * (1/p2) - x^) * fx)^2 + ((p1 * (1/p2) - y^) * fy)^2;
  *                           an observation is an inlier iff p2 > 0 and that error <= max_error^2
  *   hypotheses              the DLT of observations draw_sample(seed, k, h, 2, M) (the RANSAC kernels' sampler; rows of
@@ -472,9 +473,12 @@ int sfm_triangulate_tracks(int n_images, int S, const int64_t* offsets, const in
  *                           in (hypothesis, root) order
  *   refinement              when refine_iters > 0, at most 2 rounds while the pose has >= 3 inliers: at most refine_iters
  *                           Gauss-Newton steps on the pixel residuals of the round's inliers (sums over 256 lanes, each lane
- *                           in correspondence order, then a fixed tree; the 6 x 6 normal equations by Cholesky; the rotation
- *                           update the normalised quaternion (1, w/2), applied on the left), a step taken only if the cost
- *                           drops; the round's pose is kept iff it moved and has at least as many inliers
+ *                           in correspondence order, then a fixed tree; the 6 x 6 normal equations by Cholesky), perturbing
+ *                           the pose in the camera frame: R' = dR R, t' = dR t + dt with dR the normalised quaternion
+ *                           (1, w/2) and the Jacobian taken at p = R X + t, so the step's linearisation error scales with
+ *                           the depth and not with |X| (worlds far from their origin refine as well as centred ones); a
+ *                           step taken only if the cost drops; the round's pose is kept iff it moved and has at least as
+ *                           many inliers
  *   status                  0 registered, 1 fewer than 3 correspondences, 2 no pose from any sample, 3 fewer inliers than
  *                           min_inliers or min_inlier_ratio * M, 4 image outside [0, n_images) or a focal length that is not
  *                           positive and finite (the query is counted and none of its correspondences are read)

@@ -226,8 +226,8 @@ static void add_gn(double* v, const pnp_camera* K, double x, double y, const dou
     double ex = (u0 - x) * K->fx, ey = (u1 - y) * K->fy;
     double a0 = K->fx * iz, a2 = -(a0 * u0);
     double b1 = K->fy * iz, b2 = -(b1 * u1);
-    double ju[6] = {a2 * q1, a0 * q2 - a2 * q0, -(a0 * q1), a0, 0.0, a2};
-    double jv[6] = {b2 * q1 - b1 * q2, -(b2 * q0), b1 * q0, 0.0, b1, b2};
+    double ju[6] = {a2 * p1, a0 * p2 - a2 * p0, -(a0 * p1), a0, 0.0, a2};
+    double jv[6] = {b2 * p1 - b1 * p2, -(b2 * p0), b1 * p0, 0.0, b1, b2};
     int e = 0;
     for (int i = 0; i < 6; ++i)
         for (int j = i; j < 6; ++j) {
@@ -284,7 +284,7 @@ static int gn_step(const double* v, const pnp_camera* K, pnp_camera* O)
     O->fx = K->fx; O->fy = K->fy;
     for (int i = 0; i < 3; ++i)
         for (int j = 0; j < 3; ++j) O->r[3 * i + j] = D[3 * i] * K->r[j] + D[3 * i + 1] * K->r[3 + j] + D[3 * i + 2] * K->r[6 + j];
-    for (int i = 0; i < 3; ++i) O->t[i] = K->t[i] + dl[3 + i];
+    for (int i = 0; i < 3; ++i) O->t[i] = (D[3 * i] * K->t[0] + D[3 * i + 1] * K->t[1] + D[3 * i + 2] * K->t[2]) + dl[3 + i];
     return 1;
 }
 

@@ -27,11 +27,11 @@ static void tri_add_rows(double G[10], const tri_camera* K, double x, double y)
 {
     double a[4], b[4];
     for (int c = 0; c < 3; ++c) {
-        a[c] = x * K->r[6 + c] - K->r[0 + c];
-        b[c] = y * K->r[6 + c] - K->r[3 + c];
+        a[c] = (x * K->r[6 + c] - K->r[0 + c]) * K->fx;
+        b[c] = (y * K->r[6 + c] - K->r[3 + c]) * K->fy;
     }
-    a[3] = x * K->t[2] - K->t[0];
-    b[3] = y * K->t[2] - K->t[1];
+    a[3] = (x * K->t[2] - K->t[0]) * K->fx;
+    b[3] = (y * K->t[2] - K->t[1]) * K->fy;
     int e = 0;
     for (int i = 0; i < 4; ++i)
         for (int j = i; j < 4; ++j) {

@@ -342,7 +342,9 @@ static __device__ int block_count(const PnpPts& pts, int M, const Camera& K, dou
 }
 
 // Adds one observation's Gauss-Newton terms at pose K: the upper triangle of J^T J (21, row by row, the u row's product then
-// the v row's), J^T r (6) and the squared error.  J is d(u, v) / d(w, t) for R' = dR(w) R, t' = t + dt.
+// the v row's), J^T r (6) and the squared error.  J is d(u, v) / d(w, t) for the camera-frame perturbation R' = dR(w) R,
+// t' = dR(w) t + dt, taken at p = R X + t: its linearisation error scales with the depth, not with |X|, so the step still
+// lowers the cost when the world is far from its origin.
 static __device__ __forceinline__ void add_gn(double (&v)[kPnpSums], const Camera& K, double x, double y, const double* Xw)
 {
     const double q0 = K.r[0] * Xw[0] + K.r[1] * Xw[1] + K.r[2] * Xw[2];
@@ -354,8 +356,8 @@ static __device__ __forceinline__ void add_gn(double (&v)[kPnpSums], const Camer
     const double ex = (u0 - x) * K.fx, ey = (u1 - y) * K.fy;
     const double a0 = K.fx * iz, a2 = -(a0 * u0);
     const double b1 = K.fy * iz, b2 = -(b1 * u1);
-    const double ju[6] = {a2 * q1, a0 * q2 - a2 * q0, -(a0 * q1), a0, 0.0, a2};
-    const double jv[6] = {b2 * q1 - b1 * q2, -(b2 * q0), b1 * q0, 0.0, b1, b2};
+    const double ju[6] = {a2 * p1, a0 * p2 - a2 * p0, -(a0 * p1), a0, 0.0, a2};
+    const double jv[6] = {b2 * p1 - b1 * p2, -(b2 * p0), b1 * p0, 0.0, b1, b2};
     int e = 0;
 #pragma unroll
     for (int i = 0; i < 6; ++i)
@@ -374,7 +376,7 @@ static __device__ __forceinline__ void add_gn(double (&v)[kPnpSums], const Camer
 }
 
 // The Gauss-Newton step from the sums: Cholesky of J^T J, delta = -(J^T J)^-1 J^T r, R' = dR R with dR the rotation of the
-// normalised quaternion (1, w/2), t' = t + dt.  False when a pivot is not positive.
+// normalised quaternion (1, w/2), t' = dR t + dt.  False when a pivot is not positive.
 static __device__ __forceinline__ bool gn_step(const double (&v)[kPnpSums], const Camera& K, Camera& O)
 {
     double H[36];
@@ -432,7 +434,7 @@ static __device__ __forceinline__ bool gn_step(const double (&v)[kPnpSums], cons
 #pragma unroll
         for (int j = 0; j < 3; ++j) O.r[3 * i + j] = D[3 * i] * K.r[j] + D[3 * i + 1] * K.r[3 + j] + D[3 * i + 2] * K.r[6 + j];
 #pragma unroll
-    for (int i = 0; i < 3; ++i) O.t[i] = K.t[i] + dl[3 + i];
+    for (int i = 0; i < 3; ++i) O.t[i] = (D[3 * i] * K.t[0] + D[3 * i + 1] * K.t[1] + D[3 * i + 2] * K.t[2]) + dl[3 + i];
     return true;
 }
 

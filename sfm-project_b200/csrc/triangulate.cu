@@ -73,18 +73,19 @@ struct Point {
     int ok;
 };
 
-// Adds the two DLT rows of one observation, x^ r3 - r1 and y^ r3 - r2 of [R|t], to the 10 upper-triangle entries of the
-// 4 x 4 normal matrix (row x^ first, then row y^).
+// Adds the two DLT rows of one observation, fx (x^ r3 - r1) and fy (y^ r3 - r2) of [R|t], to the 10 upper-triangle entries
+// of the 4 x 4 normal matrix (row x^ first, then row y^).  The focal lengths make each row's residual about a pixel
+// residual times the depth, so views of different cameras weigh alike; unscaled rows would weigh a view by about 1/f.
 static __device__ __forceinline__ void add_rows(Normal& N, const Camera& K, double x, double y)
 {
     double a[4], b[4];
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        a[c] = x * K.r[6 + c] - K.r[0 + c];
-        b[c] = y * K.r[6 + c] - K.r[3 + c];
+        a[c] = (x * K.r[6 + c] - K.r[0 + c]) * K.fx;
+        b[c] = (y * K.r[6 + c] - K.r[3 + c]) * K.fy;
     }
-    a[3] = x * K.t[2] - K.t[0];
-    b[3] = y * K.t[2] - K.t[1];
+    a[3] = (x * K.t[2] - K.t[0]) * K.fx;
+    b[3] = (y * K.t[2] - K.t[1]) * K.fy;
     int e = 0;
 #pragma unroll
     for (int i = 0; i < 4; ++i)

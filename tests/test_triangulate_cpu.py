@@ -106,9 +106,9 @@ def _batch(done):
     return 32 if done < 64 else (64 if done < 128 else 128)
 
 
-def _dlt(P, x):
-    """SVD of the stacked DLT rows: P [n,3,4] ([R|t]), x [n,2] normalised."""
-    A = np.concatenate([x[:, :1] * P[:, 2] - P[:, 0], x[:, 1:] * P[:, 2] - P[:, 1]])
+def _dlt(P, x, f):
+    """SVD of the stacked DLT rows: P [n,3,4] ([R|t]), x [n,2] normalised, each row scaled by its view's focal length f [n,2]."""
+    A = np.concatenate([(x[:, :1] * P[:, 2] - P[:, 0]) * f[:, :1], (x[:, 1:] * P[:, 2] - P[:, 1]) * f[:, 1:]])
     v = np.linalg.svd(A)[2][-1]
     return None if not abs(v[3]) > 1e-300 else v[:3] / v[3]
 
@@ -143,7 +143,7 @@ def reference_triangulate(offsets, obs, xy, cams, registered, *, max_error, min_
             nb = min(_batch(done), max_iters - done)
             for h in range(done, done + nb):
                 a, b = sorted(_draw_pair(seed, k, h, M))
-                Xh = _dlt(Rt[img[[a, b]]], xn[[a, b]])
+                Xh = _dlt(Rt[img[[a, b]]], xn[[a, b]], f[img[[a, b]]])
                 if Xh is None or not (Rt[img[a], 2, :3] @ Xh + Rt[img[a], 2, 3] > 0) or not (Rt[img[b], 2, :3] @ Xh + Rt[img[b], 2, 3] > 0):
                     continue
                 da, db = Xh - centers[img[a]], Xh - centers[img[b]]
@@ -163,7 +163,7 @@ def reference_triangulate(offsets, obs, xy, cams, registered, *, max_error, min_
             if cur < 2:
                 break
             m = inliers(X)
-            Xr = _dlt(Rt[img[m]], xn[m])
+            Xr = _dlt(Rt[img[m]], xn[m], f[img[m]])
             if Xr is None or inliers(Xr).sum() < cur:
                 break
             X, cur = Xr, int(inliers(Xr).sum())
