@@ -105,19 +105,29 @@ def fast_keypoints(img: np.ndarray):
 
 def harris_responses(img: np.ndarray, xs, ys) -> np.ndarray:
     I = img.astype(np.int64)
+    xs, ys = np.asarray(xs, np.int64), np.asarray(ys, np.int64)
     r = HARRIS_BLOCK // 2
     scale = F32(1.0) / (F32(4 * HARRIS_BLOCK) * F32(255.0))
     s4 = F32(F32(F32(scale * scale) * scale) * scale)
-    out = np.zeros(len(xs), F32)
-    for n, (x0, y0) in enumerate(zip(xs, ys)):
-        P = I[y0 - r - 1: y0 + r + 2, x0 - r - 1: x0 + r + 2]                 # 9 x 9 around the 7 x 7 block
-        Ix = (P[1:-1, 2:] - P[1:-1, :-2]) * 2 + (P[:-2, 2:] - P[:-2, :-2]) + (P[2:, 2:] - P[2:, :-2])
-        Iy = (P[2:, 1:-1] - P[:-2, 1:-1]) * 2 + (P[2:, :-2] - P[:-2, :-2]) + (P[2:, 2:] - P[:-2, 2:])
-        a, b, c = int((Ix * Ix).sum()), int((Iy * Iy).sum()), int((Ix * Iy).sum())
-        fa, fb, fc = F32(a), F32(b), F32(c)
-        t = F32(fa + fb)
-        out[n] = F32(F32(F32(F32(fa * fb) - F32(fc * fc)) - F32(F32(HARRIS_K * t) * t)) * s4)
-    return out
+    o = np.arange(-r - 1, r + 2)
+    P = I[ys[:, None, None] + o[None, :, None], xs[:, None, None] + o[None, None, :]]     # [n, 9, 9] around the 7 x 7 block
+    Ix = (P[:, 1:-1, 2:] - P[:, 1:-1, :-2]) * 2 + (P[:, :-2, 2:] - P[:, :-2, :-2]) + (P[:, 2:, 2:] - P[:, 2:, :-2])
+    Iy = (P[:, 2:, 1:-1] - P[:, :-2, 1:-1]) * 2 + (P[:, 2:, :-2] - P[:, :-2, :-2]) + (P[:, 2:, 2:] - P[:, :-2, 2:])
+    a, b, c = (Ix * Ix).sum((1, 2)), (Iy * Iy).sum((1, 2)), (Ix * Iy).sum((1, 2))
+    fa, fb, fc = a.astype(F32), b.astype(F32), c.astype(F32)
+    t = fa + fb                                                         # float32 arrays: every operation rounds on its own
+    return (((fa * fb) - (fc * fc)) - ((HARRIS_K * t) * t)) * s4
+
+
+def harris_sums(img: np.ndarray, xs, ys) -> np.ndarray:
+    """int64 [n] = a + b of the Harris block (the largest value converted to float32 by the response)."""
+    I = img.astype(np.int64)
+    xs, ys = np.asarray(xs, np.int64), np.asarray(ys, np.int64)
+    o = np.arange(-HARRIS_BLOCK // 2, HARRIS_BLOCK // 2 + 2)
+    P = I[ys[:, None, None] + o[None, :, None], xs[:, None, None] + o[None, None, :]]
+    Ix = (P[:, 1:-1, 2:] - P[:, 1:-1, :-2]) * 2 + (P[:, :-2, 2:] - P[:, :-2, :-2]) + (P[:, 2:, 2:] - P[:, 2:, :-2])
+    Iy = (P[:, 2:, 1:-1] - P[:, :-2, 1:-1]) * 2 + (P[:, 2:, :-2] - P[:, :-2, :-2]) + (P[:, 2:, 2:] - P[:, :-2, 2:])
+    return (Ix * Ix).sum((1, 2)) + (Iy * Iy).sum((1, 2))
 
 
 _P1, _P3, _P5, _P7 = (F32(v) * F32(180.0 / np.pi) for v in (0.9997878412794807, -0.3258083974640975, 0.1555786518463281, -0.04432655554792128))
@@ -143,33 +153,45 @@ def fast_atan2(y: np.ndarray, x: np.ndarray) -> np.ndarray:
     return a.astype(F32)
 
 
-def ic_angles(img: np.ndarray, xs, ys) -> np.ndarray:
+def ic_moments(img: np.ndarray, xs, ys):
+    """int64 (m01, m10): intensity moments of the radius-15 disc (rows v = -15..15 of half-width umax[|v|])."""
     I = img.astype(np.int64)
+    xs, ys = np.asarray(xs, np.int64), np.asarray(ys, np.int64)
     um = umax_table()
-    m01 = np.zeros(len(xs), np.int64)
-    m10 = np.zeros(len(xs), np.int64)
-    u15 = np.arange(-HALF, HALF + 1)
-    for n, (x0, y0) in enumerate(zip(xs, ys)):
-        m10[n] = int((u15 * I[y0, x0 - HALF: x0 + HALF + 1]).sum())
-        for v in range(1, HALF + 1):
-            d = int(um[v])
-            u = np.arange(-d, d + 1)
-            plus, minus = I[y0 + v, x0 - d: x0 + d + 1], I[y0 - v, x0 - d: x0 + d + 1]
-            m01[n] += v * int((plus - minus).sum())
-            m10[n] += int((u * (plus + minus)).sum())
+    du = np.concatenate([np.arange(-um[abs(v)], um[abs(v)] + 1) for v in range(-HALF, HALF + 1)])
+    dv = np.concatenate([np.full(2 * um[abs(v)] + 1, v) for v in range(-HALF, HALF + 1)])
+    vals = I[ys[:, None] + dv[None], xs[:, None] + du[None]]
+    return (vals * dv).sum(1), (vals * du).sum(1)
+
+
+def ic_angles(img: np.ndarray, xs, ys) -> np.ndarray:
+    m01, m10 = ic_moments(img, xs, ys)
     return fast_atan2(m01.astype(F32), m10.astype(F32))
 
 
-def detect(img: np.ndarray, nfeatures: int = 500, n_levels: int = 8, levels=None) -> np.ndarray:
+def level_candidates(levels):
+    """Per level, (x, y, FAST response) of the FAST keypoints at least 31 pixels from the border, row-major: what does not
+    depend on nfeatures, so that several budgets can share it."""
+    out = []
+    for im in levels:
+        h, w = im.shape
+        if h <= 2 * EDGE or w <= 2 * EDGE:
+            out.append((np.zeros(0, np.int32), np.zeros(0, np.int32), np.zeros(0, F32)))
+            continue
+        xs, ys, resp = fast_keypoints(im)
+        inside = (xs >= EDGE) & (xs < w - EDGE) & (ys >= EDGE) & (ys < h - EDGE)
+        out.append((xs[inside], ys[inside], resp[inside]))
+    return out
+
+
+def detect(img: np.ndarray, nfeatures: int = 500, n_levels: int = 8, levels=None, candidates=None) -> np.ndarray:
     """float32 [n, 6] = (pt.x, pt.y, size, angle, response, octave) in cv2's order."""
     levels = orb_oracle.build_pyramid(img, n_levels) if levels is None else levels
+    candidates = level_candidates(levels) if candidates is None else candidates
     per = features_per_level(nfeatures, n_levels)
     rows = []
     for lv, im in enumerate(levels):
-        h, w = im.shape
-        xs, ys, resp = fast_keypoints(im)
-        inside = (xs >= EDGE) & (xs < w - EDGE) & (ys >= EDGE) & (ys < h - EDGE)
-        xs, ys, resp = xs[inside], ys[inside], resp[inside]
+        xs, ys, resp = candidates[lv]
         keep = retain_best(resp, 2 * per[lv])
         xs, ys = xs[keep], ys[keep]
         hr = harris_responses(im, xs, ys)
@@ -177,7 +199,6 @@ def detect(img: np.ndarray, nfeatures: int = 500, n_levels: int = 8, levels=None
         xs, ys, hr = xs[keep], ys[keep], hr[keep]
         ang = ic_angles(im, xs, ys)
         sf = orb_oracle.level_scale(lv)
-        for x, y, r_, a in zip(xs, ys, hr, ang):
-            px, py = (F32(x) * sf, F32(y) * sf) if lv > 0 else (F32(x), F32(y))
-            rows.append((px, py, F32(PATCH) * sf, a, r_, F32(lv)))
-    return np.array(rows, F32).reshape(-1, 6)
+        px, py = (xs.astype(F32) * sf, ys.astype(F32) * sf) if lv > 0 else (xs.astype(F32), ys.astype(F32))
+        rows.append(np.stack([px, py, np.full(len(xs), F32(PATCH) * sf, F32), ang, hr, np.full(len(xs), lv, F32)], 1).astype(F32))
+    return np.concatenate(rows).reshape(-1, 6)

@@ -4,7 +4,8 @@ Follows what ``cv2.ORB_create().detectAndCompute`` (code/feature_matching.py:42-
 as it can be observed from outside (OpenCV 4.13.0; sources not on disk, behaviour pinned by tests/test_oracle_pinned.py
 against cv2 itself):
 
-* pyramid: level k has size (round(w / s_k), round(h / s_k)), s_k = float32(1.2f ** k), and is resized from level k-1 with
+* pyramid: level k has size (round(w * (1 / s_k)), round(h * (1 / s_k))) in float32, s_k = float32(1.2f ** k), round half to
+  even, and is resized from level k-1 with
   INTER_LINEAR_EXACT (taken from cv2.resize here: the GPU stage receives the pyramid, it does not build it);
 * each level is blurred with GaussianBlur(7x7, sigma 2), which for a sub-matrix source is sepFilter2D with the float32
   kernel: rows  s = k[-3] x[-3]; s = fma(k[d], x[d], s), d = -2..3;  columns  s = k[0] x[0]; s = fma(k[d], x[d] + x[-d], s),
@@ -35,8 +36,8 @@ def build_pyramid(img: np.ndarray, n_levels: int = N_LEVELS):
     h, w = img.shape
     levels = [np.ascontiguousarray(img)]
     for k in range(1, n_levels):
-        s = level_scale(k)
-        sz = (int(np.rint(F32(w) / s)), int(np.rint(F32(h) / s)))
+        inv = F32(F32(1.0) / level_scale(k))                              # cv2 multiplies by the inverse scale; it does not divide
+        sz = (int(np.rint(F32(F32(w) * inv))), int(np.rint(F32(F32(h) * inv))))
         levels.append(cv2.resize(levels[-1], sz, interpolation=cv2.INTER_LINEAR_EXACT))
     return levels
 

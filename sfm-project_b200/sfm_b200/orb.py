@@ -32,11 +32,13 @@ def level_scale(level: int) -> np.float32:
 
 
 def level_sizes(width: int, height: int, n_levels: int = N_LEVELS):
-    """(w, h) of every pyramid level: round-half-even of the float32 quotient, as cv2 sizes them."""
+    """(w, h) of every pyramid level as cv2 sizes them: round-half-even of the float32 product w * float32(1 / scale).  Dividing
+    by the scale instead rounds differently on 281 (width, level) pairs below 8192, e.g. 525 / 1.2 = 437.49997 but
+    525 * float32(1 / 1.2) = 437.5 -> 438."""
     out = [(int(width), int(height))]
     for k in range(1, n_levels):
-        s = level_scale(k)
-        out.append((int(np.rint(F32(width) / s)), int(np.rint(F32(height) / s))))
+        inv = F32(F32(1.0) / level_scale(k))
+        out.append((int(np.rint(F32(F32(width) * inv))), int(np.rint(F32(F32(height) * inv)))))
     return out
 
 
