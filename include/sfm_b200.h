@@ -509,6 +509,78 @@ int sfm_pnp_ransac(int n_images, const double* cams, const int32_t* image, int n
                    const int32_t* count, const sfm_pnp_params* params, double* out_pose, int32_t* out_n_inliers, uint8_t* out_status,
                    uint8_t* out_mask, int32_t* out_iters, int64_t* out_counts, void* stream);
 
+/* ------------------------------------------------------------ bundle adjustment
+ * Every registered camera and every triangulated point refined together: the step that makes incremental reconstruction
+ * more than a first guess.  Cameras follow x ~ K (R X + t), as in track triangulation; the intrinsics stay fixed.
+ *
+ *   offsets, obs, track_counts   the tracks as sfm_tracks_finalize writes them (the track count is read from track_counts[0]
+ *                                on the device, clamped to max_tracks; the observation count is offsets[n_tracks], clamped to
+ *                                max_obs), so nothing waits for the host
+ *   point_status, obs_inlier, X  uint8 [max_tracks], uint8 [max_obs], double [max_tracks, 3]: as sfm_triangulate_tracks writes them
+ *   xy         float  [n_images, xy_stride, 2]   keypoint pixel coordinates; S <= xy_stride
+ *   cams       double [n_images, 16]             fx fy cx cy, R (row-major), t
+ *   registered uint8  [n_images] or NULL         NULL = every image
+ *   fixed      uint8  [n_images] or NULL         poses held fixed; NULL = the lowest-index registered image (the gauge's
+ *                                                rotation and origin; the scale is left to the damping)
+ *
+ * An observation is used iff its track has point status 0, its obs_inlier is 1 and its image is registered.  A camera is
+ * variable iff it is registered, not fixed and has a used observation; a point is adjusted iff it has 2 or more used
+ * observations.  Every other pose and point is returned bit-identical to its input.
+ * The cost is the sum over the used observations of ((p0 * (1/p2) - x^) * fx)^2 + ((p1 * (1/p2) - y^) * fy)^2 with
+ * p = R X + t and x^ = ((double)x - cx) / fx (track triangulation's residual), plain squares.  Levenberg-Marquardt in fp64:
+ *   parameters   a camera moves by registration's camera-frame perturbation R' = dR(w) R, t' = dR(w) t + dt (dR the
+ *                normalised quaternion (1, w/2), the Jacobian taken at p), a point by X' = X + dX
+ *   step         the damped normal equations (H + lambda diag(H)) [dc; dX] = -J^T r reduced to the variable cameras by the
+ *                Schur complement S = U - W V^-1 W^T (cameras compacted to 0..Nv-1, S dense, Nv <= 1024), solved by a blocked
+ *                Cholesky, then the points back-substituted; a trial with any used observation at p2 <= 0, or whose system
+ *                is not positive definite, is rejected
+ *   lambda       starts at 1e-4; Nielsen's rule: accepted (cost drops): lambda *= max(1/3, 1 - (2 rho - 1)^3), nu = 2;
+ *                rejected: lambda *= nu, nu *= 2.  The Jacobians are recomputed only after an accepted step
+ *   summary.status  0 function_tolerance: an accepted step lowered the cost by less than function_tolerance * cost
+ *                   1 parameter_tolerance: an accepted step had |dx| <= parameter_tolerance * (|x| + parameter_tolerance),
+ *                     x = (t of the variable cameras, the adjusted points), dx = (w, dt, dX)
+ *                   2 max_iterations: max_iters trials (rejected ones count)
+ *                   3 no_progress: lambda passed 1e32; the last accepted state is returned
+ *                   4 nothing_to_adjust: no variable camera and no adjusted point
+ *                   5 invalid: a used observation's track names an image outside [0, n_images) or a feature outside [0, S),
+ *                     or a registered image with used observations has a focal length that is not positive and finite
+ * Every sum runs in a fixed order (no floating-point atomics), so the result is bit-identical from run to run, on any
+ * stream, and with unregistered images added (the layout of the reduced system depends only on Nv).
+ * Outputs:
+ *   out_pose       double [n_images, 12]   R (row-major), t: drops into cams[:, 4:]
+ *   out_X          double [max_tracks, 3]
+ *   out_obs_error  float  [obs]            pixel reprojection error after the adjustment, as sfm_triangulate_tracks defines it
+ *                                          (+inf behind the camera, NaN in unregistered images and for tracks without a point)
+ *   out_summary    sfm_bundle_summary      (device memory)
+ * sfm_bundle_workspace_bytes sizes the caller-owned device workspace (the reduced system alone takes (6 n_images)^2 doubles);
+ * n_images is at most 1024.  The call issues 4 + 5 * max_iters launches whatever the data: once the solve has stopped, the
+ * remaining iterations' kernels exit at once.
+ */
+typedef struct {
+    double   function_tolerance;   /* >= 0 (default 1e-6)                          */
+    double   parameter_tolerance;  /* >= 0 (default 1e-8)                          */
+    int32_t  max_iters;            /* trials, in [1, 10000] (default 50)           */
+    int32_t  reserved[11];
+} sfm_bundle_params;
+
+typedef struct {
+    int64_t  status;               /* see above                                    */
+    int64_t  iterations;           /* trials run                                   */
+    int64_t  accepted;             /* accepted steps                               */
+    int64_t  used_obs;
+    int64_t  variable_cameras;     /* Nv                                           */
+    int64_t  adjusted_points;
+    double   initial_cost;
+    double   final_cost;
+} sfm_bundle_summary;
+
+int sfm_bundle_workspace_bytes(int n_images, int64_t max_tracks, int64_t max_obs, size_t* out_bytes);
+int sfm_bundle_adjust(int n_images, int S, const int64_t* offsets, const int32_t* obs, const int64_t* track_counts, int64_t max_tracks,
+                      int64_t max_obs, const uint8_t* point_status, const uint8_t* obs_inlier, const double* X, const float* xy,
+                      int xy_stride, const double* cams, const uint8_t* registered, const uint8_t* fixed, const sfm_bundle_params* params,
+                      void* workspace, size_t workspace_bytes, double* out_pose, double* out_X, float* out_obs_error,
+                      sfm_bundle_summary* out_summary, void* stream);
+
 /* ------------------------------------------ result regions in peer memory (multi-GPU gather)
  * Across ranks, the reference's `pair_matches.append(Pair(...))` (code/pipeline.py:43-47) becomes: every rank
  * writes the packed match rows / inlier flags of its pair block straight into a region of the gathering rank's

@@ -342,22 +342,14 @@ static __device__ int block_count(const PnpPts& pts, int M, const Camera& K, dou
 }
 
 // Adds one observation's Gauss-Newton terms at pose K: the upper triangle of J^T J (21, row by row, the u row's product then
-// the v row's), J^T r (6) and the squared error.  J is d(u, v) / d(w, t) for the camera-frame perturbation R' = dR(w) R,
-// t' = dR(w) t + dt, taken at p = R X + t: its linearisation error scales with the depth, not with |X|, so the step still
-// lowers the cost when the world is far from its origin.
+// the v row's), J^T r (6) and the squared error, with J the rows of pose_rows (ransac_common.cuh).
 static __device__ __forceinline__ void add_gn(double (&v)[kPnpSums], const Camera& K, double x, double y, const double* Xw)
 {
-    const double q0 = K.r[0] * Xw[0] + K.r[1] * Xw[1] + K.r[2] * Xw[2];
-    const double q1 = K.r[3] * Xw[0] + K.r[4] * Xw[1] + K.r[5] * Xw[2];
-    const double q2 = K.r[6] * Xw[0] + K.r[7] * Xw[1] + K.r[8] * Xw[2];
-    const double p0 = q0 + K.t[0], p1 = q1 + K.t[1], p2 = q2 + K.t[2];
-    const double iz = 1.0 / p2;
-    const double u0 = p0 * iz, u1 = p1 * iz;
-    const double ex = (u0 - x) * K.fx, ey = (u1 - y) * K.fy;
-    const double a0 = K.fx * iz, a2 = -(a0 * u0);
-    const double b1 = K.fy * iz, b2 = -(b1 * u1);
-    const double ju[6] = {a2 * p1, a0 * p2 - a2 * p0, -(a0 * p1), a0, 0.0, a2};
-    const double jv[6] = {b2 * p1 - b1 * p2, -(b2 * p0), b1 * p0, 0.0, b1, b2};
+    PoseRows J;
+    pose_rows(K, x, y, Xw, J);
+    const double ex = J.ex, ey = J.ey;
+    const double(&ju)[6] = J.ju;
+    const double(&jv)[6] = J.jv;
     int e = 0;
 #pragma unroll
     for (int i = 0; i < 6; ++i)
@@ -375,8 +367,8 @@ static __device__ __forceinline__ void add_gn(double (&v)[kPnpSums], const Camer
     v[27] = v[27] + (ex * ex + ey * ey);
 }
 
-// The Gauss-Newton step from the sums: Cholesky of J^T J, delta = -(J^T J)^-1 J^T r, R' = dR R with dR the rotation of the
-// normalised quaternion (1, w/2), t' = dR t + dt.  False when a pivot is not positive.
+// The Gauss-Newton step from the sums: Cholesky of J^T J, delta = -(J^T J)^-1 J^T r, applied by apply_pose_step
+// (ransac_common.cuh).  False when a pivot is not positive.
 static __device__ __forceinline__ bool gn_step(const double (&v)[kPnpSums], const Camera& K, Camera& O)
 {
     double H[36];
@@ -422,19 +414,7 @@ static __device__ __forceinline__ bool gn_step(const double (&v)[kPnpSums], cons
         for (int k = i + 1; k < 6; ++k) w = w - L[k * 6 + i] * dl[k];
         dl[i] = w * inv[i];
     }
-    const double hx = 0.5 * dl[0], hy = 0.5 * dl[1], hz = 0.5 * dl[2];
-    const double in = 1.0 / sqrt(1.0 + hx * hx + hy * hy + hz * hz);
-    const double qw = in, qx = hx * in, qy = hy * in, qz = hz * in;
-    const double D[9] = {1.0 - 2.0 * (qy * qy + qz * qz), 2.0 * (qx * qy - qw * qz), 2.0 * (qx * qz + qw * qy),
-                         2.0 * (qx * qy + qw * qz), 1.0 - 2.0 * (qx * qx + qz * qz), 2.0 * (qy * qz - qw * qx),
-                         2.0 * (qx * qz - qw * qy), 2.0 * (qy * qz + qw * qx), 1.0 - 2.0 * (qx * qx + qy * qy)};
-    O.fx = K.fx; O.fy = K.fy;
-#pragma unroll
-    for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int j = 0; j < 3; ++j) O.r[3 * i + j] = D[3 * i] * K.r[j] + D[3 * i + 1] * K.r[3 + j] + D[3 * i + 2] * K.r[6 + j];
-#pragma unroll
-    for (int i = 0; i < 3; ++i) O.t[i] = (D[3 * i] * K.t[0] + D[3 * i + 1] * K.t[1] + D[3 * i + 2] * K.t[2]) + dl[3 + i];
+    apply_pose_step(dl, K, O);
     return true;
 }
 

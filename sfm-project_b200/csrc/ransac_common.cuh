@@ -322,6 +322,53 @@ static __device__ __forceinline__ bool reproject(const Camera& K, const double* 
     return e2 <= thr2;
 }
 
+// The pixel residual of one observation (x^, y^) of Xw at pose K and its Jacobian rows for the camera-frame perturbation
+// R' = dR(w) R, t' = dR(w) t + dt, taken at p = R X + t: its linearisation error scales with the depth, not with |X|, so a
+// step still lowers the cost when the world is far from its origin.  Shared by registration (pnp.cu) and bundle
+// adjustment (bundle.cu); d(u, v) / dp is (a0, 0, a2) and (0, b1, b2), so d(u, v) / dX is that times R.
+struct PoseRows {
+    double p0, p1, p2;
+    double a0, a2, b1, b2;
+    double ex, ey;
+    double ju[6], jv[6];                // d(u, v) / d(w, t)
+};
+
+static __device__ __forceinline__ void pose_rows(const Camera& K, double x, double y, const double* Xw, PoseRows& J)
+{
+    const double q0 = K.r[0] * Xw[0] + K.r[1] * Xw[1] + K.r[2] * Xw[2];
+    const double q1 = K.r[3] * Xw[0] + K.r[4] * Xw[1] + K.r[5] * Xw[2];
+    const double q2 = K.r[6] * Xw[0] + K.r[7] * Xw[1] + K.r[8] * Xw[2];
+    const double p0 = q0 + K.t[0], p1 = q1 + K.t[1], p2 = q2 + K.t[2];
+    const double iz = 1.0 / p2;
+    const double u0 = p0 * iz, u1 = p1 * iz;
+    J.p0 = p0; J.p1 = p1; J.p2 = p2;
+    J.ex = (u0 - x) * K.fx;
+    J.ey = (u1 - y) * K.fy;
+    J.a0 = K.fx * iz; J.a2 = -(J.a0 * u0);
+    J.b1 = K.fy * iz; J.b2 = -(J.b1 * u1);
+    J.ju[0] = J.a2 * p1; J.ju[1] = J.a0 * p2 - J.a2 * p0; J.ju[2] = -(J.a0 * p1); J.ju[3] = J.a0; J.ju[4] = 0.0; J.ju[5] = J.a2;
+    J.jv[0] = J.b2 * p1 - J.b1 * p2; J.jv[1] = -(J.b2 * p0); J.jv[2] = J.b1 * p0; J.jv[3] = 0.0; J.jv[4] = J.b1; J.jv[5] = J.b2;
+}
+
+// The pose after the step dl = (w, dt) of that perturbation: R' = dR R with dR the rotation of the normalised quaternion
+// (1, w/2), t' = dR t + dt.
+static __device__ __forceinline__ void apply_pose_step(const double* dl, const Camera& K, Camera& O)
+{
+    const double hx = 0.5 * dl[0], hy = 0.5 * dl[1], hz = 0.5 * dl[2];
+    const double in = 1.0 / sqrt(1.0 + hx * hx + hy * hy + hz * hz);
+    const double qw = in, qx = hx * in, qy = hy * in, qz = hz * in;
+    const double D[9] = {1.0 - 2.0 * (qy * qy + qz * qz), 2.0 * (qx * qy - qw * qz), 2.0 * (qx * qz + qw * qy),
+                         2.0 * (qx * qy + qw * qz), 1.0 - 2.0 * (qx * qx + qz * qz), 2.0 * (qy * qz - qw * qx),
+                         2.0 * (qx * qz - qw * qy), 2.0 * (qy * qz + qw * qx), 1.0 - 2.0 * (qx * qx + qy * qy)};
+    O.fx = K.fx; O.fy = K.fy;
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) O.r[3 * i + j] = D[3 * i] * K.r[j] + D[3 * i + 1] * K.r[3 + j] + D[3 * i + 2] * K.r[6 + j];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) O.t[i] = (D[3 * i] * K.t[0] + D[3 * i + 1] * K.t[1] + D[3 * i + 2] * K.t[2]) + dl[3 + i];
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Cooperative Gauss-Jordan elimination with complete pivoting: 8 lanes (one aligned octet of a warp) reduce ONE
 // m x 9 system, lane r holding row r in registers (a[0..8], statically indexed).  Value for value the serial

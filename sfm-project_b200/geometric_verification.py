@@ -338,3 +338,31 @@ def register_images(tracks, points, keypoints, K, R, t, images, *, registered=No
         else:
             registered[img.cpu().numpy()] = 1
     return res
+
+
+# ------------------------------------------------------------------ bundle adjustment (cameras + points, jointly)
+def bundle_adjust(tracks, points, keypoints, K, R, t, *, registered=None, fixed=None, max_iters=50, function_tolerance=1e-6,
+                  parameter_tolerance=1e-8):
+    """Refine the registered cameras ``x ~ K (R X + t)`` and the triangulated points together (csrc/bundle.cu):
+    Levenberg-Marquardt on the squared pixel errors of every observation whose track has a point (``points``, from
+    ``triangulate_tracks``), that is an inlier of it and lies in a registered image; intrinsics fixed, no robust loss.
+
+    ``tracks``, ``keypoints``, ``K``, ``R``, ``t``, ``registered`` as ``triangulate_tracks``; ``fixed`` bool / uint8 [n] or None
+    (None: the lowest-index registered camera is held fixed).  At most 1024 cameras.  Returns a dict of numpy ``R`` [n,3,3],
+    ``t`` [n,3], ``X`` [T,3], ``obs_error`` [n_obs] (pixel error after the adjustment; NaN where triangulation writes NaN) and
+    ``status`` (one of ``sfm_b200.bundle.STATUS_NAMES``), ``iterations``, ``accepted``, ``initial_cost``, ``final_cost``,
+    ``used_obs``, ``variable_cameras``, ``adjusted_points``."""
+    from sfm_b200 import bundle
+    from sfm_b200 import triangulate as tri
+
+    cams = tri.camera_table(K, R, t)
+    n = cams.shape[0]
+    tracks = _device_tracks(tracks)
+    dev = tracks.obs_buf.device
+    xy, S = _keypoints(keypoints, n, dev)
+    reg = None if registered is None else (np.asarray(registered).reshape(-1) != 0).astype(np.uint8)
+    fix = None if fixed is None else (np.asarray(fixed).reshape(-1) != 0).astype(np.uint8)
+    res = bundle.bundle_adjust_device(tracks, points, xy, torch.from_numpy(cams).to(dev), reg, fixed=fix, S=S, max_iters=max_iters,
+                                      function_tolerance=function_tolerance, parameter_tolerance=parameter_tolerance).to_host()
+    res.pop("pose")
+    return res

@@ -32,7 +32,7 @@ EXPORTS = [
     "sfm_two_view_pose_batch", "sfm_two_view_pose_packed",
     "sfm_orb_resize", "sfm_orb_blur", "sfm_orb_describe", "sfm_orb_fast_detect", "sfm_orb_retain_best", "sfm_orb_harris_angle",
     "sfm_tracks_workspace_bytes", "sfm_tracks_init", "sfm_tracks_hook", "sfm_tracks_finalize", "sfm_triangulate_tracks",
-    "sfm_pnp_gather", "sfm_pnp_ransac",
+    "sfm_pnp_gather", "sfm_pnp_ransac", "sfm_bundle_workspace_bytes", "sfm_bundle_adjust",
     "sfm_peer_alloc", "sfm_peer_open", "sfm_peer_close", "sfm_peer_free", "sfm_copy_async", "sfm_probe_int8_mma", "sfm_debug_tc_tile", "sfm_debug_refine_stats", "sfm_launch_count",
 ]
 
@@ -71,6 +71,16 @@ class TriangulateParams(C.Structure):
 class PnpParams(C.Structure):
     _fields_ = [("max_error", C.c_double), ("confidence", C.c_double), ("seed", C.c_uint64), ("max_iters", C.c_int32),
                 ("min_inliers", C.c_int32), ("min_inlier_ratio", C.c_double), ("refine_iters", C.c_int32), ("reserved", C.c_int32 * 5)]
+
+
+class BundleParams(C.Structure):
+    _fields_ = [("function_tolerance", C.c_double), ("parameter_tolerance", C.c_double), ("max_iters", C.c_int32),
+                ("reserved", C.c_int32 * 11)]
+
+
+class BundleSummary(C.Structure):
+    _fields_ = [("status", C.c_int64), ("iterations", C.c_int64), ("accepted", C.c_int64), ("used_obs", C.c_int64),
+                ("variable_cameras", C.c_int64), ("adjusted_points", C.c_int64), ("initial_cost", C.c_double), ("final_cost", C.c_double)]
 
 
 class SfmError(RuntimeError):
@@ -128,6 +138,9 @@ def lib():
                                          vp, vp, vp]
     L.sfm_pnp_gather.argtypes = [i32, i32, vp, vp, C.c_int64, vp, vp, vp, i32, vp, i32, vp, vp, vp, vp, vp]
     L.sfm_pnp_ransac.argtypes = [i32, vp, vp, i32, vp, vp, i32, vp, C.POINTER(PnpParams), vp, vp, vp, vp, vp, vp, vp]
+    L.sfm_bundle_workspace_bytes.argtypes = [i32, C.c_int64, C.c_int64, C.POINTER(sz)]
+    L.sfm_bundle_adjust.argtypes = [i32, i32, vp, vp, vp, C.c_int64, C.c_int64, vp, vp, vp, vp, i32, vp, vp, vp, C.POINTER(BundleParams),
+                                    vp, sz, vp, vp, vp, vp, vp]
     L.sfm_peer_alloc.argtypes = [i32, sz, C.POINTER(vp), vp]
     L.sfm_peer_open.argtypes = [i32, vp, C.POINTER(vp)]
     L.sfm_peer_close.argtypes = [i32, vp]
