@@ -581,6 +581,67 @@ int sfm_bundle_adjust(int n_images, int S, const int64_t* offsets, const int32_t
                       void* workspace, size_t workspace_bytes, double* out_pose, double* out_X, float* out_obs_error,
                       sfm_bundle_summary* out_summary, void* stream);
 
+/* ------------------------------------------------------------ incremental reconstruction
+ * The two steps that join registration, triangulation and bundle adjustment into COLMAP's incremental mapper
+ * (Schoenberger & Frahm, CVPR 2016): which images to register next, and which points to keep after an adjustment.  Both
+ * read and write the arrays the other stages use, so a reconstruction loop never moves data to the host.
+ *
+ * sfm_next_images: next-best-view selection (COLMAP's IncrementalMapper::FindNextImages, visibility-pyramid score, §4.2):
+ *   track_of, track_counts   as sfm_tracks_finalize writes them ([n_images, S]; the track count is read on the device)
+ *   point_status             uint8 [max_tracks]: as sfm_triangulate_tracks (or sfm_filter_points) writes it
+ *   xy                       float [n_images, xy_stride, 2]   keypoint pixel coordinates; S <= xy_stride
+ *   image_size               int32 [n_images, 2]   (w, h) in pixels
+ *   registered               uint8 [n_images]
+ *   trials                   int32 [n_images]      registration attempts so far; incremented for every selected image
+ * The visible points of image i are its features f whose track k = track_of[i * S + f] satisfies 0 <= k < min(track_counts[0],
+ * max_tracks) and point_status[k] == 0: sfm_pnp_gather's predicate, so out_visible[i] equals the gather's out_count for i.
+ * Score: for each level l in [0, levels), d = 2^(l+1), a visible point at (x, y) occupies the cell
+ *   cx = clamp(floor((double)x * d / w), 0, d - 1), cy likewise with y and h   (fp64, IEEE; a NaN cell index is 0)
+ * and score = sum over l of d^2 * (occupied cells at level l), in int64: exact and independent of the point order.
+ * The candidates are the images with registered == 0, trials < max_trials and visible >= min_visible, ordered by score
+ * descending, then visible descending, then image ascending; the first max_select go to out_images (padded with -1), their
+ * trials are incremented, and their number goes to out_n_selected.  A -1 entry gets out_count 0 from sfm_pnp_gather and
+ * status 4 from sfm_pnp_ransac, so out_images can be registered as it stands.
+ * Outputs: out_images int32 [max_select], out_n_selected int32 [1], out_visible int32 [n_images], out_score int64 [n_images].
+ * n_images is at most 1024 (bundle adjustment's cap).  Two launches: one CTA per image for the score (the occupancy bits of
+ * every level in shared memory), then one CTA for the selection.
+ *
+ * sfm_filter_points: COLMAP's post-adjustment point filter, in place on the outputs of sfm_triangulate_tracks.  For every
+ * track with point_status 0:
+ *   an observation stays an inlier iff it was one, its image is registered and (double)obs_error <= max_error (NaN and +inf
+ *   fail); n_inliers becomes the number that stay
+ *   with fewer than min_inliers left the status becomes 3 (too_few_inliers); otherwise, when no pair a < b of the remaining
+ *   inliers has cos(angle(X - C_a, X - C_b)) <= cos(min_angle) (C = -R^T t; the operations of triangulation's hypothesis
+ *   test, cos(min_angle) computed once on the host in the same way), the status becomes 2 (no_model)
+ * A track whose status changes gets X = 0 and every obs_inlier 0, and n_inliers 0 for status 2, so the outputs keep
+ * triangulation's invariants and every consumer reads them as it reads triangulation's.  obs_error is read only.  Tracks of
+ * other statuses are left as they are (a status-0 track has only observations inside [0, n_images) x [0, S): triangulation
+ * gives any other track status 4).  out_counts int64 [5] receives the tracks per status after the filter.  One warp per
+ * track; one launch after a memset of out_counts.
+ */
+typedef struct {
+    int32_t  min_visible;   /* >= 0 (default 30: registration's min_inliers)                          */
+    int32_t  max_trials;    /* >= 1 (default 3: COLMAP's max_reg_trials)                              */
+    int32_t  max_select;    /* >= 1: images selected per call                                         */
+    int32_t  levels;        /* pyramid levels, in [1, 8] (default 6: 5,460 cells)                     */
+    int32_t  reserved[12];
+} sfm_next_images_params;
+
+typedef struct {
+    double   max_error;     /* pixels, >= 0 and finite (COLMAP's filter_max_reproj_error: 4)           */
+    double   min_angle;     /* degrees, in [0, 90) (COLMAP's filter_min_tri_angle: 1.5)               */
+    int32_t  min_inliers;   /* >= 2                                                                   */
+    int32_t  reserved[11];
+} sfm_filter_points_params;
+
+int sfm_next_images(int n_images, int S, const int32_t* track_of, const int64_t* track_counts, int64_t max_tracks,
+                    const uint8_t* point_status, const float* xy, int xy_stride, const int32_t* image_size, const uint8_t* registered,
+                    int32_t* trials, const sfm_next_images_params* params, int32_t* out_images, int32_t* out_n_selected,
+                    int32_t* out_visible, int64_t* out_score, void* stream);
+int sfm_filter_points(int n_images, const int64_t* offsets, const int32_t* obs, const int64_t* track_counts, int64_t max_tracks,
+                      const double* cams, const uint8_t* registered, const float* obs_error, const sfm_filter_points_params* params,
+                      double* X, int32_t* n_inliers, uint8_t* point_status, uint8_t* obs_inlier, int64_t* out_counts, void* stream);
+
 /* ------------------------------------------ result regions in peer memory (multi-GPU gather)
  * Across ranks, the reference's `pair_matches.append(Pair(...))` (code/pipeline.py:43-47) becomes: every rank
  * writes the packed match rows / inlier flags of its pair block straight into a region of the gathering rank's

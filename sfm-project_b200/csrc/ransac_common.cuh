@@ -322,6 +322,26 @@ static __device__ __forceinline__ bool reproject(const Camera& K, const double* 
     return e2 <= thr2;
 }
 
+// Camera centre C = -R^T t
+static __device__ __forceinline__ void camera_center(const Camera& K, double* C)
+{
+#pragma unroll
+    for (int i = 0; i < 3; ++i) C[i] = -(K.r[i] * K.t[0] + K.r[3 + i] * K.t[1] + K.r[6 + i] * K.t[2]);
+}
+
+// cos of the angle at X between the rays from the centres Ca and Cb: the triangulation angle.  Track triangulation
+// (triangulate.cu) keeps a hypothesis and the point filter (mapper.cu) keeps a point only when some pair of its views has
+// ray_cos <= cos(min_angle); both use this one sequence of operations, so they agree to the bit.  Symmetric in a and b.
+static __device__ __forceinline__ double ray_cos(const double* X, const double* Ca, const double* Cb)
+{
+    const double da0 = X[0] - Ca[0], da1 = X[1] - Ca[1], da2 = X[2] - Ca[2];
+    const double db0 = X[0] - Cb[0], db1 = X[1] - Cb[1], db2 = X[2] - Cb[2];
+    const double dot = da0 * db0 + da1 * db1 + da2 * db2;
+    const double na = da0 * da0 + da1 * da1 + da2 * da2;
+    const double nb = db0 * db0 + db1 * db1 + db2 * db2;
+    return dot / sqrt(na * nb);
+}
+
 // The pixel residual of one observation (x^, y^) of Xw at pose K and its Jacobian rows for the camera-frame perturbation
 // R' = dR(w) R, t' = dR(w) t + dt, taken at p = R X + t: its linearisation error scales with the depth, not with |X|, so a
 // step still lowers the cost when the world is far from its origin.  Shared by registration (pnp.cu) and bundle

@@ -134,13 +134,6 @@ static __device__ __forceinline__ double depth(const Camera& K, const double* X)
     return K.r[6] * X[0] + K.r[7] * X[1] + K.r[8] * X[2] + K.t[2];
 }
 
-// C = -R^T t
-static __device__ __forceinline__ void center(const Camera& K, double* C)
-{
-#pragma unroll
-    for (int i = 0; i < 3; ++i) C[i] = -(K.r[i] * K.t[0] + K.r[3 + i] * K.t[1] + K.r[6 + i] * K.t[2]);
-}
-
 // Hypothesis `hyp` of track `k`: the DLT point of two usable observations (the earlier one's rows first), kept (ok = 1) iff
 // both depths are positive and the ray angle at the point is at least min_angle (cos <= cos_min).
 static __device__ __forceinline__ Point hypothesis(const TriInputs& in, const TriTrack& tk, uint64_t seed, uint32_t k, int hyp, int M,
@@ -165,14 +158,9 @@ static __device__ __forceinline__ Point hypothesis(const TriInputs& in, const Tr
     if (!P.ok) return P;
     const double* X = P.x;
     double Ca[3], Cb[3];
-    center(A, Ca);
-    center(B, Cb);
-    const double da0 = X[0] - Ca[0], da1 = X[1] - Ca[1], da2 = X[2] - Ca[2];
-    const double db0 = X[0] - Cb[0], db1 = X[1] - Cb[1], db2 = X[2] - Cb[2];
-    const double dot = da0 * db0 + da1 * db1 + da2 * db2;
-    const double na = da0 * da0 + da1 * da1 + da2 * da2;
-    const double nb = db0 * db0 + db1 * db1 + db2 * db2;
-    const double cosang = dot / sqrt(na * nb);
+    camera_center(A, Ca);
+    camera_center(B, Cb);
+    const double cosang = ray_cos(X, Ca, Cb);
     P.ok = depth(A, X) > 0.0 && depth(B, X) > 0.0 && cosang <= cos_min;
     return P;
 }

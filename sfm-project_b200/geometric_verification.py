@@ -366,3 +366,16 @@ def bundle_adjust(tracks, points, keypoints, K, R, t, *, registered=None, fixed=
                                       function_tolerance=function_tolerance, parameter_tolerance=parameter_tolerance).to_host()
     res.pop("pose")
     return res
+
+
+def reconstruct(result, bank, K, **kw):
+    """Cameras and points from the verified matches: incremental reconstruction on the GPU (``sfm_b200.reconstruct_device``,
+    COLMAP's incremental mapper) of a ``match_and_verify(bank, pairs, intrinsics=K, tracks=True)`` result (``homography=True``
+    adds the initial pair's planarity test).  ``K`` one pinhole [3,3] or [n_images,3,3]; ``kw`` as ``reconstruct_device``.
+    Returns a dict of numpy ``R`` [n,3,3], ``t`` [n,3] (x ~ K (R X + t)), ``registered`` [n], ``round`` [n] (the round that
+    registered each image, -1 if never), ``X`` [T,3], ``point_status`` [T] (``sfm_b200.triangulate.STATUS_NAMES`` codes),
+    ``obs_inlier`` and ``obs_error`` [n_obs], and ``init_pair``, ``status`` ("ok" or "no_initial_pair") and ``rounds`` (the
+    per-round log)."""
+    from sfm_b200 import mapper
+
+    return mapper.reconstruct_device(result, bank.xy, K, **kw).to_host()

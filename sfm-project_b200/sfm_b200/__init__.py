@@ -15,4 +15,5 @@ from .tracks import Tracks, build_tracks_device  # noqa: F401
 from .triangulate import TrackPoints, triangulate_tracks_device  # noqa: F401
 from .pnp import AbsolutePoses, pnp_ransac_device, register_images_device  # noqa: F401
 from .bundle import BundleResult, bundle_adjust_device  # noqa: F401
+from .mapper import NextImages, Reconstruction, filter_points_device, next_images_device, reconstruct_device  # noqa: F401
 from .pairs import Pair, blocked_exhaustive_pairs, exhaustive_pairs, ordered_pairs, to_reference_pairs, windowed_pairs  # noqa: F401
